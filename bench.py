@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — PAF liftover + stats hot path on B200 (the metric of BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--haps H]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--haps H] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload, the SAME FIXED JOB at every N ("scaling": "strong"): BASELINE.json's C5 — H = 94 synthetic haplotypes
@@ -17,6 +17,9 @@ per-row `rb stats --paf` counters.  A step = one pass of the hot path over the w
 At N = 1 the line also carries "c4": BASELINE's C4 (one haplotype, 1 kb windows: the workload of round 1's headline) with its
 own resident / e2e / per-kernel roofline numbers, and the rows of a few contigs of BOTH workloads are compared byte for byte
 with the CPU oracle ("parity_checked_rows").
+--dump-outputs DIR: what the last timed resident step of C4 and C5 computed (the PAF rows, their line offsets and the stats
+counters), as a fixed, seeded sample of rows in DIR/<name>.npy, so that two builds can be compared output for output.  The
+synthetic inputs depend only on the arguments.
 """
 import argparse
 import ctypes as C
@@ -42,6 +45,10 @@ REF_SAMPLE_CONTIGS = ["chr21", "chr22", "chrM"]  # --impl reference, per step: ~
 CPU_BASELINE_CONTIGS = ["chr16", "chr17", "chr18", "chr19", "chr20", "chr21", "chr22", "chrM"]  # cpu_baseline: ~0.5 Gbp, one pass
 C4_PARITY_CONTIGS = ["chr20", "chr21", "chr22", "chrM"]
 DTYPE = "u32/u64 (+f32 identities)"
+# --dump-outputs, per workload: rows drawn, and bytes of their text kept (4 B each as float32): ~22 MB, C4 + C5 under 64 MB
+DUMP_ROWS, DUMP_TEXT_BYTES, DUMP_SEED = 65536, 4 << 20, 0
+STATS_U32 = ("equal", "diff", "ins", "del", "ins_events", "del_events", "matches")
+STATS_F32 = ("id_by_matches", "id_by_events", "id_by_all")
 
 
 def workload_name(haps):
@@ -258,8 +265,39 @@ def algorithmic_bytes(summ, n_win, n_rec):
     return per_kernel, whole
 
 
-def measure_resident(torch, ctx, stream, flush, paf, wins, steps, warmup, barrier):
-    """W + K resident steps (inputs uploaded once), then a pass with CUDA events around every kernel."""
+def sample_outputs(views, prefix, share=1.0):
+    """A fixed, seeded sample of one liftover's outputs as float arrays: the line offset, length and stats counters of
+    `share` * DUMP_ROWS rows drawn without replacement (u32 / u64 values are exact in float64, the f32 identities stay f32),
+    the text bytes of the first drawn rows that fit `share` * DUMP_TEXT_BYTES (as float32), the row count and byte total, and
+    every counter summed over all rows."""
+    import numpy as np
+    n = views["n_out"]
+    off, text, st = views["line_off"], views["paf_text"], views["stats"]
+    drawn = np.random.default_rng(DUMP_SEED).choice(n, size=min(n, int(DUMP_ROWS * share)), replace=False)
+    rows = np.sort(drawn)
+    start, end = off[rows].astype(np.int64), off[rows + 1].astype(np.int64)
+    out = {"counts": np.array([n, views["n_pairs"], views["paf_nbytes"]], dtype=np.float64),
+           "rows": rows.astype(np.float64), "line_off": start.astype(np.float64), "line_len": (end - start).astype(np.float64),
+           "stats_totals": np.array([st[k].sum(dtype=np.uint64) for k in STATS_U32], dtype=np.float64)}
+    out.update({k: st[k][rows].astype(np.float64) for k in STATS_U32})
+    out.update({k: st[k][rows].astype(np.float32) for k in STATS_F32})
+    lens = (off[drawn + 1] - off[drawn]).astype(np.int64)
+    text_rows = np.sort(drawn[:int(np.searchsorted(np.cumsum(lens), DUMP_TEXT_BYTES * share, side="right"))])
+    out["text_rows"] = text_rows.astype(np.float64)
+    out["text"] = np.concatenate([text[int(off[r]):int(off[r + 1])] for r in text_rows] or [np.zeros(0, np.uint8)]).astype(np.float32)
+    return {f"{prefix}_{k}": v for k, v in out.items()}
+
+
+def write_outputs(directory, arrays):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
+def measure_resident(torch, ctx, stream, flush, paf, wins, steps, warmup, barrier, dump=None, dump_share=1.0):
+    """W + K resident steps (inputs uploaded once), then a pass with CUDA events around every kernel.  dump: a name prefix
+    under which the outputs of the last timed step are sampled (sample_outputs) into the result's "dump"."""
     from rustybam_b200 import capi
     b = ctx.upload(paf, wins)
     summ = None
@@ -276,6 +314,12 @@ def measure_resident(torch, ctx, stream, flush, paf, wins, steps, warmup, barrie
         e1.synchronize()
         step_ms.append(e0.elapsed_time(e1))
     barrier()
+    dumped = None
+    if dump:
+        views, release = ctx.batch_download_lift_view(b, want=capi.WANT_TEXT, stats=True)
+        dumped = sample_outputs(views, dump, dump_share)
+        release()
+        barrier()
     ctx.set_profiling(True)
     ctx.kernel_times(reset=True)
     n_prof = max(3, steps // 4)
@@ -292,7 +336,7 @@ def measure_resident(torch, ctx, stream, flush, paf, wins, steps, warmup, barrie
     ktimes = ctx.kernel_times(reset=True)
     ctx.set_profiling(False)
     ctx.batch_free(b)
-    return dict(ms=sum(step_ms) / len(step_ms), summ=summ, ktimes=ktimes, n_prof=n_prof, prof_ms=sum(prof_ms) / len(prof_ms))
+    return dict(ms=sum(step_ms) / len(step_ms), summ=summ, ktimes=ktimes, n_prof=n_prof, prof_ms=sum(prof_ms) / len(prof_ms), dump=dumped)
 
 
 def measure_e2e(ctx, paf, wins, steps, warmup, barrier, stream=None, torch=None, flush=None, want=None):
@@ -378,7 +422,10 @@ def main():
     ap.add_argument("--scale", type=float, default=1.0, help="genome scale (1.0 = ~3.1 Gbp, the BASELINE configs)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--only-c4", action="store_true", help="only the C4 sub-bench (one haplotype, 1 kb windows): tuning runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs samples the outputs of the B200 path; --impl reference has none to sample")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -432,10 +479,12 @@ def main():
         wins4 = paf4.tiling_windows(C4_WINDOW)
         pin4 = Pinner(lib)
         ids4 = pin4.pin(paf4, wins4)
-        r4 = measure_resident(torch, ctx, stream, flush, paf4, wins4, max(args.steps, 10), args.warmup, barrier)
-        e4 = measure_e2e(ctx, paf4, wins4, max(args.steps, 10), args.warmup, barrier, stream, torch, flush)
+        r4 = measure_resident(torch, ctx, stream, flush, paf4, wins4, args.steps, args.warmup, barrier, dump=args.dump_outputs and "c4")
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, r4["dump"])
+        e4 = measure_e2e(ctx, paf4, wins4, args.steps, args.warmup, barrier, stream, torch, flush)
         h2d4, d2h4 = copy_bytes(paf4, wins4, ids4, e4["n_out"], e4["out_bytes"])
-        t4 = measure_e2e(ctx, paf4, wins4, max(args.steps, 10), args.warmup, barrier, stream, torch, flush, want=capi.WANT_STATS_TEXT)
+        t4 = measure_e2e(ctx, paf4, wins4, args.steps, args.warmup, barrier, stream, torch, flush, want=capi.WANT_STATS_TEXT)
         s4 = r4["summ"]
         c4 = {"workload": "C4: rb liftover --bed <1 kb tiling windows> over synthetic HG002-vs-CHM13-scale eqx PAF + per-row rb stats --paf",
               "value": s4["n_out"] / (r4["ms"] * 1e-3), "unit": UNIT, "ms_per_step": r4["ms"], "records": paf4.n_rec, "bed_rows": wins4.n_win,
@@ -474,7 +523,10 @@ def main():
     gen_s = time.time() - t0
     pin = Pinner(lib)
     ids_bytes = pin.pin(shard, wins)
-    res = measure_resident(torch, ctx, stream, flush, shard, wins, args.steps, args.warmup, barrier)
+    res = measure_resident(torch, ctx, stream, flush, shard, wins, args.steps, args.warmup, barrier,
+                           dump=args.dump_outputs and ("c5" if world == 1 else f"c5_rank{rank}"), dump_share=1.0 / world)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, res["dump"])
     # per-rank end to end: every rank lifts its own shard through rb_liftover (host buffers both ways)
     e2e_rank = measure_e2e(ctx, shard, wins, args.steps, args.warmup, barrier, stream, torch, flush)
     e2e_st = measure_e2e(ctx, shard, wins, args.steps, args.warmup, barrier, stream, torch, flush, want=capi.WANT_STATS_TEXT)

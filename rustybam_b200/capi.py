@@ -258,6 +258,9 @@ class Context:
         out, st = RbLiftOut(), RbStatsOut()
         self._check(self.lib.rb_liftover(self.h, C.byref(recs.c), C.byref(wins.c), policy, want, C.byref(out),
                                          C.byref(st) if stats else None))
+        return self._lift_views(out, st, want, stats)
+
+    def _lift_views(self, out, st, want, stats):
         n, nb = int(out.n_out), int(out.paf_nbytes)
 
         def view(ptr, cnt, dt):
@@ -398,6 +401,12 @@ class Context:
         if stats:
             self.lib.rb_free_stats_out(self.h, C.byref(st))
         return res
+
+    def batch_download_lift_view(self, b, want=WANT_TEXT | WANT_NUMERIC, stats=True):
+        """rb_batch_download_lift without copying: (views, release) as liftover_view returns them."""
+        out, st = RbLiftOut(), RbStatsOut()
+        self._check(self.lib.rb_batch_download_lift(self.h, b, want, C.byref(out), C.byref(st) if stats else None))
+        return self._lift_views(out, st, want, stats)
 
     def batch_download_stats(self, b):
         st = RbStatsOut()

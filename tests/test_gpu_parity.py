@@ -280,6 +280,13 @@ def test_resident_batch_is_repeatable(ctx):
     assert s1 == s2
     out = ctx.batch_download_lift(b)
     assert out["paf_text"] == orc.run_liftover(paf_text, gen.tiling_bed(contigs, 9))
+    views, release = ctx.batch_download_lift_view(b)  # the same outputs, left in the library's pinned block
+    assert views["paf_text"].tobytes() == out["paf_text"]
+    for k in ("line_off", "q_st", "t_en", "rec_idx", "win_idx"):
+        assert (views[k] == out[k]).all(), k
+    for k in ("equal", "diff", "ins", "del", "ins_events", "del_events", "matches", "id_by_all"):
+        assert (views["stats"][k] == out["stats"][k]).all(), k
+    release()
     ctx.batch_free(b)
 
 
