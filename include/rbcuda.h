@@ -47,7 +47,8 @@ typedef enum rb_status {
     RB_ERR_REF_STRIP = -6,       /* remove_trailing_indels panics: empty CIGAR, leading deletion, all-indel; paf.rs:663,782 */
     RB_ERR_REF_INDEX = -7,       /* "Problem getting index in cigar", liftover.rs:31-49 */
     RB_ERR_UNSUPPORTED = -8,     /* outside this path's documented domain: op length >= 2^28, per-record sums >= 2^32 */
-    RB_ERR_OOM = -9
+    RB_ERR_OOM = -9,
+    RB_ERR_REF_PAF_PARSE = -10   /* PafRecord::new asserts: a line of < 12 columns, or an extra token that is not a tag (paf.rs:381,387-389) */
 } rb_status;
 
 /* binary_search duplicate policy of the reference's toolchain (SURVEY.md Q2): which of several
@@ -225,6 +226,27 @@ int rb_batch_break(rb_ctx* ctx, rb_batch* b, uint32_t max_size, int policy, uint
 int rb_batch_download_lift(rb_ctx* ctx, rb_batch* b, uint32_t want, rb_lift_out* out, rb_stats_out* stats);
 int rb_batch_download_stats(rb_ctx* ctx, rb_batch* b, rb_stats_out* stats);
 void rb_batch_free(rb_ctx* ctx, rb_batch* b);
+
+/* ---- PAF text parsed on the device (Paf::from_file, paf.rs:62-78,379-430, quirk for quirk as the host reader restates it) ---- */
+typedef struct rb_paf_info {
+    uint64_t text_bytes;  /* PAF text parsed (the inflated size for BGZF input) */
+    uint64_t n_lines, skipped;
+    uint32_t n_rec, n_names;
+    const uint8_t* names; const uint64_t* names_off;  /* the batch's name table: ids by first appearance in file order, query name
+                                                          before target name per record; library-owned, valid until rb_batch_free */
+    uint64_t cigar_bytes;
+} rb_paf_info;
+/* PAF text, or BGZF bytes (recognised with rb_is_bgzf), -> a resident batch without windows; lines are split, tokenised and packed on
+ * the device (the context's first device), only the name bytes of the records come back for interning.  Where the reference panics
+ * the call fails: RB_ERR_REF_PAF_PARSE (< 12 columns, a bad tag), RB_ERR_REF_CIGAR_PARSE (a skipped line with a malformed cg tag);
+ * rb_last_error names the 1-based line.  A plain (single-member) gzip file is refused with RB_ERR_BAD_ARG: inflate it first.
+ * info is nullable. */
+rb_batch* rb_batch_upload_paf(rb_ctx* ctx, const uint8_t* data, uint64_t nbytes, rb_paf_info* info, int* status);
+/* windows for a batch that was uploaded without them (t_id = ids of that batch's name table); replaces any it had */
+int rb_batch_set_windows(rb_ctx* ctx, rb_batch* b, const rb_windows* wins);
+/* the batch's records as rb_records in library-owned pinned memory (CIGAR bytes only if with_cigar), valid until rb_batch_free or the
+ * next rb_batch_records on the batch */
+int rb_batch_records(rb_ctx* ctx, rb_batch* b, int with_cigar, rb_records* out);
 
 /* ---- host helper: stable sort of BED rows by (t_id, st) into the rb_windows layout ----
  * perm_out[n_win] receives, for each sorted position, the BED row it came from. */

@@ -7,6 +7,7 @@
 use std::os::raw::{c_char, c_int, c_void};
 
 #[repr(C)] pub struct rb_ctx { _p: [u8; 0] }
+#[repr(C)] pub struct rb_batch { _p: [u8; 0] }
 
 #[repr(C)]
 pub struct rb_records {
@@ -37,6 +38,15 @@ pub struct rb_stats_out {
     pub id_by_matches: *mut f32, pub id_by_events: *mut f32, pub id_by_all: *mut f32,
     pub _owner: *mut c_void,
 }
+#[repr(C)]
+pub struct rb_paf_info {
+    pub text_bytes: u64, pub n_lines: u64, pub skipped: u64,
+    pub n_rec: u32, pub n_names: u32,
+    pub names: *const u8, pub names_off: *const u64,
+    pub cigar_bytes: u64,
+}
+#[repr(C)]
+pub struct rb_summary { pub n_ops: u64, pub n_pairs: u64, pub n_out: u64, pub out_bytes: u64, pub cigar_bytes: u64 }
 extern "C" {
     pub fn rb_ctx_create(device_ids: *const c_int, n: c_int, status: *mut c_int) -> *mut rb_ctx;
     pub fn rb_ctx_destroy(ctx: *mut rb_ctx);
@@ -61,6 +71,13 @@ extern "C" {
     pub fn rb_trim_paf_begin(ctx: *mut rb_ctx, recs: *const rb_records, match_score: c_int, diff_score: c_int, indel_score: c_int, policy: c_int) -> c_int;
     pub fn rb_trim_paf_round(ctx: *mut rb_ctx, waiting: *mut c_int) -> c_int;
     pub fn rb_trim_paf_end(ctx: *mut rb_ctx, remove_contained: c_int, want: u32, out: *mut rb_lift_out, stats: *mut rb_stats_out) -> c_int;
+    /// paf.rs:62-78 Paf::from_file on the device: PAF text or BGZF bytes -> a resident batch (name table in `info`, library-owned)
+    pub fn rb_batch_upload_paf(ctx: *mut rb_ctx, data: *const u8, nbytes: u64, info: *mut rb_paf_info, status: *mut c_int) -> *mut rb_batch;
+    pub fn rb_batch_set_windows(ctx: *mut rb_ctx, b: *mut rb_batch, wins: *const rb_windows) -> c_int;
+    pub fn rb_batch_records(ctx: *mut rb_ctx, b: *mut rb_batch, with_cigar: c_int, out: *mut rb_records) -> c_int;
+    pub fn rb_batch_liftover(ctx: *mut rb_ctx, b: *mut rb_batch, policy: c_int, want: u32, with_stats: c_int, summary: *mut rb_summary) -> c_int;
+    pub fn rb_batch_download_lift(ctx: *mut rb_ctx, b: *mut rb_batch, want: u32, out: *mut rb_lift_out, stats: *mut rb_stats_out) -> c_int;
+    pub fn rb_batch_free(ctx: *mut rb_ctx, b: *mut rb_batch);
     // tuning (optional): slice threshold of rb_liftover, boundary driver
     pub fn rb_ctx_set_slicing(ctx: *mut rb_ctx, min_slice_bytes: u64) -> c_int;
     pub fn rb_ctx_set_lift_mode(ctx: *mut rb_ctx, mode: c_int) -> c_int;

@@ -34,7 +34,7 @@ def _sources(d, exts):
 def build_cuda(force=False, verbose=False):
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     srcs = _sources(CSRC, (".cu",))
-    deps = srcs + _sources(CSRC, (".cuh",)) + [os.path.join(ROOT, "include", "rbcuda.h"), os.path.abspath(__file__)]
+    deps = srcs + _sources(CSRC, (".cuh", ".hpp")) + [os.path.join(ROOT, "include", "rbcuda.h"), os.path.abspath(__file__)]
     if not force and not _newer(LIB, deps):
         return LIB
     extra = os.environ.get("RB_NVCC_DEFS", "").split()  # e.g. "-DRB_LIFT_THREADS=256 -DRB_LIFT_MINB=2" (tuning sweeps)
@@ -55,7 +55,8 @@ def build_host(force=False, verbose=False):
     if not srcs:
         return None
     deps = srcs + _sources(HOST, (".hpp", ".h")) + [os.path.join(ROOT, "include", "rbcuda.h"), os.path.abspath(__file__),
-                                                    os.path.join(CSRC, "f32_fmt.cuh"), os.path.join(CSRC, "rb_common.cuh")]  # (f32_fast.hpp includes them)
+                                                    os.path.join(CSRC, "f32_fmt.cuh"), os.path.join(CSRC, "rb_common.cuh"),  # (f32_fast.hpp includes them)
+                                                    os.path.join(CSRC, "name_intern.hpp")]
     gxx = shutil.which("g++") or "g++"
     common = ["-O2", "-std=c++17", "-fPIC", "-Wall", "-Wextra", "-pthread", "-I", os.path.join(ROOT, "include"), "-I", HOST]
     lib_srcs = [s for s in srcs if not s.endswith("rb_main.cpp")]

@@ -16,6 +16,7 @@ RB_OK = 0
 RB_ERR_NO_DEVICE, RB_ERR_CUDA, RB_ERR_BAD_ARG = -1, -2, -3
 RB_ERR_REF_CIGAR_PARSE, RB_ERR_REF_INTEGRITY, RB_ERR_REF_STRIP, RB_ERR_REF_INDEX = -4, -5, -6, -7
 RB_ERR_UNSUPPORTED, RB_ERR_OOM = -8, -9
+RB_ERR_REF_PAF_PARSE = -10
 REF_PANIC_CODES = (RB_ERR_REF_CIGAR_PARSE, RB_ERR_REF_INTEGRITY, RB_ERR_REF_STRIP, RB_ERR_REF_INDEX)
 POLICY_RIGHTMOST, POLICY_EARLY_EXIT = 0, 1
 WANT_TEXT, WANT_NUMERIC, WANT_QBED, WANT_STATS_TEXT = 1, 2, 4, 8
@@ -25,7 +26,7 @@ EXPORTS = [
     "rb_ctx_create", "rb_ctx_destroy", "rb_last_error", "rb_ctx_set_stream", "rb_ctx_set_profiling", "rb_ctx_set_lift_mode", "rb_ctx_set_slicing", "rb_ctx_kernel_times",
     "rb_liftover", "rb_stats", "rb_break_paf", "rb_invert", "rb_trim_paf", "rb_trim_paf_begin", "rb_trim_paf_round", "rb_trim_paf_end", "rb_batch_break", "rb_free_lift_out", "rb_free_stats_out", "rb_batch_upload", "rb_batch_liftover", "rb_batch_stats",
     "rb_batch_download_lift", "rb_batch_download_stats", "rb_batch_free", "rb_sort_windows", "rb_version", "rb_host_register",
-    "rb_host_unregister", "rb_is_bgzf", "rb_inflate_bgzf", "rb_free_text",
+    "rb_host_unregister", "rb_is_bgzf", "rb_inflate_bgzf", "rb_free_text", "rb_batch_upload_paf", "rb_batch_set_windows", "rb_batch_records",
 ]
 
 u8p, u32p, u64p, f32p = C.POINTER(C.c_uint8), C.POINTER(C.c_uint32), C.POINTER(C.c_uint64), C.POINTER(C.c_float)
@@ -56,6 +57,11 @@ class RbStatsOut(C.Structure):
 class RbSummary(C.Structure):
     _fields_ = [("n_ops", C.c_uint64), ("n_pairs", C.c_uint64), ("n_out", C.c_uint64), ("out_bytes", C.c_uint64),
                 ("cigar_bytes", C.c_uint64)]
+
+
+class RbPafInfo(C.Structure):
+    _fields_ = [("text_bytes", C.c_uint64), ("n_lines", C.c_uint64), ("skipped", C.c_uint64), ("n_rec", C.c_uint32), ("n_names", C.c_uint32),
+                ("names", u8p), ("names_off", u64p), ("cigar_bytes", C.c_uint64)]
 
 
 class RbKernelTime(C.Structure):
@@ -114,6 +120,10 @@ def load():
     lib.rb_is_bgzf.argtypes = [C.c_char_p, C.c_uint64]
     lib.rb_inflate_bgzf.argtypes = [C.c_void_p, C.c_char_p, C.c_uint64, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
     lib.rb_free_text.argtypes = [C.c_void_p, C.c_void_p]
+    lib.rb_batch_upload_paf.restype = C.c_void_p
+    lib.rb_batch_upload_paf.argtypes = [C.c_void_p, C.c_char_p, C.c_uint64, C.POINTER(RbPafInfo), C.POINTER(C.c_int)]
+    lib.rb_batch_set_windows.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(RbWindows)]
+    lib.rb_batch_records.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(RbRecords)]
     lib.rb_host_register.argtypes = [C.c_void_p, C.c_uint64]
     lib.rb_host_unregister.argtypes = [C.c_void_p]
     _lib = lib
@@ -382,6 +392,42 @@ class Context:
         if not b:
             raise RbError(st.value, self.lib.rb_last_error(self.h).decode())
         return b
+
+    def upload_paf(self, data: bytes):
+        """rb_batch_upload_paf: PAF text (or BGZF bytes) parsed on the device into a resident batch without windows.
+        Returns (batch, info); info["names"] is the batch's name table (list of bytes, ids by first appearance)."""
+        st, info = C.c_int(0), RbPafInfo()
+        b = self.lib.rb_batch_upload_paf(self.h, data, len(data), C.byref(info), C.byref(st))
+        if not b:
+            raise RbError(st.value, self.lib.rb_last_error(self.h).decode())
+        nn = int(info.n_names)
+        off = _np(info.names_off, nn + 1, np.uint64)
+        blob = C.string_at(info.names, int(off[-1])) if nn and int(off[-1]) else b""
+        names = [blob[int(off[i]):int(off[i + 1])] for i in range(nn)]
+        return b, dict(names=names, n_rec=int(info.n_rec), n_lines=int(info.n_lines), skipped=int(info.skipped),
+                       text_bytes=int(info.text_bytes), cigar_bytes=int(info.cigar_bytes))
+
+    def batch_set_windows(self, b, wins):
+        """rb_batch_set_windows: windows (t_id = ids of the batch's name table) for a batch uploaded without them."""
+        self._check(self.lib.rb_batch_set_windows(self.h, b, C.byref(wins.c) if wins is not None else None))
+
+    def batch_records(self, b, with_cigar=True) -> dict:
+        """rb_batch_records: the batch's records as numpy arrays named like Records' fields (names: list of bytes)."""
+        r = RbRecords()
+        self._check(self.lib.rb_batch_records(self.h, b, int(with_cigar), C.byref(r)))
+        n, nn = int(r.n_rec), int(r.n_names)
+        names_off = _np(r.names_off, nn + 1, np.uint64)
+        blob = C.string_at(r.names, int(names_off[-1])) if nn and int(names_off[-1]) else b""
+        res = dict(n_rec=n, cigar_off=_np(r.cigar_off, n + 1, np.uint64), strand=_np(r.strand, n, np.uint8),
+                   q_id=_np(r.q_id, n, np.uint32), t_id=_np(r.t_id, n, np.uint32),
+                   names=[blob[int(names_off[i]):int(names_off[i + 1])] for i in range(nn)])
+        for k in ("q_len", "q_st", "q_en", "t_len", "t_st", "t_en", "mapq"):
+            res[k] = _np(getattr(r, k), n, np.uint64)
+        if with_cigar:
+            nb = int(r.cigar_nbytes)
+            addr = C.cast(r.cigar, C.c_void_p).value  # (a buffer view: string_at takes a C int)
+            res["cigar"] = np.frombuffer((C.c_ubyte * nb).from_address(addr), dtype=np.uint8).copy() if nb else np.zeros(0, np.uint8)
+        return res
 
     def batch_liftover(self, b, policy=POLICY_RIGHTMOST, with_stats=True, want=WANT_TEXT | WANT_NUMERIC):
         s = RbSummary()

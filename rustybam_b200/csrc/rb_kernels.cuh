@@ -233,6 +233,31 @@ struct BgzfBlock {
     uint32_t clen, out_len, crc, pad;  // payload bytes, ISIZE and CRC-32 of the trailer
 };
 void launch_inflate_bgzf(const uint8_t* comp, const BgzfBlock* blk, uint32_t n_blk, uint8_t* out, unsigned long long* err, cudaStream_t s);
+// PAF text -> a resident batch (paf_parse_kernels.cu; the rules are paf_parse_core.cuh's).  Per-line columns of k_paf_fields:
+struct PafLineCols {
+    uint8_t* state;      // paf_parse_core.cuh LS_*
+    uint64_t* keep;      // 1 for a kept line (scan input: record index)
+    uint64_t* cg_len;    // cg payload bytes of a kept line (scan input: cigar_off)
+    uint64_t* name_len;  // q + t name bytes of a kept line (scan input: name bytes)
+    uint64_t* v;         // 7 x n_lines: q_len q_st q_en t_len t_st t_en mapq
+    uint8_t* strand;
+    uint64_t *qn_off, *tn_off, *cg_off;
+    uint32_t* qn_len;
+};
+uint64_t paf_chunks(uint64_t n);      // k_paf_lines_* blocks (64 KiB of text each): entries of chunk_cnt
+uint64_t paf_tiles(uint64_t n);       // 4 KiB whitespace tiles: entries of tile_ws
+uint64_t paf_scan_parts(uint64_t n);  // u64 per scanned column of the scan's block sums
+void launch_paf_lines_count(const uint8_t* text, uint64_t n, uint64_t* chunk_cnt, uint8_t* tile_ws, uint32_t* last_byte, cudaStream_t s);
+void launch_paf_lines_fill(const uint8_t* text, uint64_t n, const uint64_t* chunk_off, uint64_t* line_start, cudaStream_t s);
+// exclusive scans of nv <= 3 columns: out[v][0 .. n) and the total at out[v][n]; part = nv * paf_scan_parts(n) u64
+void launch_paf_scan(int nv, const uint64_t* const* in, uint64_t* const* out, uint64_t n, uint64_t* part, cudaStream_t s);
+void launch_paf_fields(const uint8_t* text, const uint64_t* line_start, uint64_t n_lines, const uint8_t* tile_ws, PafLineCols L,
+                       unsigned long long* first_panic, cudaStream_t s);
+void launch_paf_pack(const uint8_t* text, uint64_t n_lines, PafLineCols L, const uint64_t* rec_idx, const uint64_t* cg_pos,
+                     const uint64_t* name_pos, uint32_t n_rec, uint64_t* cols64, uint8_t* strand, uint64_t* cigar_off, uint32_t* rec_line,
+                     uint8_t* names, uint64_t* rec_name_off, uint32_t* rec_qlen, cudaStream_t s);
+void launch_paf_copy_cg(const uint8_t* text, uint32_t n_rec, const uint64_t* cigar_off, const uint32_t* rec_line, const uint64_t* cg_off,
+                        uint64_t cg_bytes, uint8_t* dst, cudaStream_t s);
 void launch_win_check(const uint32_t* t_id, const uint64_t* st, const uint64_t* en, const uint32_t* row, uint32_t n_win,
                       uint32_t n_names, uint32_t* flags, cudaStream_t s);
 // general path (unsorted / nested BED rows): the reference's cartesian product + overlap filter (liftover.rs:123-127)

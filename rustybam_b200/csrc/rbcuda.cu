@@ -13,11 +13,14 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <unordered_map>
 #include <vector>
 
 #include <sys/mman.h>
 
 #include "../../include/rbcuda.h"
+#include "name_intern.hpp"
+#include "paf_parse_core.cuh"
 #include "rb_kernels.cuh"
 #include "rec_core.cuh"
 #include "trim_rounds.hpp"
@@ -206,6 +209,10 @@ struct rb_batch {
     bool have_lift = false, have_stats = false, with_stats = false;
     uint32_t want = 0;
     uint64_t stats_n = 0;
+    // rb_batch_upload_paf: the name table handed out through rb_paf_info; rb_batch_records: its pinned copy of the records
+    std::vector<uint8_t> h_names;
+    std::vector<uint64_t> h_names_off;
+    PinBuf rec_out;
 };
 
 namespace {
@@ -576,6 +583,7 @@ void rb_batch_free(rb_ctx* ctx, rb_batch* b) {
     for (DevBuf* d : all) d->release();
     b->stage.release();
     b->wstage.release();
+    b->rec_out.release();
     delete b;
 }
 
@@ -675,6 +683,15 @@ struct RecSel {
     uint32_t at(uint32_t i) const { return idx ? idx[i] : r0 + i; }
 };
 
+// n_bytes of CIGAR text: the tokeniser's tiles and op bound; returns the bytes text_raw holds behind its front pad (the text, then
+// '0' up to the end of the last tile and 32 more)
+static size_t text_layout(rb_batch* b, uint64_t n_bytes) {
+    b->n_bytes = n_bytes;
+    b->n_tiles = b->n_bytes / TOK_TILE + 1;
+    b->ops_bound = b->n_bytes / 2 + 1;
+    return b->n_tiles * (size_t)TOK_TILE + 32;
+}
+
 static int upload_cigar(rb_ctx* ctx, rb_batch* b, const rb_records* R, RecSel sel) {
     cudaStream_t s = ctx->upload_on ? ctx->upload_on : ctx->stream;
     if (!R || (R->n_rec && (!R->cigar_off || !R->q_len || !R->q_st || !R->q_en || !R->t_len || !R->t_st || !R->t_en || !R->mapq ||
@@ -694,13 +711,11 @@ static int upload_cigar(rb_ctx* ctx, rb_batch* b, const rb_records* R, RecSel se
             return fail(ctx, RB_ERR_BAD_ARG, "cigar_off not monotone at record %u", r);
         b->h_cigar_off[i + 1] = b->h_cigar_off[i] + (R->cigar_off[r + 1] - R->cigar_off[r]);
     }
-    b->n_rec = n; b->n_names = R->n_names; b->n_bytes = b->h_cigar_off[n];
+    b->n_rec = n; b->n_names = R->n_names;
     b->rec_base = sel.idx ? 0 : sel.r0; b->byte_base = 0;
     b->invert = ctx->invert;
     b->have_lift = b->have_stats = false;
-    b->n_tiles = b->n_bytes / TOK_TILE + 1;
-    b->ops_bound = b->n_bytes / 2 + 1;
-    const size_t padded = b->n_tiles * (size_t)TOK_TILE + 32;
+    const size_t padded = text_layout(b, b->h_cigar_off[n]);
     CU(b->text_raw.ensure(TEXT_FRONT_PAD + padded));
     uint8_t* raw = b->text_raw.as<uint8_t>();
     CU(cudaMemsetAsync(raw, 0xFF, TEXT_FRONT_PAD, s));
@@ -846,21 +861,12 @@ static int upload_windows_end(rb_ctx* ctx, rb_batch* b, const rb_records* R, con
     return RB_OK;
 }
 
-// records [r0, r1) of R: numeric columns, names, emission order (small)
-static int upload_columns(rb_ctx* ctx, rb_batch* b, const rb_records* R, RecSel sel) {
-    cudaStream_t s = ctx->upload_on ? ctx->upload_on : ctx->stream;
-    const uint32_t n = sel.n;
-    for (uint32_t i = 0; i < n; i++) {
-        const uint32_t r = sel.at(i);
-        if (R->q_id[r] >= R->n_names || R->t_id[r] >= R->n_names) return fail(ctx, RB_ERR_BAD_ARG, "name id out of range at record %u", r);
-    }
+// device buffers for n records (columns, emission order, and what the kernels of every later call write); text_layout first
+static int ensure_rec_buffers(rb_ctx* ctx, rb_batch* b, uint32_t n) {
     CU(b->cigar_off.ensure((size_t)(n + 1) * 8));
     CU(b->cols64.ensure((size_t)n * 7 * 8 + 8));
     CU(b->strand.ensure(n + 8));
     CU(b->ids32.ensure((size_t)n * 2 * 4 + 8));
-    CU(b->names_off.ensure((size_t)(R->n_names + 1) * 8));
-    const uint64_t names_bytes = R->n_names ? R->names_off[R->n_names] : 0;
-    CU(b->names.ensure(names_bytes + 8));
     CU(b->rec_order.ensure((size_t)n * 4 + 8));
     CU(b->rec_rank.ensure((size_t)n * 4 + 8));
     CU(b->ops.ensure(b->ops_bound * 4 + 64));
@@ -882,6 +888,44 @@ static int upload_columns(rb_ctx* ctx, rb_batch* b, const rb_records* R, RecSel 
     CU(b->recs.ensure((size_t)n * sizeof(RecInfo) + 8));
     CU(b->pair_cnt.ensure((size_t)n * 4 + 8));
     CU(b->pair_off.ensure((size_t)(n + 1) * 8));
+    return RB_OK;
+}
+
+// emission order (liftover.rs:151-164): contigs by first appearance of t_name, records in file order inside (file_order: the
+// identity); order[k] = the record emitted k-th, rank = its inverse
+static void emission_ranks(const uint32_t* tid, uint32_t n, uint32_t n_names, bool file_order, uint32_t* order, uint32_t* rank) {
+    std::vector<int64_t> first(n_names, -1);
+    std::vector<uint32_t> cnt;
+    std::vector<uint32_t> grp(n);
+    for (uint32_t i = 0; i < n; i++) {
+        int64_t& f = first[tid[i]];
+        if (f < 0) { f = (int64_t)cnt.size(); cnt.push_back(0); }
+        grp[i] = (uint32_t)f;
+        cnt[grp[i]]++;
+    }
+    std::vector<uint32_t> start(cnt.size() + 1, 0);
+    for (size_t g = 0; g < cnt.size(); g++) start[g + 1] = start[g] + cnt[g];
+    for (uint32_t i = 0; i < n; i++) {
+        const uint32_t k = file_order ? i : start[grp[i]]++;
+        order[k] = i;
+        rank[i] = k;
+    }
+}
+
+// records [r0, r1) of R: numeric columns, names, emission order (small)
+static int upload_columns(rb_ctx* ctx, rb_batch* b, const rb_records* R, RecSel sel) {
+    cudaStream_t s = ctx->upload_on ? ctx->upload_on : ctx->stream;
+    const uint32_t n = sel.n;
+    for (uint32_t i = 0; i < n; i++) {
+        const uint32_t r = sel.at(i);
+        if (R->q_id[r] >= R->n_names || R->t_id[r] >= R->n_names) return fail(ctx, RB_ERR_BAD_ARG, "name id out of range at record %u", r);
+    }
+    int rc = ensure_rec_buffers(ctx, b, n);
+    if (rc != RB_OK) return rc;
+    CU(b->names_off.ensure((size_t)(R->n_names + 1) * 8));
+    const uint64_t names_bytes = R->n_names ? R->names_off[R->n_names] : 0;
+    CU(b->names.ensure(names_bytes + 8));
+
 
     // gather every small column into the batch's pinned staging area, then one asynchronous copy each
     const uint64_t* cols[7] = {R->q_len, R->q_st, R->q_en, R->t_len, R->t_st, R->t_en, R->mapq};
@@ -933,25 +977,7 @@ static int upload_columns(rb_ctx* ctx, rb_batch* b, const rb_records* R, RecSel 
     uint32_t* s_order = reinterpret_cast<uint32_t*>(sp + o_order);
     uint32_t* s_rank = reinterpret_cast<uint32_t*>(sp + o_rank);
 
-    // emission order (liftover.rs:151-164): contigs by first appearance of t_name, records in file order inside
-    {
-        std::vector<int64_t> first(R->n_names, -1);
-        std::vector<uint32_t> cnt;
-        std::vector<uint32_t> grp(n);
-        for (uint32_t i = 0; i < n; i++) {
-            int64_t& f = first[h_tid[i]];
-            if (f < 0) { f = (int64_t)cnt.size(); cnt.push_back(0); }
-            grp[i] = (uint32_t)f;
-            cnt[grp[i]]++;
-        }
-        std::vector<uint32_t> start(cnt.size() + 1, 0);
-        for (size_t g = 0; g < cnt.size(); g++) start[g + 1] = start[g] + cnt[g];
-        for (uint32_t i = 0; i < n; i++) {
-            const uint32_t k = b->file_order ? i : start[grp[i]]++;
-            s_order[k] = i;
-            s_rank[i] = k;
-        }
-    }
+    emission_ranks(h_tid, n, R->n_names, b->file_order, s_order, s_rank);
     if (n) {
         CU(cudaMemcpyAsync(b->rec_order.p, s_order, (size_t)n * 4, cudaMemcpyHostToDevice, s));
         CU(cudaMemcpyAsync(b->rec_rank.p, s_rank, (size_t)n * 4, cudaMemcpyHostToDevice, s));
@@ -1560,27 +1586,22 @@ static bool bgzf_blocks(const uint8_t* p, uint64_t n, std::vector<BgzfBlock>& bl
 int rb_is_bgzf(const uint8_t* data, uint64_t nbytes) {
     return data && nbytes >= 18 && data[0] == 0x1f && data[1] == 0x8b && data[2] == 8 && (data[3] & 4) && data[12] == 'B' && data[13] == 'C';
 }
-int rb_inflate_bgzf(rb_ctx* ctx, const uint8_t* bgzf, uint64_t nbytes, uint8_t** text, uint64_t* text_nbytes) {
-    if (!ctx) return RB_ERR_NO_DEVICE;
-    if (!text || !text_nbytes || (!bgzf && nbytes)) return fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: null argument");
-    *text = nullptr; *text_nbytes = 0;
+// The inflate step: block table, compressed bytes -> HBM, k_inflate_bgzf, CRC-32 / ISIZE verdict.  On RB_OK `out` holds the
+// `total` inflated bytes followed by `pad` bytes of head-room (the stream has been synchronised).
+static int inflate_to_device(rb_ctx* ctx, const uint8_t* bgzf, uint64_t nbytes, DevBuf& out, uint64_t& total, size_t pad) {
     std::vector<BgzfBlock> blocks;
-    uint64_t total = 0;
+    total = 0;
     if (!bgzf_blocks(bgzf, nbytes, blocks, total)) return fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: not a well-formed series of BGZF blocks");
     if (blocks.size() > 0xFFFFFFF0ull) return fail(ctx, RB_ERR_UNSUPPORTED, "rb_inflate_bgzf: more than 2^32 blocks");
-    cudaSetDevice(ctx->device);
+    if (total == 0) return out.ensure(pad + 64) == cudaSuccess ? RB_OK : fail(ctx, RB_ERR_OOM, "rb_inflate_bgzf: device memory");
     cudaStream_t s = ctx->stream;
-    PinnedBlock* blk = pinned_get(ctx, (size_t)total + 64);
-    if (!blk) return fail(ctx, RB_ERR_OOM, "rb_inflate_bgzf: %llu bytes of pinned host memory", (unsigned long long)total);
-    auto bail = [&](int rc) { blk->in_use = false; return rc; };
-    if (total == 0) { *text = static_cast<uint8_t*>(blk->p); return RB_OK; }
-    DevBuf d_comp, d_blk, d_out, d_err;
-    auto release = [&] { d_comp.release(); d_blk.release(); d_out.release(); d_err.release(); };
+    DevBuf d_comp, d_blk, d_err;
+    auto release = [&] { d_comp.release(); d_blk.release(); d_err.release(); };
     if (d_comp.ensure(nbytes + 64) != cudaSuccess || d_blk.ensure(blocks.size() * sizeof(BgzfBlock)) != cudaSuccess ||
-        d_out.ensure(total + 64) != cudaSuccess || d_err.ensure(8) != cudaSuccess) {
+        out.ensure(total + pad + 64) != cudaSuccess || d_err.ensure(8) != cudaSuccess) {
         (void)cudaGetLastError();
         release();
-        return bail(fail(ctx, RB_ERR_OOM, "rb_inflate_bgzf: device memory for %llu + %llu bytes", (unsigned long long)nbytes, (unsigned long long)total));
+        return fail(ctx, RB_ERR_OOM, "rb_inflate_bgzf: device memory for %llu + %llu bytes", (unsigned long long)nbytes, (unsigned long long)total);
     }
     unsigned long long h_err = ~0ull;
     cudaError_t e = h2d_copy(d_comp.p, bgzf, nbytes, s);
@@ -1588,17 +1609,42 @@ int rb_inflate_bgzf(rb_ctx* ctx, const uint8_t* bgzf, uint64_t nbytes, uint8_t**
     if (e == cudaSuccess) e = cudaMemsetAsync(d_err.p, 0xFF, 8, s);
     if (e == cudaSuccess) {
         KScope k(ctx, "k_inflate_bgzf");
-        launch_inflate_bgzf(d_comp.as<uint8_t>(), d_blk.as<BgzfBlock>(), (uint32_t)blocks.size(), d_out.as<uint8_t>(), d_err.as<unsigned long long>(), s);
+        launch_inflate_bgzf(d_comp.as<uint8_t>(), d_blk.as<BgzfBlock>(), (uint32_t)blocks.size(), out.as<uint8_t>(), d_err.as<unsigned long long>(), s);
         e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaMemcpyAsync(&h_err, d_err.p, 8, cudaMemcpyDeviceToHost, s);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(blk->p, d_out.p, total, cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
     flush_times(ctx);
     release();
-    if (e != cudaSuccess) { (void)cudaGetLastError(); return bail(fail(ctx, RB_ERR_CUDA, "rb_inflate_bgzf: %s", cudaGetErrorString(e))); }
+    if (e != cudaSuccess) { (void)cudaGetLastError(); return fail(ctx, RB_ERR_CUDA, "rb_inflate_bgzf: %s", cudaGetErrorString(e)); }
     if (h_err != ~0ull)
-        return bail(fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: corrupt DEFLATE data in block %llu (code %u)", (unsigned long long)(h_err >> 8), (unsigned)(h_err & 0xFF)));
+        return fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: corrupt DEFLATE data in block %llu (code %u)", (unsigned long long)(h_err >> 8), (unsigned)(h_err & 0xFF));
+    return RB_OK;
+}
+int rb_inflate_bgzf(rb_ctx* ctx, const uint8_t* bgzf, uint64_t nbytes, uint8_t** text, uint64_t* text_nbytes) {
+    if (!ctx) return RB_ERR_NO_DEVICE;
+    if (!text || !text_nbytes || (!bgzf && nbytes)) return fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: null argument");
+    *text = nullptr; *text_nbytes = 0;
+    cudaSetDevice(ctx->device);
+    DevBuf d_out;
+    uint64_t total = 0;
+    int rc = inflate_to_device(ctx, bgzf, nbytes, d_out, total, 0);
+    PinnedBlock* blk = nullptr;
+    if (rc == RB_OK) {
+        blk = pinned_get(ctx, (size_t)total + 64);
+        if (!blk) rc = fail(ctx, RB_ERR_OOM, "rb_inflate_bgzf: %llu bytes of pinned host memory", (unsigned long long)total);
+    }
+    if (rc == RB_OK && total) {
+        cudaError_t e = cudaMemcpyAsync(blk->p, d_out.p, total, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();
+            blk->in_use = false;
+            rc = fail(ctx, RB_ERR_CUDA, "rb_inflate_bgzf: %s", cudaGetErrorString(e));
+        }
+    }
+    d_out.release();
+    if (rc != RB_OK) return rc;
     *text = static_cast<uint8_t*>(blk->p);
     *text_nbytes = total;
     return RB_OK;
@@ -1607,6 +1653,284 @@ void rb_free_text(rb_ctx* ctx, uint8_t* text) {
     if (!ctx || !text) return;
     for (PinnedBlock* b : ctx->pinned)
         if (b->p == text) b->in_use = false;
+}
+
+// ---- PAF text on the device (rb_batch_upload_paf; kernels in paf_parse_kernels.cu) -----------------------------------------
+// text -> HBM (or BGZF -> inflated in HBM) -> line starts -> per-line fields -> scans -> the batch's columns and CIGAR text, byte
+// for byte what upload_cigar + upload_columns build from the host reader's records.  The name bytes of the records come back and
+// are interned here with the host reader's loop (name_intern.hpp); ids, names and the emission order go up again.  The text and
+// every per-line table are freed before the call returns: the peak is about twice the text, during the call only.
+struct DevScratch {  // device buffers of one call, released on every way out
+    std::vector<DevBuf*> bufs;
+    ~DevScratch() { for (DevBuf* d : bufs) d->release(); }
+};
+
+static int paf_upload_into(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64_t nbytes, rb_paf_info* info) {
+    cudaStream_t s = ctx->stream;
+    uint32_t* sc = ctx->scalars.as<uint32_t>();
+    volatile uint64_t* hs = reinterpret_cast<volatile uint64_t*>(ctx->h_scalars);
+    DevBuf d_text, d_chunk, d_tws, d_part, d_lines, d_cols, d_rec;
+    DevScratch scratch{{&d_text, &d_chunk, &d_tws, &d_part, &d_lines, &d_cols, &d_rec}};
+    constexpr size_t TEXT_PAD = 4096;  // (16-byte loads of the last bytes)
+    uint64_t n = 0;
+    if (rb_is_bgzf(data, nbytes)) {
+        const int rc = inflate_to_device(ctx, data, nbytes, d_text, n, TEXT_PAD);
+        if (rc != RB_OK) return rc;
+    } else if (nbytes >= 2 && data[0] == 0x1f && data[1] == 0x8b) {
+        return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_upload_paf: a plain gzip stream (not BGZF); inflate it first");
+    } else {
+        n = nbytes;
+        CU(d_text.ensure(n + TEXT_PAD));
+        if (n) CU(h2d_copy(d_text.p, data, n, s));
+    }
+    const uint8_t* text = d_text.as<uint8_t>();
+    // 1. line starts: newline counts per 64 KiB, their scan, the starts; a last line without a terminator ends at n + 1 - 1
+    uint64_t n_lines = 0;
+    if (n) {
+        const uint64_t nc = paf_chunks(n);
+        CU(d_chunk.ensure((2 * nc + 2) * 8));
+        CU(d_tws.ensure(paf_tiles(n) + 64));
+        CU(d_part.ensure(paf_scan_parts(nc) * 8));
+        uint64_t* cnt = d_chunk.as<uint64_t>();
+        uint64_t* off = cnt + nc;
+        CU(cudaMemsetAsync(sc + SC_MISC, 0, 4, s));
+        {
+            KScope k(ctx, "k_paf_lines_count");
+            launch_paf_lines_count(text, n, cnt, d_tws.as<uint8_t>(), sc + SC_MISC, s);
+        }
+        {
+            KScope k(ctx, "k_paf_scan");
+            const uint64_t* in[1] = {cnt};
+            uint64_t* out[1] = {off};
+            launch_paf_scan(1, in, out, nc, d_part.as<uint64_t>(), s);
+        }
+        Publisher(ctx).u64(0, off + nc).u32(1, sc + SC_MISC).go(s);
+        CU(cudaStreamSynchronize(s));
+        n_lines = hs[0] + ((uint8_t)hs[1] != '\n' ? 1 : 0);
+        if (n_lines > 0xFFFFFFFFull) return fail(ctx, RB_ERR_REF_PAF_PARSE, "more than 2^32 lines");
+        CU(d_lines.ensure((n_lines + 2) * 8));
+        {
+            KScope k(ctx, "k_paf_lines_fill");
+            launch_paf_lines_fill(text, n, off, d_lines.as<uint64_t>(), s);
+        }
+        if (n_lines > hs[0]) {
+            const uint64_t end = n + 1;  // (pageable source: the copy is staged before the call returns)
+            CU(cudaMemcpyAsync(d_lines.as<uint64_t>() + n_lines, &end, 8, cudaMemcpyHostToDevice, s));
+        }
+    }
+    // 2. per-line fields, first panic, scans of (kept, cg bytes, name bytes)
+    const uint64_t nl = n_lines;
+    size_t o = 0;
+    auto carve = [&](size_t bytes) { const size_t at = o; o += align_up(bytes, 256); return at; };
+    const size_t o_state = carve(nl + 8), o_keep = carve(nl * 8), o_cgl = carve(nl * 8), o_nml = carve(nl * 8), o_v = carve(nl * 56),
+                 o_strand = carve(nl + 8), o_qo = carve(nl * 8), o_to = carve(nl * 8), o_co = carve(nl * 8), o_ql = carve(nl * 4),
+                 o_s0 = carve((nl + 1) * 8), o_s1 = carve((nl + 1) * 8), o_s2 = carve((nl + 1) * 8);
+    CU(d_cols.ensure(o + 256));
+    CU(d_part.ensure(3 * paf_scan_parts(nl) * 8));
+    uint8_t* cb = d_cols.as<uint8_t>();
+    PafLineCols L{};
+    L.state = cb + o_state; L.keep = reinterpret_cast<uint64_t*>(cb + o_keep); L.cg_len = reinterpret_cast<uint64_t*>(cb + o_cgl);
+    L.name_len = reinterpret_cast<uint64_t*>(cb + o_nml); L.v = reinterpret_cast<uint64_t*>(cb + o_v); L.strand = cb + o_strand;
+    L.qn_off = reinterpret_cast<uint64_t*>(cb + o_qo); L.tn_off = reinterpret_cast<uint64_t*>(cb + o_to);
+    L.cg_off = reinterpret_cast<uint64_t*>(cb + o_co); L.qn_len = reinterpret_cast<uint32_t*>(cb + o_ql);
+    uint64_t* rec_idx = reinterpret_cast<uint64_t*>(cb + o_s0);
+    uint64_t* cg_pos = reinterpret_cast<uint64_t*>(cb + o_s1);
+    uint64_t* name_pos = reinterpret_cast<uint64_t*>(cb + o_s2);
+    CU(cudaMemsetAsync(sc + SC_ERR_TOK, 0xFF, 8, s));
+    {
+        KScope k(ctx, "k_paf_fields");
+        launch_paf_fields(text, d_lines.as<uint64_t>(), nl, d_tws.as<uint8_t>(), L, reinterpret_cast<unsigned long long*>(sc + SC_ERR_TOK), s);
+    }
+    {
+        KScope k(ctx, "k_paf_scan");
+        const uint64_t* in[3] = {L.keep, L.cg_len, L.name_len};
+        uint64_t* out[3] = {rec_idx, cg_pos, name_pos};
+        launch_paf_scan(3, in, out, nl, d_part.as<uint64_t>(), s);
+    }
+    Publisher(ctx).u64(0, sc + SC_ERR_TOK).u64(1, rec_idx + nl).u64(2, cg_pos + nl).u64(3, name_pos + nl).go(s);
+    CU(cudaStreamSynchronize(s));
+    CU(cudaGetLastError());
+    const uint64_t panic = hs[0], n_rec64 = hs[1], cg_bytes = hs[2], name_bytes = hs[3];
+    if (panic != ~0ull) {
+        flush_times(ctx);
+        const unsigned long long line = (panic >> 8) + 1;
+        switch ((uint32_t)(panic & 0xFF)) {
+            case rbpp::LS_FEW_COLUMNS: return fail(ctx, RB_ERR_REF_PAF_PARSE, "line %llu: assertion failed: t.len() >= 12", line);
+            case rbpp::LS_BAD_TAG: return fail(ctx, RB_ERR_REF_PAF_PARSE, "line %llu: assertion failed: PAF_TAG.is_match(token)", line);
+            default: return fail(ctx, RB_ERR_REF_CIGAR_PARSE, "line %llu: Unable to parse cigar string.", line);
+        }
+    }
+    const uint32_t n_rec = (uint32_t)n_rec64;
+    // 3. the batch's columns and CIGAR text
+    b->n_rec = n_rec;
+    b->rec_base = 0; b->byte_base = 0;
+    b->invert = false;
+    b->have_lift = b->have_stats = false;
+    const size_t padded = text_layout(b, cg_bytes);
+    CU(b->text_raw.ensure(TEXT_FRONT_PAD + padded));
+    int rc = ensure_rec_buffers(ctx, b, n_rec);
+    if (rc != RB_OK) return rc;
+    const size_t r_line = 0, r_noff = align_up((size_t)n_rec * 4 + 8, 256), r_qlen = r_noff + align_up(((size_t)n_rec + 1) * 8, 256),
+                 r_names = r_qlen + align_up((size_t)n_rec * 4 + 8, 256);
+    CU(d_rec.ensure(r_names + name_bytes + 64));
+    uint8_t* rb = d_rec.as<uint8_t>();
+    {
+        KScope k(ctx, "k_paf_pack");
+        launch_paf_pack(text, nl, L, rec_idx, cg_pos, name_pos, n_rec, b->cols64.as<uint64_t>(), b->strand.as<uint8_t>(),
+                        b->cigar_off.as<uint64_t>(), reinterpret_cast<uint32_t*>(rb + r_line), rb + r_names,
+                        reinterpret_cast<uint64_t*>(rb + r_noff), reinterpret_cast<uint32_t*>(rb + r_qlen), s);
+    }
+    uint8_t* raw = b->text_raw.as<uint8_t>();
+    CU(cudaMemsetAsync(raw, 0xFF, TEXT_FRONT_PAD, s));
+    {
+        KScope k(ctx, "k_paf_copy_cg");
+        launch_paf_copy_cg(text, n_rec, b->cigar_off.as<uint64_t>(), reinterpret_cast<const uint32_t*>(rb + r_line), L.cg_off, cg_bytes,
+                           raw + TEXT_FRONT_PAD, s);
+    }
+    const uint64_t tail0 = align_up(cg_bytes, 16);  // (k_paf_copy_cg wrote '0' up to here)
+    CU(cudaMemsetAsync(raw + TEXT_FRONT_PAD + tail0, '0', padded - tail0, s));
+    // 4. names back to the host, interned, ids / names / emission order up again
+    b->h_cigar_off.resize((size_t)n_rec + 1);
+    std::vector<uint64_t> noff((size_t)n_rec + 1);
+    std::vector<uint32_t> qlen(n_rec);
+    std::vector<char> nbytes_h(name_bytes + 1);
+    CU(cudaMemcpyAsync(b->h_cigar_off.data(), b->cigar_off.p, ((size_t)n_rec + 1) * 8, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(noff.data(), rb + r_noff, ((size_t)n_rec + 1) * 8, cudaMemcpyDeviceToHost, s));
+    if (n_rec) CU(cudaMemcpyAsync(qlen.data(), rb + r_qlen, (size_t)n_rec * 4, cudaMemcpyDeviceToHost, s));
+    if (name_bytes) CU(cudaMemcpyAsync(nbytes_h.data(), rb + r_names, name_bytes, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    flush_times(ctx);
+    d_text.release(); d_cols.release(); d_lines.release();  // (before the host work: the text is not needed any more)
+    const char* nb = nbytes_h.data();
+    std::unordered_map<std::string, uint32_t> index;
+    b->h_names.clear();
+    b->h_names_off.assign(1, 0);
+    std::vector<uint32_t> h_ids((size_t)n_rec * 2);
+    rbn::intern_record_names(
+        n_rec, [&](size_t r) { return std::make_pair(nb + noff[r], (size_t)qlen[r]); },
+        [&](size_t r) { return std::make_pair(nb + noff[r] + qlen[r], (size_t)(noff[r + 1] - noff[r] - qlen[r])); },
+        [&](const char* p, size_t len) {
+            const auto ins = index.emplace(std::string(p, len), (uint32_t)(b->h_names_off.size() - 1));
+            if (ins.second) {
+                b->h_names.insert(b->h_names.end(), p, p + len);
+                b->h_names_off.push_back(b->h_names.size());
+            }
+            return ins.first->second;
+        },
+        h_ids.data(), h_ids.data() + n_rec);
+    const uint32_t n_names = (uint32_t)(b->h_names_off.size() - 1);
+    const uint64_t tbl_bytes = b->h_names.size();
+    b->n_names = n_names;
+    CU(b->names_off.ensure(((size_t)n_names + 1) * 8));
+    CU(b->names.ensure(tbl_bytes + 8));
+    const size_t s_ids = 0, s_noff = align_up((size_t)n_rec * 8, 64), s_names = s_noff + align_up(((size_t)n_names + 1) * 8, 64),
+                 s_order = s_names + align_up(tbl_bytes + 1, 64), s_rank = s_order + align_up((size_t)n_rec * 4, 64),
+                 s_end = s_rank + align_up((size_t)n_rec * 4, 64);
+    CU(b->stage.ensure(s_end));
+    uint8_t* sp = b->stage.p;
+    memcpy(sp + s_ids, h_ids.data(), (size_t)n_rec * 8);
+    memcpy(sp + s_noff, b->h_names_off.data(), ((size_t)n_names + 1) * 8);
+    if (tbl_bytes) memcpy(sp + s_names, b->h_names.data(), tbl_bytes);
+    emission_ranks(h_ids.data() + n_rec, n_rec, n_names, b->file_order, reinterpret_cast<uint32_t*>(sp + s_order),
+                   reinterpret_cast<uint32_t*>(sp + s_rank));
+    if (n_rec) {
+        CU(cudaMemcpyAsync(b->ids32.p, sp + s_ids, (size_t)n_rec * 8, cudaMemcpyHostToDevice, s));
+        CU(cudaMemcpyAsync(b->rec_order.p, sp + s_order, (size_t)n_rec * 4, cudaMemcpyHostToDevice, s));
+        CU(cudaMemcpyAsync(b->rec_rank.p, sp + s_rank, (size_t)n_rec * 4, cudaMemcpyHostToDevice, s));
+    }
+    CU(cudaMemcpyAsync(b->names_off.p, sp + s_noff, ((size_t)n_names + 1) * 8, cudaMemcpyHostToDevice, s));
+    if (tbl_bytes) CU(cudaMemcpyAsync(b->names.p, sp + s_names, tbl_bytes, cudaMemcpyHostToDevice, s));
+    b->busy = true;
+    b->sum = rb_summary{};
+    b->sum.cigar_bytes = b->n_bytes;
+    if (info) {
+        info->text_bytes = n; info->n_lines = nl; info->skipped = nl - n_rec;
+        info->n_rec = n_rec; info->n_names = n_names;
+        info->names = b->h_names.empty() ? nullptr : b->h_names.data();
+        info->names_off = b->h_names_off.data();
+        info->cigar_bytes = cg_bytes;
+    }
+    return RB_OK;
+}
+
+rb_batch* rb_batch_upload_paf(rb_ctx* ctx, const uint8_t* data, uint64_t nbytes, rb_paf_info* info, int* status) {
+    auto set = [&](int s) { if (status) *status = s; };
+    if (!ctx) { set(RB_ERR_NO_DEVICE); return nullptr; }
+    if (!data && nbytes) { set(fail(ctx, RB_ERR_BAD_ARG, "rb_batch_upload_paf: null data")); return nullptr; }
+    if (info) memset(info, 0, sizeof *info);
+    cudaSetDevice(ctx->device);
+    rb_batch* b = new rb_batch();
+    int rc = paf_upload_into(ctx, b, data, nbytes, info);
+    if (rc == RB_OK && cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+        (void)cudaGetLastError();
+        rc = fail(ctx, RB_ERR_CUDA, "upload failed");
+    }
+    if (rc != RB_OK) cudaStreamSynchronize(ctx->stream);
+    b->busy = false;
+    set(rc);
+    if (rc != RB_OK) {
+        if (info) memset(info, 0, sizeof *info);
+        rb_batch_free(ctx, b);
+        return nullptr;
+    }
+    return b;
+}
+
+int rb_batch_set_windows(rb_ctx* ctx, rb_batch* b, const rb_windows* wins) {
+    if (!ctx || !b) return RB_ERR_BAD_ARG;
+    if (b->wsrc) return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_set_windows: not on a slice");
+    cudaSetDevice(ctx->device);
+    rb_records R{};
+    R.n_names = b->n_names;
+    b->have_lift = false;
+    int rc = upload_windows_begin(ctx, b, &R, wins);
+    if (rc == RB_OK) rc = upload_windows_end(ctx, b, &R, wins);
+    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess && rc == RB_OK) {  // the caller may reuse its tables after this call
+        (void)cudaGetLastError();
+        rc = fail(ctx, RB_ERR_CUDA, "window upload failed");
+    }
+    b->busy = false;
+    if (rc != RB_OK) b->n_win = 0;
+    return rc;
+}
+
+int rb_batch_records(rb_ctx* ctx, rb_batch* b, int with_cigar, rb_records* out) {
+    if (!ctx || !b || !out) return RB_ERR_BAD_ARG;
+    cudaSetDevice(ctx->device);
+    cudaStream_t s = ctx->stream;
+    memset(out, 0, sizeof *out);
+    const size_t n = b->n_rec, nn = b->n_names;
+    uint64_t names_bytes = 0;
+    CU(cudaMemcpyAsync(&names_bytes, b->names_off.as<uint64_t>() + nn, 8, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    const uint64_t cg = with_cigar ? b->n_bytes : 0;
+    const size_t o_off = 0, o_cols = align_up((n + 1) * 8, 64), o_ids = o_cols + align_up(n * 56, 64), o_strand = o_ids + align_up(n * 8, 64),
+                 o_noff = o_strand + align_up(n + 1, 64), o_names = o_noff + align_up((nn + 1) * 8, 64),
+                 o_cigar = o_names + align_up(names_bytes + 1, 64), o_end = o_cigar + align_up(cg + 1, 64);
+    if (b->busy) { CU(cudaStreamSynchronize(s)); b->busy = false; }  // (the staging area may still feed an upload)
+    CU(b->rec_out.ensure(o_end));
+    uint8_t* p = b->rec_out.p;
+    CU(cudaMemcpyAsync(p + o_off, b->cigar_off.p, (n + 1) * 8, cudaMemcpyDeviceToHost, s));
+    if (n) {
+        CU(cudaMemcpyAsync(p + o_cols, b->cols64.p, n * 56, cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(p + o_ids, b->ids32.p, n * 8, cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(p + o_strand, b->strand.p, n, cudaMemcpyDeviceToHost, s));
+    }
+    CU(cudaMemcpyAsync(p + o_noff, b->names_off.p, (nn + 1) * 8, cudaMemcpyDeviceToHost, s));
+    if (names_bytes) CU(cudaMemcpyAsync(p + o_names, b->names.p, names_bytes, cudaMemcpyDeviceToHost, s));
+    if (cg) CU(cudaMemcpyAsync(p + o_cigar, b->text_raw.as<uint8_t>() + TEXT_FRONT_PAD, cg, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    const uint64_t* cols = reinterpret_cast<const uint64_t*>(p + o_cols);
+    out->n_rec = (uint32_t)n;
+    out->cigar = with_cigar ? p + o_cigar : nullptr;
+    out->cigar_nbytes = cg;
+    out->cigar_off = reinterpret_cast<const uint64_t*>(p + o_off);
+    out->q_len = cols; out->q_st = cols + n; out->q_en = cols + 2 * n; out->t_len = cols + 3 * n; out->t_st = cols + 4 * n;
+    out->t_en = cols + 5 * n; out->mapq = cols + 6 * n;
+    out->strand = p + o_strand;
+    out->q_id = reinterpret_cast<const uint32_t*>(p + o_ids); out->t_id = out->q_id + n;
+    out->names = p + o_names; out->names_off = reinterpret_cast<const uint64_t*>(p + o_noff); out->n_names = (uint32_t)nn;
+    return RB_OK;
 }
 
 // ---- rb_liftover in slices -----------------------------------------------------------------------

@@ -17,6 +17,11 @@
 #include <cstring>
 #include <string>
 
+#include <fcntl.h>
+#include <sys/mman.h>
+#include <sys/stat.h>
+#include <unistd.h>
+
 #include "rbhost.hpp"
 
 static int usage() {
@@ -106,9 +111,97 @@ int main(int argc, char** argv) {
         }
         return rbh::Paf::from_file(path);
     };
+    // RB_DEVICE_PARSE=1: `rb liftover` (plain, --stats, --largest) and `rb stats --paf` on one GPU hand the file's bytes to
+    // rb_batch_upload_paf — lines are split and parsed on the device — instead of parsing them on the host.  A plain file is mapped,
+    // a .bgz goes as it is (inflated on the device), a plain .gz and stdin are inflated / read by rbh::read_all first.
+    const char* dp = getenv("RB_DEVICE_PARSE");
+    const bool device_parse = dp && dp[0] == '1' && n_gpus == 1 && !qbed && (cmd == "liftover" || cmd == "stats");
+    rb_batch* batch = nullptr;
+    rb_paf_info info{};
+    auto upload_paf = [&](const std::string& path) {
+        auto ends_with = [&](const char* suf) { const size_t n = strlen(suf); return path.size() >= n && path.compare(path.size() - n, n, suf) == 0; };
+        std::string owned;
+        const uint8_t* data = nullptr;
+        size_t n = 0;
+        void* map = nullptr;
+        if (path != "-" && !ends_with(".gz") && !ends_with(".bgz")) {
+            const int fd = ::open(path.c_str(), O_RDONLY);
+            if (fd < 0) throw rbh::Panic("Error: cannot read input file " + path);
+            struct stat st;
+            if (fstat(fd, &st) == 0 && S_ISREG(st.st_mode) && st.st_size > 0) {
+                map = mmap(nullptr, (size_t)st.st_size, PROT_READ, MAP_PRIVATE, fd, 0);
+                if (map == MAP_FAILED) map = nullptr;
+                else { data = static_cast<const uint8_t*>(map); n = (size_t)st.st_size; }
+            }
+            ::close(fd);
+            if (!map) owned = rbh::read_raw(path);
+        } else if (path != "-") {
+            owned = rbh::read_raw(path);
+            if (!rb_is_bgzf(reinterpret_cast<const uint8_t*>(owned.data()), owned.size())) owned = rbh::read_all(path);
+        } else {
+            owned = rbh::read_all(path);
+        }
+        if (!map) { data = reinterpret_cast<const uint8_t*>(owned.data()); n = owned.size(); }
+        int st = 0;
+        batch = rb_batch_upload_paf(ctx, data, n, &info, &st);
+        if (map) munmap(map, n);
+        if (!batch) return st;
+        if (info.skipped) fprintf(stderr, "\nUnable to parse %zu PAF record(s). Skipped.\n", (size_t)info.skipped);
+        return (int)RB_OK;
+    };
     int rc = 0;
     try {
-        if (cmd == "stats") {
+        if (device_parse && cmd == "stats") {
+            fputs(rbh::stats_header(qbed).c_str(), stdout);  // printed before the input is read (main.rs:51)
+            fflush(stdout);
+            rc = upload_paf(input);
+            mark("device_parse_paf");
+            rb_stats_out st{};
+            rb_records recs{};
+            if (rc == RB_OK) rc = rb_batch_stats(ctx, batch, nullptr);
+            if (rc == RB_OK) rc = rb_batch_download_stats(ctx, batch, &st);
+            if (rc == RB_OK) rc = rb_batch_records(ctx, batch, 0, &recs);
+            mark("rb_batch_stats");
+            if (rc == RB_OK) {
+                rbh::write_stats_rows(stdout, recs, st, qbed);
+                fflush(stdout);
+                mark("format_write");
+                rb_free_stats_out(ctx, &st);
+            }
+        } else if (device_parse) {
+            if (bed.empty()) return usage();
+            if (stats_rows && largest) return usage();
+            const std::string bed_text = rbh::read_all(bed);
+            mark("read_bed");
+            rc = upload_paf(input);
+            mark("device_parse_paf");
+            if (rc == RB_OK) {
+                if (stats_rows) { fputs(rbh::stats_header(false).c_str(), stdout); fflush(stdout); }  // main.rs:51
+                rbh::Paf names;  // the batch's name table, interned in id order: BED rows get the batch's ids
+                for (uint32_t i = 0; i < info.n_names; i++)
+                    names.name_id(std::string(reinterpret_cast<const char*>(info.names) + info.names_off[i], (size_t)(info.names_off[i + 1] - info.names_off[i])));
+                rbh::Windows wins = rbh::Windows::pack_text(bed_text.data(), bed_text.size(), names);
+                mark("pack_bed");
+                const rb_windows w = wins.view();
+                const uint32_t want = (stats_rows ? RB_WANT_STATS_TEXT : RB_WANT_TEXT) | (largest ? RB_WANT_NUMERIC : 0u);
+                rb_lift_out out{};
+                rc = rb_batch_set_windows(ctx, batch, &w);
+                if (rc == RB_OK) rc = rb_batch_liftover(ctx, batch, policy, want, 0, nullptr);
+                if (rc == RB_OK) rc = rb_batch_download_lift(ctx, batch, want, &out, nullptr);
+                mark("rb_batch_liftover");
+                if (rc == RB_OK) {
+                    if (largest) {  // main.rs:200-208
+                        const std::string rows = rbh::largest_rows(out);
+                        fwrite(rows.data(), 1, rows.size(), stdout);
+                    } else {
+                        fwrite(out.paf_text, 1, out.paf_nbytes, stdout);
+                    }
+                    fflush(stdout);
+                    mark("write");
+                    rb_free_lift_out(ctx, &out);
+                }
+            }
+        } else if (cmd == "stats") {
             fputs(rbh::stats_header(qbed).c_str(), stdout);  // printed before the input is read (main.rs:51)
             fflush(stdout);
             rbh::Paf paf = load_paf(input);
@@ -185,15 +278,18 @@ int main(int argc, char** argv) {
         }
     } catch (const rbh::Panic& e) {
         fprintf(stderr, "thread 'main' panicked: %s\n", e.what());
+        if (batch) rb_batch_free(ctx, batch);
         rb_ctx_destroy(ctx);
         return 101;
     }
     if (rc != RB_OK) {
         fprintf(stderr, "rb: %s\n", rb_last_error(ctx));
-        const bool ref_panic = rc <= RB_ERR_REF_CIGAR_PARSE && rc >= RB_ERR_REF_INDEX;
+        const bool ref_panic = (rc <= RB_ERR_REF_CIGAR_PARSE && rc >= RB_ERR_REF_INDEX) || rc == RB_ERR_REF_PAF_PARSE;
+        if (batch) rb_batch_free(ctx, batch);
         rb_ctx_destroy(ctx);
         return ref_panic ? 101 : 1;
     }
+    if (batch) rb_batch_free(ctx, batch);
     rb_ctx_destroy(ctx);
     mark("destroy");
     if (timing)

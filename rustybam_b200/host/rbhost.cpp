@@ -1,6 +1,7 @@
 // rbhost.cpp — host-side text I/O, packing and printing (see rbhost.hpp for the reference lines).
 #include "rbhost.hpp"
 #include "f32_fast.hpp"
+#include "../csrc/name_intern.hpp"
 
 #include <cerrno>
 #include <unistd.h>
@@ -379,27 +380,11 @@ Paf Paf::from_text(const char* text, size_t n) {
                     fill_range(grabs[g], grabs[g + 1]);
                 }
             });
-    // names meanwhile, on this thread, in file order (ids are handed out by first appearance).  Consecutive records mostly repeat
-    // their names (rows of one window run, reads of one contig): the name of the record before is compared first, the hash
-    // map only sees the changes — millions of short rows otherwise spend their time hashing
-    {
-        const char *lq = nullptr, *lt = nullptr;
-        size_t lqn = 0, ltn = 0;
-        uint32_t lq_id = 0, lt_id = 0;
-        for (size_t r = 0; r < n_ok; r++) {
-            const ParsedLine& L = parsed[kept[r]];
-            if (!(lq && lqn == L.q_name_n && memcmp(lq, L.q_name, lqn) == 0)) {
-                lq_id = paf.name_id(std::string(L.q_name, L.q_name_n));
-                lq = L.q_name; lqn = L.q_name_n;
-            }
-            if (!(lt && ltn == L.t_name_n && memcmp(lt, L.t_name, ltn) == 0)) {
-                lt_id = paf.name_id(std::string(L.t_name, L.t_name_n));
-                lt = L.t_name; ltn = L.t_name_n;
-            }
-            paf.q_id[r] = lq_id;
-            paf.t_id[r] = lt_id;
-        }
-    }
+    // names meanwhile, on this thread, in file order (ids are handed out by first appearance)
+    rbn::intern_record_names(
+        n_ok, [&](size_t r) { const ParsedLine& L = parsed[kept[r]]; return std::make_pair(L.q_name, L.q_name_n); },
+        [&](size_t r) { const ParsedLine& L = parsed[kept[r]]; return std::make_pair(L.t_name, L.t_name_n); },
+        [&](const char* p, size_t len) { return paf.name_id(std::string(p, len)); }, paf.q_id.data(), paf.t_id.data());
     for (;;) {  // ... then it helps with what is left
         const size_t g = next.fetch_add(1);
         if (g + 1 >= grabs.size()) break;
@@ -688,15 +673,16 @@ rb_windows Windows::view() const {
     return v;
 }
 
-void write_stats_rows(FILE* f, const Paf& paf, const rb_stats_out& st, bool qbed) {
-    const size_t n = paf.size();
+// rows [0, n) formatted by append(out, i) on all host threads, written to `f` in row order
+template <class Append>
+static void write_rows(FILE* f, size_t n, Append append) {
     const size_t block = 1u << 15;  // rows per work item
     const size_t n_blocks = (n + block - 1) / block;
     const unsigned nt = (unsigned)std::min<size_t>(std::max(1u, std::thread::hardware_concurrency()), std::max<size_t>(1, n_blocks));
     if (nt <= 1) {
         std::string out;
         for (size_t i = 0; i < n; i++) {
-            append_stats_row(out, paf, i, st, qbed);
+            append(out, i);
             if (out.size() > (1u << 20)) { fwrite(out.data(), 1, out.size(), f); out.clear(); }
         }
         fwrite(out.data(), 1, out.size(), f);
@@ -712,11 +698,25 @@ void write_stats_rows(FILE* f, const Paf& paf, const rb_stats_out& st, bool qbed
                 std::string& out = bufs[k];
                 out.clear();
                 const size_t lo = (b0 + k) * block, hi = std::min(n, lo + block);
-                for (size_t i = lo; i < hi; i++) append_stats_row(out, paf, i, st, qbed);
+                for (size_t i = lo; i < hi; i++) append(out, i);
             });
         for (auto& th : pool) th.join();
         for (size_t k = 0; k < nb; k++) fwrite(bufs[k].data(), 1, bufs[k].size(), f);
     }
+}
+
+void write_stats_rows(FILE* f, const Paf& paf, const rb_stats_out& st, bool qbed) {
+    write_rows(f, paf.size(), [&](std::string& out, size_t i) { append_stats_row(out, paf, i, st, qbed); });
+}
+
+void write_stats_rows(FILE* f, const rb_records& recs, const rb_stats_out& st, bool qbed) {
+    auto name = [&](uint32_t id) {
+        return std::string(reinterpret_cast<const char*>(recs.names) + recs.names_off[id], (size_t)(recs.names_off[id + 1] - recs.names_off[id]));
+    };
+    write_rows(f, recs.n_rec, [&](std::string& out, size_t i) {
+        append_row(out, name(recs.q_id[i]), name(recs.t_id[i]), recs.strand[i], recs.q_st[i], recs.q_en[i], recs.q_len[i], recs.t_st[i],
+                   recs.t_en[i], recs.t_len[i], st, i, qbed);
+    });
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -770,17 +770,18 @@ std::string stats_header(bool qbed) {
     return s;
 }
 
-void append_stats_row(std::string& s, const Paf& paf, size_t i, const rb_stats_out& st, bool qbed) {
+void append_row(std::string& s, const std::string& q_name, const std::string& t_name, uint8_t strand, uint64_t q_st, uint64_t q_en,
+                uint64_t q_len, uint64_t t_st, uint64_t t_en, uint64_t t_len, const rb_stats_out& st, size_t i, bool qbed) {
     auto q = [&] {
-        s += paf.names[paf.q_id[i]]; s += '\t'; s += std::to_string((int64_t)paf.q_st[i]); s += '\t';
-        s += std::to_string((int64_t)paf.q_en[i]); s += '\t'; s += std::to_string((int64_t)paf.q_len[i]); s += '\t';
+        s += q_name; s += '\t'; s += std::to_string((int64_t)q_st); s += '\t';
+        s += std::to_string((int64_t)q_en); s += '\t'; s += std::to_string((int64_t)q_len); s += '\t';
     };
     auto r = [&] {
-        s += paf.names[paf.t_id[i]]; s += '\t'; s += std::to_string((int64_t)paf.t_st[i]); s += '\t';
-        s += std::to_string((int64_t)paf.t_en[i]); s += '\t'; s += std::to_string((int64_t)paf.t_len[i]); s += '\t';
+        s += t_name; s += '\t'; s += std::to_string((int64_t)t_st); s += '\t';
+        s += std::to_string((int64_t)t_en); s += '\t'; s += std::to_string((int64_t)t_len); s += '\t';
     };
-    if (qbed) { q(); s += (char)paf.strand[i]; s += '\t'; r(); }
-    else { r(); s += (char)paf.strand[i]; s += '\t'; q(); }
+    if (qbed) { q(); s += (char)strand; s += '\t'; r(); }
+    else { r(); s += (char)strand; s += '\t'; q(); }
     s += fmt_f32(st.id_by_matches[i]); s += '\t';
     s += fmt_f32(st.id_by_events[i]); s += '\t';
     s += fmt_f32(st.id_by_all[i]); s += '\t';
@@ -790,6 +791,11 @@ void append_stats_row(std::string& s, const Paf& paf, size_t i, const rb_stats_o
     s += std::to_string(st.ins_events[i]); s += '\t';
     s += std::to_string(st.del[i]); s += '\t';
     s += std::to_string(st.ins[i]); s += '\n';
+}
+
+void append_stats_row(std::string& s, const Paf& paf, size_t i, const rb_stats_out& st, bool qbed) {
+    append_row(s, paf.names[paf.q_id[i]], paf.names[paf.t_id[i]], paf.strand[i], paf.q_st[i], paf.q_en[i], paf.q_len[i], paf.t_st[i],
+               paf.t_en[i], paf.t_len[i], st, i, qbed);
 }
 
 std::string paf_text(const Paf& paf, size_t lo, size_t hi) {

@@ -116,8 +116,13 @@ std::string fmt_f32(float v);                 // Rust `{}` for f32 (shortest rou
 std::string stats_header(bool qbed);          // bamstats.rs:225-236
 // bamstats.rs:239-270 for row i of `paf` with the GPU counters of row i
 void append_stats_row(std::string& out, const Paf& paf, size_t i, const rb_stats_out& st, bool qbed);
+// one row from its fields (what append_stats_row formats for a record of `paf`)
+void append_row(std::string& out, const std::string& q_name, const std::string& t_name, uint8_t strand, uint64_t q_st, uint64_t q_en,
+                uint64_t q_len, uint64_t t_st, uint64_t t_en, uint64_t t_len, const rb_stats_out& st, size_t i, bool qbed);
 // every row of `paf` (bamstats.rs:239-270), formatted on all host threads, written to `f` in row order
 void write_stats_rows(FILE* f, const Paf& paf, const rb_stats_out& st, bool qbed);
+// the same for records the library holds (rb_batch_records of a batch parsed on the device)
+void write_stats_rows(FILE* f, const rb_records& recs, const rb_stats_out& st, bool qbed);
 
 // ---- synthetic whole-genome-scale eqx PAF (SURVEY §8d, configs C2-C5) ----
 struct SynthParams {
