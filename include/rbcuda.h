@@ -248,6 +248,26 @@ int rb_batch_set_windows(rb_ctx* ctx, rb_batch* b, const rb_windows* wins);
  * next rb_batch_records on the batch */
 int rb_batch_records(rb_ctx* ctx, rb_batch* b, int with_cigar, rb_records* out);
 
+/* ---- BED text parsed on the device (bed::parse_bed, bed.rs:140-194, quirk for quirk as rbh::Windows::pack_text restates it) ---- */
+typedef struct rb_bed_info {
+    uint64_t text_bytes;   /* BED text parsed (the inflated size for BGZF input) */
+    uint64_t n_lines;      /* non-empty lines: runs of '\n' / '\r' separate lines */
+    uint64_t n_comments;   /* lines whose first byte is '#' */
+    uint64_t n_parsed;     /* rows that parse: these number the BED rows (bed_row), whether or not their contig is in the batch */
+    uint32_t n_win;        /* rows kept: contig name present in the batch's name table */
+    uint32_t n_fields;     /* field count of the first non-comment line: every row must have it */
+    int default_ids;       /* 1: n_fields <= 3, ids are "{chrom}:{st+1}-{en}" formatted on the device */
+    int general;           /* 1: rows nested / file order != sorted order -> the brute-force join layout (Q5) */
+} rb_bed_info;
+/* BED text, or BGZF bytes (rb_is_bgzf), -> the windows of batch b, replacing any it had; contig names resolve against b's name
+ * table (query and target names, like Paf::find_name).  Parsed, sorted and packed on the device. info is nullable.
+ * RB_ERR_BAD_ARG: a slice, null data, a plain (single-member) gzip stream, corrupt BGZF; RB_ERR_UNSUPPORTED: more than 2^32 - 1
+ * parsed rows.  On failure the batch is left without windows. */
+int rb_batch_set_windows_bed(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64_t nbytes, rb_bed_info* info);
+/* the batch's windows in the rb_windows layout (sorted by (t_id, st), stable; ids NULL when default), library-owned pinned,
+ * valid until rb_batch_free or the next rb_batch_windows on the batch */
+int rb_batch_windows(rb_ctx* ctx, rb_batch* b, rb_windows* out);
+
 /* ---- host helper: stable sort of BED rows by (t_id, st) into the rb_windows layout ----
  * perm_out[n_win] receives, for each sorted position, the BED row it came from. */
 int rb_sort_windows(uint32_t n_win, const uint32_t* t_id, const uint64_t* st, uint32_t* perm_out);

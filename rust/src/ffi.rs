@@ -46,6 +46,12 @@ pub struct rb_paf_info {
     pub cigar_bytes: u64,
 }
 #[repr(C)]
+pub struct rb_bed_info {
+    pub text_bytes: u64, pub n_lines: u64, pub n_comments: u64, pub n_parsed: u64,
+    pub n_win: u32, pub n_fields: u32,
+    pub default_ids: c_int, pub general: c_int,
+}
+#[repr(C)]
 pub struct rb_summary { pub n_ops: u64, pub n_pairs: u64, pub n_out: u64, pub out_bytes: u64, pub cigar_bytes: u64 }
 extern "C" {
     pub fn rb_ctx_create(device_ids: *const c_int, n: c_int, status: *mut c_int) -> *mut rb_ctx;
@@ -75,6 +81,9 @@ extern "C" {
     pub fn rb_batch_upload_paf(ctx: *mut rb_ctx, data: *const u8, nbytes: u64, info: *mut rb_paf_info, status: *mut c_int) -> *mut rb_batch;
     pub fn rb_batch_set_windows(ctx: *mut rb_ctx, b: *mut rb_batch, wins: *const rb_windows) -> c_int;
     pub fn rb_batch_records(ctx: *mut rb_ctx, b: *mut rb_batch, with_cigar: c_int, out: *mut rb_records) -> c_int;
+    /// bed.rs:140-194 bed::parse_bed on the device: BED text or BGZF bytes -> the batch's windows (names resolve against its name table)
+    pub fn rb_batch_set_windows_bed(ctx: *mut rb_ctx, b: *mut rb_batch, data: *const u8, nbytes: u64, info: *mut rb_bed_info) -> c_int;
+    pub fn rb_batch_windows(ctx: *mut rb_ctx, b: *mut rb_batch, out: *mut rb_windows) -> c_int;
     pub fn rb_batch_liftover(ctx: *mut rb_ctx, b: *mut rb_batch, policy: c_int, want: u32, with_stats: c_int, summary: *mut rb_summary) -> c_int;
     pub fn rb_batch_download_lift(ctx: *mut rb_ctx, b: *mut rb_batch, want: u32, out: *mut rb_lift_out, stats: *mut rb_stats_out) -> c_int;
     pub fn rb_batch_free(ctx: *mut rb_ctx, b: *mut rb_batch);

@@ -27,6 +27,7 @@ EXPORTS = [
     "rb_liftover", "rb_stats", "rb_break_paf", "rb_invert", "rb_trim_paf", "rb_trim_paf_begin", "rb_trim_paf_round", "rb_trim_paf_end", "rb_batch_break", "rb_free_lift_out", "rb_free_stats_out", "rb_batch_upload", "rb_batch_liftover", "rb_batch_stats",
     "rb_batch_download_lift", "rb_batch_download_stats", "rb_batch_free", "rb_sort_windows", "rb_version", "rb_host_register",
     "rb_host_unregister", "rb_is_bgzf", "rb_inflate_bgzf", "rb_free_text", "rb_batch_upload_paf", "rb_batch_set_windows", "rb_batch_records",
+    "rb_batch_set_windows_bed", "rb_batch_windows",
 ]
 
 u8p, u32p, u64p, f32p = C.POINTER(C.c_uint8), C.POINTER(C.c_uint32), C.POINTER(C.c_uint64), C.POINTER(C.c_float)
@@ -62,6 +63,11 @@ class RbSummary(C.Structure):
 class RbPafInfo(C.Structure):
     _fields_ = [("text_bytes", C.c_uint64), ("n_lines", C.c_uint64), ("skipped", C.c_uint64), ("n_rec", C.c_uint32), ("n_names", C.c_uint32),
                 ("names", u8p), ("names_off", u64p), ("cigar_bytes", C.c_uint64)]
+
+
+class RbBedInfo(C.Structure):
+    _fields_ = [("text_bytes", C.c_uint64), ("n_lines", C.c_uint64), ("n_comments", C.c_uint64), ("n_parsed", C.c_uint64),
+                ("n_win", C.c_uint32), ("n_fields", C.c_uint32), ("default_ids", C.c_int), ("general", C.c_int)]
 
 
 class RbKernelTime(C.Structure):
@@ -124,6 +130,8 @@ def load():
     lib.rb_batch_upload_paf.argtypes = [C.c_void_p, C.c_char_p, C.c_uint64, C.POINTER(RbPafInfo), C.POINTER(C.c_int)]
     lib.rb_batch_set_windows.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(RbWindows)]
     lib.rb_batch_records.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(RbRecords)]
+    lib.rb_batch_set_windows_bed.argtypes = [C.c_void_p, C.c_void_p, C.c_char_p, C.c_uint64, C.POINTER(RbBedInfo)]
+    lib.rb_batch_windows.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(RbWindows)]
     lib.rb_host_register.argtypes = [C.c_void_p, C.c_uint64]
     lib.rb_host_unregister.argtypes = [C.c_void_p]
     _lib = lib
@@ -410,6 +418,25 @@ class Context:
     def batch_set_windows(self, b, wins):
         """rb_batch_set_windows: windows (t_id = ids of the batch's name table) for a batch uploaded without them."""
         self._check(self.lib.rb_batch_set_windows(self.h, b, C.byref(wins.c) if wins is not None else None))
+
+    def batch_set_windows_bed(self, b, data: bytes) -> dict:
+        """rb_batch_set_windows_bed: BED text (or BGZF bytes) parsed on the device into the batch's windows; returns rb_bed_info."""
+        info = RbBedInfo()
+        self._check(self.lib.rb_batch_set_windows_bed(self.h, b, data, len(data), C.byref(info)))
+        return {k: int(getattr(info, k)) for k, _ in RbBedInfo._fields_}
+
+    def batch_windows(self, b) -> dict:
+        """rb_batch_windows: the batch's windows as numpy arrays in the rb_windows layout; ids_off / ids are None for default ids."""
+        w = RbWindows()
+        self._check(self.lib.rb_batch_windows(self.h, b, C.byref(w)))
+        n = int(w.n_win)
+        res = dict(n_win=n, t_id=_np(w.t_id, n, np.uint32), st=_np(w.st, n, np.uint64), en=_np(w.en, n, np.uint64),
+                   bed_row=_np(w.bed_row, n, np.uint32), ids_off=None, ids=None)
+        if w.ids_off:
+            res["ids_off"] = _np(w.ids_off, n + 1, np.uint64)
+            nb = int(res["ids_off"][-1])
+            res["ids"] = C.string_at(w.ids, nb) if nb else b""
+        return res
 
     def batch_records(self, b, with_cigar=True) -> dict:
         """rb_batch_records: the batch's records as numpy arrays named like Records' fields (names: list of bytes)."""

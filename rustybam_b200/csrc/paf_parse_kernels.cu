@@ -2,7 +2,7 @@
 // paf_parse_core.cuh applied on the GPU:
 //
 //   k_paf_lines_count  per 64 KiB of text: '\n' count (16-byte loads, per-byte masks, popcount, warp sums) and, per 4 KiB
-//                      tile, whether it holds any whitespace byte at all
+//                      tile, whether it holds any whitespace byte at all (also BED line starts: bed_parse_kernels.cu)
 //   k_paf_scan_*       exclusive scans (reduce -> scan of the block sums -> scan down) of up to three u64 columns at once
 //   k_paf_lines_fill   line start offsets: the newline of rank k starts line k + 1
 //   k_paf_fields       one warp per line: tokens, the tag test of every extra token, the first cg payload, the numeric columns
@@ -17,6 +17,7 @@
 #include <algorithm>
 #include <cstdint>
 
+#include "bed_parse_core.cuh"
 #include "paf_parse_core.cuh"
 #include "rb_kernels.cuh"
 
@@ -96,17 +97,46 @@ __device__ __forceinline__ uint64_t block_excl_scan(uint64_t v, uint64_t* sh, ui
 
 }  // namespace
 
+// Line starts, for two definitions of a line (the template parameter):
+//   LINES_PAF  a line ends at each '\n' (paf.rs lines()): the newline of rank k starts line k + 1, line 0 starts at 0; the count
+//              pass also flags the 4 KiB tiles that hold any whitespace byte and reads the last byte of the text
+//   LINES_BED  a line starts at a byte that is neither '\n' nor '\r' at offset 0 or right after one of them (bio's BED reader: a
+//              run of line ends is one separator, there are no empty lines); start of rank k starts line k
+enum : int { LINES_PAF = 0, LINES_BED = 1 };
+
+// bit j: a mark at pos + j (LINES_PAF: a '\n'; LINES_BED: a line start), ws = whitespace bits (LINES_PAF only)
+template <int MODE>
+__device__ __forceinline__ uint32_t line_marks(const uint8_t* text, uint64_t pos, uint64_t n, uint32_t& ws) {
+    uint32_t nl;
+    const uint4 w = load16(text, pos, n);
+    masks16(w, nl, ws);
+    if (MODE == LINES_PAF) return nl;
+    const uint32_t wd[4] = {w.x, w.y, w.z, w.w};
+    uint32_t eol = 0;
+#pragma unroll
+    for (int k = 0; k < 4; k++)
+#pragma unroll
+        for (int j = 0; j < 4; j++) eol |= (uint32_t)rbbp::is_eol((uint8_t)(wd[k] >> (8 * j))) << (4 * k + j);
+    const uint32_t prev_eol = pos == 0 || rbbp::is_eol(text[pos - 1]) ? 1u : 0u;
+    uint32_t st = ~eol & ((eol << 1) | prev_eol) & 0xFFFFu;
+    if (pos + 16 > n) st &= (1u << (n - pos)) - 1;  // (load16 pads with non-EOL bytes)
+    return st;
+}
+
+template <int MODE>
 __global__ void __launch_bounds__(PP_THREADS) k_paf_lines_count(const uint8_t* text, uint64_t n, uint64_t* chunk_cnt, uint8_t* tile_ws,
-                                                                 uint32_t* last_byte) {
+                                                             uint32_t* last_byte) {
     const uint64_t c0 = (uint64_t)blockIdx.x * PP_CHUNK;
     uint32_t cnt = 0;
     for (uint64_t t0 = c0; t0 < c0 + PP_CHUNK && t0 < n; t0 += PP_THREADS * 16) {
         const uint64_t pos = t0 + threadIdx.x * 16;
-        uint32_t nl = 0, ws = 0;
-        if (pos < n) masks16(load16(text, pos, n), nl, ws);
-        cnt += __popc(nl);
-        const int any = __syncthreads_or(ws != 0);
-        if (threadIdx.x == 0) tile_ws[t0 >> PP_TILE_SHIFT] = (uint8_t)any;
+        uint32_t m = 0, ws = 0;
+        if (pos < n) m = line_marks<MODE>(text, pos, n, ws);
+        cnt += __popc(m);
+        if (MODE == LINES_PAF) {
+            const int any = __syncthreads_or(ws != 0);
+            if (threadIdx.x == 0) tile_ws[t0 >> PP_TILE_SHIFT] = (uint8_t)any;
+        }
     }
     cnt = __reduce_add_sync(FULL, cnt);
     __shared__ uint32_t sh[PP_THREADS / 32];
@@ -116,27 +146,28 @@ __global__ void __launch_bounds__(PP_THREADS) k_paf_lines_count(const uint8_t* t
         uint32_t s = 0;
         for (int k = 0; k < PP_THREADS / 32; k++) s += sh[k];
         chunk_cnt[blockIdx.x] = s;
-        if (n && c0 <= n - 1 && n - 1 < c0 + PP_CHUNK) *last_byte = text[n - 1];
+        if (MODE == LINES_PAF && n && c0 <= n - 1 && n - 1 < c0 + PP_CHUNK) *last_byte = text[n - 1];
     }
 }
 
-// newline of rank k (chunk_off = exclusive scan of the chunk counts) at position p: line k + 1 starts at p + 1
-__global__ void __launch_bounds__(PP_THREADS) k_paf_lines_fill(const uint8_t* text, uint64_t n, const uint64_t* chunk_off,
-                                                                uint64_t* line_start) {
+// chunk_off = exclusive scan of the chunk counts
+template <int MODE>
+__global__ void __launch_bounds__(PP_THREADS) k_paf_lines_fill(const uint8_t* text, uint64_t n, const uint64_t* chunk_off, uint64_t* line_start) {
     __shared__ uint64_t sh[PP_THREADS / 32];
     const uint64_t c0 = (uint64_t)blockIdx.x * PP_CHUNK;
     uint64_t carry = chunk_off[blockIdx.x];
-    if (blockIdx.x == 0 && threadIdx.x == 0) line_start[0] = 0;
+    if (MODE == LINES_PAF && blockIdx.x == 0 && threadIdx.x == 0) line_start[0] = 0;
     for (uint64_t t0 = c0; t0 < c0 + PP_CHUNK && t0 < n; t0 += PP_THREADS * 16) {
         const uint64_t pos = t0 + threadIdx.x * 16;
-        uint32_t nl = 0, ws = 0;
-        if (pos < n) masks16(load16(text, pos, n), nl, ws);
+        uint32_t m = 0, ws = 0;
+        if (pos < n) m = line_marks<MODE>(text, pos, n, ws);
         uint64_t tot;
-        uint64_t k = carry + block_excl_scan(__popc(nl), sh, tot);
-        while (nl) {
-            const int j = __ffs(nl) - 1;
-            nl &= nl - 1;
-            line_start[++k] = pos + j + 1;
+        uint64_t k = carry + block_excl_scan(__popc(m), sh, tot);
+        while (m) {
+            const int j = __ffs(m) - 1;
+            m &= m - 1;
+            if (MODE == LINES_PAF) line_start[++k] = pos + j + 1;
+            else line_start[k++] = pos + j;
         }
         carry += tot;
     }
@@ -325,7 +356,7 @@ __global__ void __launch_bounds__(PP_THREADS) k_paf_pack(const uint8_t* text, ui
     rec_qlen[r] = ql;
 }
 
-// destination bytes [16 t, 16 t + 16) of the packed CIGAR text
+// destination bytes [16 t, 16 t + 16) of the packed CIGAR text (also the packed BED ids: rec_line nullptr, cg_off per row)
 __global__ void __launch_bounds__(PP_THREADS) k_paf_copy_cg(const uint8_t* text, uint32_t n_rec, const uint64_t* cigar_off,
                                                              const uint32_t* rec_line, const uint64_t* cg_off, uint8_t* dst) {
     const uint64_t total = cigar_off[n_rec];
@@ -343,7 +374,7 @@ __global__ void __launch_bounds__(PP_THREADS) k_paf_copy_cg(const uint8_t* text,
         const uint64_t pos = pos0 + j;
         if (pos >= total) { b[j] = '0'; continue; }  // (the tail padding of the text is '0' bytes)
         while (pos >= cigar_off[r + 1]) r++;
-        b[j] = text[cg_off[rec_line[r]] + (pos - cigar_off[r])];
+        b[j] = text[cg_off[rec_line ? rec_line[r] : r] + (pos - cigar_off[r])];
     }
     uint4 w;
     w.x = b[0] | (b[1] << 8) | (b[2] << 16) | ((uint32_t)b[3] << 24);
@@ -358,10 +389,16 @@ uint64_t paf_tiles(uint64_t n) { return (n >> PP_TILE_SHIFT) + 1; }
 uint64_t paf_scan_parts(uint64_t n) { return (n + SCAN_CH - 1) / SCAN_CH + 1; }
 
 void launch_paf_lines_count(const uint8_t* text, uint64_t n, uint64_t* chunk_cnt, uint8_t* tile_ws, uint32_t* last_byte, cudaStream_t s) {
-    if (n) k_paf_lines_count<<<(unsigned)paf_chunks(n), PP_THREADS, 0, s>>>(text, n, chunk_cnt, tile_ws, last_byte);
+    if (n) k_paf_lines_count<LINES_PAF><<<(unsigned)paf_chunks(n), PP_THREADS, 0, s>>>(text, n, chunk_cnt, tile_ws, last_byte);
 }
 void launch_paf_lines_fill(const uint8_t* text, uint64_t n, const uint64_t* chunk_off, uint64_t* line_start, cudaStream_t s) {
-    if (n) k_paf_lines_fill<<<(unsigned)paf_chunks(n), PP_THREADS, 0, s>>>(text, n, chunk_off, line_start);
+    if (n) k_paf_lines_fill<LINES_PAF><<<(unsigned)paf_chunks(n), PP_THREADS, 0, s>>>(text, n, chunk_off, line_start);
+}
+void launch_bed_lines_count(const uint8_t* text, uint64_t n, uint64_t* chunk_cnt, cudaStream_t s) {
+    if (n) k_paf_lines_count<LINES_BED><<<(unsigned)paf_chunks(n), PP_THREADS, 0, s>>>(text, n, chunk_cnt, nullptr, nullptr);
+}
+void launch_bed_lines_fill(const uint8_t* text, uint64_t n, const uint64_t* chunk_off, uint64_t* line_start, cudaStream_t s) {
+    if (n) k_paf_lines_fill<LINES_BED><<<(unsigned)paf_chunks(n), PP_THREADS, 0, s>>>(text, n, chunk_off, line_start);
 }
 void launch_paf_scan(int nv, const uint64_t* const* in, uint64_t* const* out, uint64_t n, uint64_t* part, cudaStream_t s) {
     ScanCols c{};

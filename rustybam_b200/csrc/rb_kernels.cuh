@@ -258,6 +258,35 @@ void launch_paf_pack(const uint8_t* text, uint64_t n_lines, PafLineCols L, const
                      uint8_t* names, uint64_t* rec_name_off, uint32_t* rec_qlen, cudaStream_t s);
 void launch_paf_copy_cg(const uint8_t* text, uint32_t n_rec, const uint64_t* cigar_off, const uint32_t* rec_line, const uint64_t* cg_off,
                         uint64_t cg_bytes, uint8_t* dst, cudaStream_t s);
+// BED text -> the window tables of a batch (bed_parse_kernels.cu; the rules are bed_parse_core.cuh's).  Per-line columns:
+struct BedLineCols {
+    const uint64_t* line_start;
+    uint64_t *n_fields, *st, *en, *name_len, *id_off, *id_len;
+    uint8_t* nums_ok;
+    uint64_t *comment, *parses, *kept;  // 0 / 1 (scan inputs: comment count, bed_row, window index)
+    uint32_t* tid;                      // name id of a kept line, ~0 otherwise
+};
+struct BedRows {  // kept rows in file order
+    uint32_t *tid, *row;
+    uint64_t *st, *en, *line;
+};
+void launch_bed_lines_count(const uint8_t* text, uint64_t n, uint64_t* chunk_cnt, cudaStream_t s);
+void launch_bed_lines_fill(const uint8_t* text, uint64_t n, const uint64_t* chunk_off, uint64_t* line_start, cudaStream_t s);
+uint64_t bed_name_slots(uint32_t n_names);  // u32 slots of the device name table (a power of two)
+void launch_bed_names(const uint8_t* names, const uint64_t* names_off, uint32_t n_names, uint32_t* table, uint64_t slots, cudaStream_t s);
+void launch_bed_fields(const uint8_t* text, uint64_t n, uint64_t n_lines, BedLineCols L, unsigned long long* first_row, cudaStream_t s);
+void launch_bed_judge(const uint8_t* text, uint64_t n_lines, BedLineCols L, const unsigned long long* first_row, const uint8_t* names,
+                      const uint64_t* names_off, const uint32_t* table, uint64_t slots, unsigned long long* nf0_out, cudaStream_t s);
+void launch_bed_compact(uint64_t n_lines, BedLineCols L, const uint64_t* row_idx, const uint64_t* win_idx, BedRows R, unsigned long long* max_st,
+                        cudaStream_t s);
+void launch_bed_order(BedRows R, uint32_t n, uint32_t* unsorted, cudaStream_t s);  // *unsorted |= 1 if R is not in (t_id, st) order
+size_t bed_sort_scratch(uint32_t n);
+cudaError_t launch_bed_sort(BedRows R, uint32_t n, int tb, int sb, bool by_tid_only, void* scratch, size_t scratch_bytes, uint32_t* perm,
+                            cudaStream_t s);
+// rows perm[k] (perm nullptr: k) of R -> row k of the w_* tables; id_off / id_len (nullable) = the field-4 span of that row's line
+void launch_bed_gather(BedRows R, uint32_t n, const uint32_t* perm, const uint64_t* line_id_off, const uint64_t* line_id_len, uint32_t* w_tid,
+                       uint64_t* w_st, uint64_t* w_en, uint32_t* w_row, uint64_t* id_off, uint64_t* id_len, cudaStream_t s);
+void launch_bed_cont(const uint32_t* w_tid, uint32_t n, uint32_t* cont_lo, uint32_t* cont_hi, cudaStream_t s);
 void launch_win_check(const uint32_t* t_id, const uint64_t* st, const uint64_t* en, const uint32_t* row, uint32_t n_win,
                       uint32_t n_names, uint32_t* flags, cudaStream_t s);
 // general path (unsorted / nested BED rows): the reference's cartesian product + overlap filter (liftover.rs:123-127)

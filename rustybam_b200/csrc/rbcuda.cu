@@ -213,6 +213,7 @@ struct rb_batch {
     std::vector<uint8_t> h_names;
     std::vector<uint64_t> h_names_off;
     PinBuf rec_out;
+    PinBuf win_out;  // rb_batch_windows: its pinned copy of the window tables
 };
 
 namespace {
@@ -1892,6 +1893,297 @@ int rb_batch_set_windows(rb_ctx* ctx, rb_batch* b, const rb_windows* wins) {
     b->busy = false;
     if (rc != RB_OK) b->n_win = 0;
     return rc;
+}
+
+// ---- BED text on the device (rb_batch_set_windows_bed; kernels in bed_parse_kernels.cu) -------------------------------------
+// text -> HBM (or BGZF -> inflated in HBM) -> line starts -> per-line fields -> first non-comment line's field count -> contig
+// lookup in a hash table of the batch's resident name table -> scans (bed_row, window index, comments) -> kept rows in file
+// order -> (only if they are not in (t_id, st) order already) a stable radix sort -> the batch's w_* tables, contig ranges ->
+// k_win_check -> the general layout ((t_id, bed_row) order) when its verdict asks for it -> ids.  Only the rb_bed_info scalars
+// come back to the host; the text and every per-line table are freed before the call returns.
+static int bed_upload_into(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64_t nbytes, rb_bed_info* info) {
+    cudaStream_t s = ctx->stream;
+    uint32_t* sc = ctx->scalars.as<uint32_t>();
+    volatile uint64_t* hs = reinterpret_cast<volatile uint64_t*>(ctx->h_scalars);
+    DevBuf d_text, d_chunk, d_part, d_lines, d_cols, d_tbl, d_rows, d_sort, d_ids;
+    DevScratch scratch{{&d_text, &d_chunk, &d_part, &d_lines, &d_cols, &d_tbl, &d_rows, &d_sort, &d_ids}};
+    constexpr size_t TEXT_PAD = 4096;  // (16-byte loads of the last bytes)
+    b->n_win = 0;
+    b->wsrc = nullptr;
+    b->general = false; b->default_ids = true; b->win_pending = false;
+    b->have_lift = false;
+    uint64_t n = 0;
+    if (rb_is_bgzf(data, nbytes)) {
+        const int rc = inflate_to_device(ctx, data, nbytes, d_text, n, TEXT_PAD);
+        if (rc != RB_OK) return rc;
+    } else if (nbytes >= 2 && data[0] == 0x1f && data[1] == 0x8b) {
+        return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_set_windows_bed: a plain gzip stream (not BGZF); inflate it first");
+    } else {
+        n = nbytes;
+        CU(d_text.ensure(n + TEXT_PAD));
+        if (n) CU(h2d_copy(d_text.p, data, n, s));
+    }
+    const uint8_t* text = d_text.as<uint8_t>();
+    // 1. line starts
+    uint64_t nl = 0;
+    if (n) {
+        const uint64_t nc = paf_chunks(n);
+        CU(d_chunk.ensure((2 * nc + 2) * 8));
+        CU(d_part.ensure(paf_scan_parts(nc) * 8));
+        uint64_t* cnt = d_chunk.as<uint64_t>();
+        uint64_t* off = cnt + nc;
+        {
+            KScope k(ctx, "k_paf_lines_count");
+            launch_bed_lines_count(text, n, cnt, s);
+        }
+        {
+            KScope k(ctx, "k_paf_scan");
+            const uint64_t* in[1] = {cnt};
+            uint64_t* out[1] = {off};
+            launch_paf_scan(1, in, out, nc, d_part.as<uint64_t>(), s);
+        }
+        Publisher(ctx).u64(0, off + nc).go(s);
+        CU(cudaStreamSynchronize(s));
+        nl = hs[0];
+        CU(d_lines.ensure((nl + 1) * 8));
+        {
+            KScope k(ctx, "k_paf_lines_fill");
+            launch_bed_lines_fill(text, n, off, d_lines.as<uint64_t>(), s);
+        }
+    }
+    // 2. per-line fields, the field count, contig lookup, scans, rows in file order
+    size_t o = 0;
+    auto carve = [&](size_t bytes) { const size_t at = o; o += align_up(bytes, 256); return at; };
+    const size_t o_nf = carve(nl * 8), o_st = carve(nl * 8), o_en = carve(nl * 8), o_nm = carve(nl * 8), o_io = carve(nl * 8),
+                 o_il = carve(nl * 8), o_ok = carve(nl + 8), o_cm = carve(nl * 8), o_pa = carve(nl * 8), o_ke = carve(nl * 8),
+                 o_tid = carve(nl * 4), o_s0 = carve((nl + 1) * 8), o_s1 = carve((nl + 1) * 8), o_s2 = carve((nl + 1) * 8), o_sc = carve(64);
+    CU(d_cols.ensure(o + 256));
+    CU(d_part.ensure(3 * paf_scan_parts(nl) * 8));
+    uint8_t* cb = d_cols.as<uint8_t>();
+    auto u64at = [&](size_t at) { return reinterpret_cast<uint64_t*>(cb + at); };
+    BedLineCols L{};
+    L.line_start = d_lines.as<uint64_t>();
+    L.n_fields = u64at(o_nf); L.st = u64at(o_st); L.en = u64at(o_en); L.name_len = u64at(o_nm); L.id_off = u64at(o_io); L.id_len = u64at(o_il);
+    L.nums_ok = cb + o_ok; L.comment = u64at(o_cm); L.parses = u64at(o_pa); L.kept = u64at(o_ke);
+    L.tid = reinterpret_cast<uint32_t*>(cb + o_tid);
+    uint64_t* row_idx = u64at(o_s0);
+    uint64_t* win_idx = u64at(o_s1);
+    uint64_t* cmt_idx = u64at(o_s2);
+    unsigned long long* dsc = reinterpret_cast<unsigned long long*>(cb + o_sc);  // first row, nf0, max st, unsorted flag
+    CU(cudaMemsetAsync(dsc, 0, 32, s));
+    CU(cudaMemsetAsync(dsc, 0xFF, 8, s));
+    const uint64_t slots = bed_name_slots(b->n_names);
+    CU(d_tbl.ensure(slots * 4));
+    CU(cudaMemsetAsync(d_tbl.p, 0, slots * 4, s));
+    {
+        KScope k(ctx, "k_bed_names");
+        launch_bed_names(b->names.as<uint8_t>(), b->names_off.as<uint64_t>(), b->n_names, d_tbl.as<uint32_t>(), slots, s);
+    }
+    {
+        KScope k(ctx, "k_bed_fields");
+        launch_bed_fields(text, n, nl, L, dsc, s);
+    }
+    {
+        KScope k(ctx, "k_bed_judge");
+        launch_bed_judge(text, nl, L, dsc, b->names.as<uint8_t>(), b->names_off.as<uint64_t>(), d_tbl.as<uint32_t>(), slots, dsc + 1, s);
+    }
+    {
+        KScope k(ctx, "k_paf_scan");
+        const uint64_t* in[3] = {L.parses, L.kept, L.comment};
+        uint64_t* out[3] = {row_idx, win_idx, cmt_idx};
+        launch_paf_scan(3, in, out, nl, d_part.as<uint64_t>(), s);
+    }
+    Publisher(ctx).u64(0, row_idx + nl).u64(1, win_idx + nl).u64(2, cmt_idx + nl).u64(3, dsc + 1).go(s);
+    CU(cudaStreamSynchronize(s));
+    CU(cudaGetLastError());
+    const uint64_t n_parsed = hs[0], n_kept = hs[1], n_comments = hs[2], nf0 = hs[3];
+    if (n_parsed > 0xFFFFFFFFull) { flush_times(ctx); return fail(ctx, RB_ERR_UNSUPPORTED, "rb_batch_set_windows_bed: more than 2^32 - 1 BED rows"); }
+    const uint32_t nw = (uint32_t)n_kept;
+    const bool default_ids = nf0 <= 3;
+    CU(d_rows.ensure((size_t)nw * 32 + 5 * 256));
+    BedRows R{};
+    {
+        size_t ro = 0;
+        auto rcarve = [&](size_t bytes) { const size_t at = ro; ro += align_up(bytes, 256); return d_rows.as<uint8_t>() + at; };
+        R.tid = reinterpret_cast<uint32_t*>(rcarve((size_t)nw * 4)); R.row = reinterpret_cast<uint32_t*>(rcarve((size_t)nw * 4));
+        R.st = reinterpret_cast<uint64_t*>(rcarve((size_t)nw * 8)); R.en = reinterpret_cast<uint64_t*>(rcarve((size_t)nw * 8));
+        R.line = reinterpret_cast<uint64_t*>(rcarve((size_t)nw * 8));
+    }
+    {
+        KScope k(ctx, "k_bed_compact");
+        launch_bed_compact(nl, L, row_idx, win_idx, R, dsc + 2, s);
+    }
+    {
+        KScope k(ctx, "k_bed_order");
+        launch_bed_order(R, nw, reinterpret_cast<uint32_t*>(dsc + 3), s);
+    }
+    Publisher(ctx).u64(0, dsc + 2).u32(1, dsc + 3).go(s);
+    CU(cudaStreamSynchronize(s));
+    const uint64_t max_st = hs[0];
+    const bool unsorted = (hs[1] & 1u) != 0;
+    // 3. the (t_id, st) layout, contig ranges, the layout check
+    CU(b->w_st.ensure((size_t)nw * 8 + 8)); CU(b->w_en.ensure((size_t)nw * 8 + 8)); CU(b->w_bed_row.ensure((size_t)nw * 4 + 8));
+    CU(b->w_tid.ensure((size_t)nw * 4 + 8));
+    CU(b->cont_lo.ensure(((size_t)b->n_names + 1) * 4)); CU(b->cont_hi.ensure(((size_t)b->n_names + 1) * 4));
+    auto bits = [](uint64_t v) { int k = 0; while (v) { k++; v >>= 1; } return k; };
+    const int tb = bits(b->n_names ? b->n_names - 1 : 0), sb = bits(max_st);
+    const size_t sort_bytes = bed_sort_scratch(nw);
+    uint32_t* perm = nullptr;
+    if (nw && unsorted) {
+        CU(d_sort.ensure(sort_bytes + (size_t)nw * 4 + 256));
+        perm = reinterpret_cast<uint32_t*>(d_sort.as<uint8_t>() + align_up(sort_bytes, 256));
+        KScope k(ctx, "k_bed_sort");
+        CU(launch_bed_sort(R, nw, tb, sb, false, d_sort.p, sort_bytes, perm, s));
+    }
+    uint64_t* id_span = nullptr;  // id offset / length per row in the final layout, then their scan input
+    if (!default_ids) {
+        CU(d_ids.ensure((size_t)nw * 16 + 512));
+        id_span = d_ids.as<uint64_t>();
+    }
+    {
+        KScope k(ctx, "k_bed_gather");
+        launch_bed_gather(R, nw, perm, L.id_off, L.id_len, b->w_tid.as<uint32_t>(), b->w_st.as<uint64_t>(), b->w_en.as<uint64_t>(),
+                          b->w_bed_row.as<uint32_t>(), id_span, id_span ? id_span + nw + 32 : nullptr, s);
+    }
+    CU(cudaMemsetAsync(b->cont_lo.p, 0, ((size_t)b->n_names + 1) * 4, s));
+    CU(cudaMemsetAsync(b->cont_hi.p, 0, ((size_t)b->n_names + 1) * 4, s));
+    {
+        KScope k(ctx, "k_bed_cont");
+        launch_bed_cont(b->w_tid.as<uint32_t>(), nw, b->cont_lo.as<uint32_t>(), b->cont_hi.as<uint32_t>(), s);
+    }
+    b->n_win = nw;
+    b->default_ids = default_ids;
+    rb_records Rn{};
+    Rn.n_names = b->n_names;
+    int rc = windows_check(ctx, b, &Rn, s);
+    if (rc != RB_OK) return rc;
+    b->win_pending = false;
+    if (nw) {
+        CU(cudaEventSynchronize(ctx->ev_win));
+        b->general = (((uint32_t)hs[16]) & 2u) != 0;
+    }
+    if (b->general) {  // file order grouped by contig = (t_id, bed_row) order: R is in file order, so a stable sort by t_id
+        CU(d_sort.ensure(sort_bytes + (size_t)nw * 4 + 256));
+        perm = reinterpret_cast<uint32_t*>(d_sort.as<uint8_t>() + align_up(sort_bytes, 256));
+        {
+            KScope k(ctx, "k_bed_sort");
+            CU(launch_bed_sort(R, nw, tb, sb, true, d_sort.p, sort_bytes, perm, s));
+        }
+        KScope k(ctx, "k_bed_gather");
+        launch_bed_gather(R, nw, perm, L.id_off, L.id_len, b->w_tid.as<uint32_t>(), b->w_st.as<uint64_t>(), b->w_en.as<uint64_t>(),
+                          b->w_bed_row.as<uint32_t>(), id_span, id_span ? id_span + nw + 32 : nullptr, s);
+    }
+    // 4. ids: offsets = scan of the lengths in the final layout, then the bytes
+    uint64_t ids_bytes = 0;
+    if (!default_ids) {
+        CU(b->w_ids_off.ensure(((size_t)nw + 1) * 8));
+        CU(d_part.ensure(paf_scan_parts(nw) * 8));
+        {
+            KScope k(ctx, "k_paf_scan");
+            const uint64_t* in[1] = {id_span + nw + 32};
+            uint64_t* out[1] = {b->w_ids_off.as<uint64_t>()};
+            launch_paf_scan(1, in, out, nw, d_part.as<uint64_t>(), s);
+        }
+        Publisher(ctx).u64(0, b->w_ids_off.as<uint64_t>() + nw).go(s);
+        CU(cudaStreamSynchronize(s));
+        ids_bytes = hs[0];
+        CU(b->w_ids.ensure(align_up(ids_bytes, 16) + 64));
+        KScope k(ctx, "k_paf_copy_cg");
+        launch_paf_copy_cg(text, nw, b->w_ids_off.as<uint64_t>(), nullptr, id_span, ids_bytes, b->w_ids.as<uint8_t>(), s);
+    }
+    CU(cudaStreamSynchronize(s));
+    CU(cudaGetLastError());
+    flush_times(ctx);
+    if (info) {
+        info->text_bytes = n; info->n_lines = nl; info->n_comments = n_comments; info->n_parsed = n_parsed;
+        info->n_win = nw; info->n_fields = (uint32_t)std::min<uint64_t>(nf0, 0xFFFFFFFFull);
+        info->default_ids = default_ids ? 1 : 0; info->general = b->general ? 1 : 0;
+    }
+    return RB_OK;
+}
+
+int rb_batch_set_windows_bed(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64_t nbytes, rb_bed_info* info) {
+    if (!ctx || !b) return RB_ERR_BAD_ARG;
+    if (info) memset(info, 0, sizeof *info);
+    if (!data && nbytes) return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_set_windows_bed: null data");
+    if (b->wsrc) return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_set_windows_bed: not on a slice");
+    cudaSetDevice(ctx->device);
+    if (b->busy) { CU(cudaStreamSynchronize(ctx->stream)); b->busy = false; }
+    int rc = bed_upload_into(ctx, b, data, nbytes, info);
+    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess && rc == RB_OK) {
+        (void)cudaGetLastError();
+        rc = fail(ctx, RB_ERR_CUDA, "BED parse failed");
+    }
+    if (rc != RB_OK) {
+        flush_times(ctx);
+        b->n_win = 0; b->general = false; b->win_pending = false;
+        if (info) memset(info, 0, sizeof *info);
+    }
+    return rc;
+}
+
+int rb_batch_windows(rb_ctx* ctx, rb_batch* b, rb_windows* out) {
+    if (!ctx || !b || !out) return RB_ERR_BAD_ARG;
+    if (b->wsrc) return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_windows: not on a slice");
+    cudaSetDevice(ctx->device);
+    cudaStream_t s = ctx->stream;
+    memset(out, 0, sizeof *out);
+    if (b->busy) { CU(cudaStreamSynchronize(s)); b->busy = false; }
+    const size_t nw = b->n_win;
+    uint64_t ids_bytes = 0;
+    if (!b->default_ids && nw) {
+        CU(cudaMemcpyAsync(&ids_bytes, b->w_ids_off.as<uint64_t>() + nw, 8, cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
+    }
+    // device copy at [0, o_end), the (t_id, st) layout of a general table after it
+    const size_t o_tid = 0, o_st = align_up(nw * 4 + 1, 64), o_en = o_st + align_up(nw * 8 + 1, 64), o_row = o_en + align_up(nw * 8 + 1, 64),
+                 o_off = o_row + align_up(nw * 4 + 1, 64), o_ids = o_off + align_up((nw + 1) * 8, 64), o_end = o_ids + align_up(ids_bytes + 1, 64);
+    CU(b->win_out.ensure(b->general ? 2 * o_end : o_end));
+    uint8_t* p = b->win_out.p;
+    uint64_t* off = reinterpret_cast<uint64_t*>(p + o_off);
+    off[0] = 0;
+    if (nw) {
+        CU(cudaMemcpyAsync(p + o_tid, b->w_tid.p, nw * 4, cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(p + o_st, b->w_st.p, nw * 8, cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(p + o_en, b->w_en.p, nw * 8, cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(p + o_row, b->w_bed_row.p, nw * 4, cudaMemcpyDeviceToHost, s));
+        if (!b->default_ids) {
+            CU(cudaMemcpyAsync(off, b->w_ids_off.p, (nw + 1) * 8, cudaMemcpyDeviceToHost, s));
+            if (ids_bytes) CU(cudaMemcpyAsync(p + o_ids, b->w_ids.p, ids_bytes, cudaMemcpyDeviceToHost, s));
+        }
+        CU(cudaStreamSynchronize(s));
+    }
+    if (b->general && nw) {  // stored in (t_id, bed_row) order: a stable sort by (t_id, st) gives the rb_windows table back
+        const uint32_t* tid = reinterpret_cast<const uint32_t*>(p + o_tid);
+        const uint64_t* st = reinterpret_cast<const uint64_t*>(p + o_st);
+        std::vector<uint32_t> perm(nw);
+        for (size_t i = 0; i < nw; i++) perm[i] = (uint32_t)i;
+        std::stable_sort(perm.begin(), perm.end(), [&](uint32_t a, uint32_t c) { return tid[a] != tid[c] ? tid[a] < tid[c] : st[a] < st[c]; });
+        uint8_t* q = p + o_end;
+        uint64_t* qoff = reinterpret_cast<uint64_t*>(q + o_off);
+        qoff[0] = 0;
+        for (size_t i = 0; i < nw; i++) {
+            const uint32_t j = perm[i];
+            reinterpret_cast<uint32_t*>(q + o_tid)[i] = tid[j];
+            reinterpret_cast<uint64_t*>(q + o_st)[i] = st[j];
+            reinterpret_cast<uint64_t*>(q + o_en)[i] = reinterpret_cast<const uint64_t*>(p + o_en)[j];
+            reinterpret_cast<uint32_t*>(q + o_row)[i] = reinterpret_cast<const uint32_t*>(p + o_row)[j];
+            if (!b->default_ids) {
+                const uint64_t len = off[j + 1] - off[j];
+                memcpy(q + o_ids + qoff[i], p + o_ids + off[j], len);
+                qoff[i + 1] = qoff[i] + len;
+            }
+        }
+        p = q;
+    }
+    out->n_win = (uint32_t)nw;
+    out->t_id = reinterpret_cast<const uint32_t*>(p + o_tid);
+    out->st = reinterpret_cast<const uint64_t*>(p + o_st);
+    out->en = reinterpret_cast<const uint64_t*>(p + o_en);
+    out->bed_row = reinterpret_cast<const uint32_t*>(p + o_row);
+    out->ids = b->default_ids ? nullptr : p + o_ids;
+    out->ids_off = b->default_ids ? nullptr : reinterpret_cast<const uint64_t*>(p + o_off);
+    return RB_OK;
 }
 
 int rb_batch_records(rb_ctx* ctx, rb_batch* b, int with_cigar, rb_records* out) {

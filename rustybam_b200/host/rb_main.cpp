@@ -112,39 +112,48 @@ int main(int argc, char** argv) {
         return rbh::Paf::from_file(path);
     };
     // RB_DEVICE_PARSE=1: `rb liftover` (plain, --stats, --largest) and `rb stats --paf` on one GPU hand the file's bytes to
-    // rb_batch_upload_paf — lines are split and parsed on the device — instead of parsing them on the host.  A plain file is mapped,
-    // a .bgz goes as it is (inflated on the device), a plain .gz and stdin are inflated / read by rbh::read_all first.
+    // rb_batch_upload_paf — lines are split and parsed on the device — instead of parsing them on the host; `rb liftover` hands the
+    // BED's bytes to rb_batch_set_windows_bed the same way.  A plain file is mapped, a .bgz / .gz that is BGZF goes as it is
+    // (inflated on the device), a plain .gz and stdin are inflated / read by rbh::read_all first.
     const char* dp = getenv("RB_DEVICE_PARSE");
     const bool device_parse = dp && dp[0] == '1' && n_gpus == 1 && !qbed && (cmd == "liftover" || cmd == "stats");
     rb_batch* batch = nullptr;
     rb_paf_info info{};
-    auto upload_paf = [&](const std::string& path) {
-        auto ends_with = [&](const char* suf) { const size_t n = strlen(suf); return path.size() >= n && path.compare(path.size() - n, n, suf) == 0; };
+    struct InputBytes {
         std::string owned;
         const uint8_t* data = nullptr;
         size_t n = 0;
         void* map = nullptr;
+        ~InputBytes() { if (map) munmap(map, n); }
+    };
+    auto input_bytes = [&](const std::string& path, InputBytes& in) {
+        auto ends_with = [&](const char* suf) { const size_t n = strlen(suf); return path.size() >= n && path.compare(path.size() - n, n, suf) == 0; };
         if (path != "-" && !ends_with(".gz") && !ends_with(".bgz")) {
             const int fd = ::open(path.c_str(), O_RDONLY);
             if (fd < 0) throw rbh::Panic("Error: cannot read input file " + path);
             struct stat st;
             if (fstat(fd, &st) == 0 && S_ISREG(st.st_mode) && st.st_size > 0) {
-                map = mmap(nullptr, (size_t)st.st_size, PROT_READ, MAP_PRIVATE, fd, 0);
-                if (map == MAP_FAILED) map = nullptr;
-                else { data = static_cast<const uint8_t*>(map); n = (size_t)st.st_size; }
+                in.map = mmap(nullptr, (size_t)st.st_size, PROT_READ, MAP_PRIVATE, fd, 0);
+                if (in.map == MAP_FAILED) in.map = nullptr;
+                else { in.data = static_cast<const uint8_t*>(in.map); in.n = (size_t)st.st_size; }
             }
             ::close(fd);
-            if (!map) owned = rbh::read_raw(path);
+            if (!in.map) in.owned = rbh::read_raw(path);
         } else if (path != "-") {
-            owned = rbh::read_raw(path);
-            if (!rb_is_bgzf(reinterpret_cast<const uint8_t*>(owned.data()), owned.size())) owned = rbh::read_all(path);
+            in.owned = rbh::read_raw(path);
+            if (!rb_is_bgzf(reinterpret_cast<const uint8_t*>(in.owned.data()), in.owned.size())) in.owned = rbh::read_all(path);
         } else {
-            owned = rbh::read_all(path);
+            in.owned = rbh::read_all(path);
         }
-        if (!map) { data = reinterpret_cast<const uint8_t*>(owned.data()); n = owned.size(); }
+        if (!in.map) { in.data = reinterpret_cast<const uint8_t*>(in.owned.data()); in.n = in.owned.size(); }
+    };
+    auto upload_paf = [&](const std::string& path) {
         int st = 0;
-        batch = rb_batch_upload_paf(ctx, data, n, &info, &st);
-        if (map) munmap(map, n);
+        {
+            InputBytes in;
+            input_bytes(path, in);
+            batch = rb_batch_upload_paf(ctx, in.data, in.n, &info, &st);
+        }
         if (!batch) return st;
         if (info.skipped) fprintf(stderr, "\nUnable to parse %zu PAF record(s). Skipped.\n", (size_t)info.skipped);
         return (int)RB_OK;
@@ -171,21 +180,17 @@ int main(int argc, char** argv) {
         } else if (device_parse) {
             if (bed.empty()) return usage();
             if (stats_rows && largest) return usage();
-            const std::string bed_text = rbh::read_all(bed);
+            InputBytes bed_in;
+            input_bytes(bed, bed_in);
             mark("read_bed");
             rc = upload_paf(input);
             mark("device_parse_paf");
             if (rc == RB_OK) {
                 if (stats_rows) { fputs(rbh::stats_header(false).c_str(), stdout); fflush(stdout); }  // main.rs:51
-                rbh::Paf names;  // the batch's name table, interned in id order: BED rows get the batch's ids
-                for (uint32_t i = 0; i < info.n_names; i++)
-                    names.name_id(std::string(reinterpret_cast<const char*>(info.names) + info.names_off[i], (size_t)(info.names_off[i + 1] - info.names_off[i])));
-                rbh::Windows wins = rbh::Windows::pack_text(bed_text.data(), bed_text.size(), names);
-                mark("pack_bed");
-                const rb_windows w = wins.view();
+                rc = rb_batch_set_windows_bed(ctx, batch, bed_in.data, bed_in.n, nullptr);
+                mark("device_parse_bed");
                 const uint32_t want = (stats_rows ? RB_WANT_STATS_TEXT : RB_WANT_TEXT) | (largest ? RB_WANT_NUMERIC : 0u);
                 rb_lift_out out{};
-                rc = rb_batch_set_windows(ctx, batch, &w);
                 if (rc == RB_OK) rc = rb_batch_liftover(ctx, batch, policy, want, 0, nullptr);
                 if (rc == RB_OK) rc = rb_batch_download_lift(ctx, batch, want, &out, nullptr);
                 mark("rb_batch_liftover");
