@@ -268,6 +268,17 @@ int rb_batch_set_windows_bed(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint
  * valid until rb_batch_free or the next rb_batch_windows on the batch */
 int rb_batch_windows(rb_ctx* ctx, rb_batch* b, rb_windows* out);
 
+/* `rb liftover --bed` from the files' bytes: paf / bed = plain text or BGZF (rb_is_bgzf), as rb_batch_upload_paf /
+ * rb_batch_set_windows_bed take them.  On an N-device context the PAF is split into N byte ranges cut at line starts, and every
+ * device parses, tokenises and lifts its own lines (a PAF below multi_min_bytes, RB_MULTI_MIN_BYTES, stays on the first device). The
+ * rows are returned in the reference's emission order in one pinned block, laid out exactly as rb_liftover lays them out.  want:
+ * RB_WANT_TEXT / RB_WANT_NUMERIC / RB_WANT_STATS_TEXT as in rb_liftover; RB_WANT_QBED -> RB_ERR_BAD_ARG.  Errors, statuses and
+ * messages are those of the one-device batch path. Line numbers and record indices count over the whole file. infos are nullable;
+ * paf_info is filled once the PAF has parsed (also when a later step fails), bed_info on success; paf_info->names stays valid until
+ * the next call on ctx. */
+int rb_liftover_text(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, const uint8_t* bed, uint64_t bed_nbytes, int policy,
+                     uint32_t want, rb_lift_out* out, rb_stats_out* stats /* nullable */, rb_paf_info* paf_info, rb_bed_info* bed_info);
+
 /* ---- host helper: stable sort of BED rows by (t_id, st) into the rb_windows layout ----
  * perm_out[n_win] receives, for each sorted position, the BED row it came from. */
 int rb_sort_windows(uint32_t n_win, const uint32_t* t_id, const uint64_t* st, uint32_t* perm_out);

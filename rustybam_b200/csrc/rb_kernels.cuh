@@ -258,6 +258,14 @@ void launch_paf_pack(const uint8_t* text, uint64_t n_lines, PafLineCols L, const
                      uint8_t* names, uint64_t* rec_name_off, uint32_t* rec_qlen, cudaStream_t s);
 void launch_paf_copy_cg(const uint8_t* text, uint32_t n_rec, const uint64_t* cigar_off, const uint32_t* rec_line, const uint64_t* cg_off,
                         uint64_t cg_bytes, uint8_t* dst, cudaStream_t s);
+// rb_liftover_text on several devices (text_multi_kernels.cu).  *first = min(*first, offset of the first '\n' in text[0, n));
+// runs = 4 u64 tables of n_ranks entries (row start, row end, byte start, byte end of each contig's rows), zeroed by the caller;
+// a row's contig rank is rank_of[t_id[rec_idx - rec_base]]; rebase: line_off[row] += delta[its rank]
+void launch_first_newline(const uint8_t* text, uint64_t n, unsigned long long* first, cudaStream_t s);
+void launch_contig_runs(uint64_t n, const uint32_t* rec_idx, uint32_t rec_base, const uint32_t* t_id, const uint32_t* rank_of,
+                        const uint64_t* line_off, uint64_t out_bytes, uint64_t* runs, uint32_t n_ranks, cudaStream_t s);
+void launch_rebase_runs(uint64_t n, const uint32_t* rec_idx, uint32_t rec_base, const uint32_t* t_id, const uint32_t* rank_of,
+                        const uint64_t* delta, uint64_t* line_off, cudaStream_t s);
 // BED text -> the window tables of a batch (bed_parse_kernels.cu; the rules are bed_parse_core.cuh's).  Per-line columns:
 struct BedLineCols {
     const uint64_t* line_start;

@@ -23,6 +23,7 @@
 #include "paf_parse_core.cuh"
 #include "rb_kernels.cuh"
 #include "rec_core.cuh"
+#include "text_split.hpp"
 #include "trim_rounds.hpp"
 
 using namespace rb;
@@ -893,15 +894,21 @@ static int ensure_rec_buffers(rb_ctx* ctx, rb_batch* b, uint32_t n) {
 }
 
 // emission order (liftover.rs:151-164): contigs by first appearance of t_name, records in file order inside (file_order: the
-// identity); order[k] = the record emitted k-th, rank = its inverse
-static void emission_ranks(const uint32_t* tid, uint32_t n, uint32_t n_names, bool file_order, uint32_t* order, uint32_t* rank) {
-    std::vector<int64_t> first(n_names, -1);
-    std::vector<uint32_t> cnt;
+// identity); order[k] = the record emitted k-th, rank = its inverse.  contig_rank (nullable): the contigs' ranks by first appearance
+// in a larger file these records are part of (rb_liftover_text: one device's share), in place of their first appearance here.
+static void emission_ranks(const uint32_t* tid, uint32_t n, uint32_t n_names, bool file_order, const uint32_t* contig_rank, uint32_t* order,
+                           uint32_t* rank) {
+    std::vector<int64_t> first(contig_rank ? 0 : n_names, -1);
+    std::vector<uint32_t> cnt(contig_rank ? n_names : 0, 0);
     std::vector<uint32_t> grp(n);
     for (uint32_t i = 0; i < n; i++) {
-        int64_t& f = first[tid[i]];
-        if (f < 0) { f = (int64_t)cnt.size(); cnt.push_back(0); }
-        grp[i] = (uint32_t)f;
+        if (contig_rank) {
+            grp[i] = contig_rank[tid[i]];
+        } else {
+            int64_t& f = first[tid[i]];
+            if (f < 0) { f = (int64_t)cnt.size(); cnt.push_back(0); }
+            grp[i] = (uint32_t)f;
+        }
         cnt[grp[i]]++;
     }
     std::vector<uint32_t> start(cnt.size() + 1, 0);
@@ -978,7 +985,7 @@ static int upload_columns(rb_ctx* ctx, rb_batch* b, const rb_records* R, RecSel 
     uint32_t* s_order = reinterpret_cast<uint32_t*>(sp + o_order);
     uint32_t* s_rank = reinterpret_cast<uint32_t*>(sp + o_rank);
 
-    emission_ranks(h_tid, n, R->n_names, b->file_order, s_order, s_rank);
+    emission_ranks(h_tid, n, R->n_names, b->file_order, nullptr, s_order, s_rank);
     if (n) {
         CU(cudaMemcpyAsync(b->rec_order.p, s_order, (size_t)n * 4, cudaMemcpyHostToDevice, s));
         CU(cudaMemcpyAsync(b->rec_rank.p, s_rank, (size_t)n * 4, cudaMemcpyHostToDevice, s));
@@ -1557,8 +1564,8 @@ void rb_free_stats_out(rb_ctx*, rb_stats_out* st) {
 
 // ---- BGZF inflate (myio.rs:41-64: the `.bgz` reader) ----------------------------------------------
 // One table row per block from a hop over the headers (RFC 1952 + the 'BC' extra field of the SAM spec, 4.1); false if
-// `p` is not a well-formed series of BGZF blocks.
-static bool bgzf_blocks(const uint8_t* p, uint64_t n, std::vector<BgzfBlock>& blocks, uint64_t& total) {
+// `p` is not a well-formed series of BGZF blocks.  starts (nullable): where each row's block begins in `p`.
+static bool bgzf_blocks(const uint8_t* p, uint64_t n, std::vector<BgzfBlock>& blocks, uint64_t& total, std::vector<uint64_t>* starts = nullptr) {
     uint64_t pos = 0;
     total = 0;
     while (pos < n) {
@@ -1578,7 +1585,10 @@ static bool bgzf_blocks(const uint8_t* p, uint64_t n, std::vector<BgzfBlock>& bl
         b.cdata = xend; b.clen = (uint32_t)(bsize - xlen - 20); b.out_off = total;
         b.crc = le32(pos + bsize - 8); b.out_len = le32(pos + bsize - 4);
         if (b.out_len > 65536u) return false;  // (the format's bound; keeps a block's output offsets in 32 bits)
-        if (b.out_len) blocks.push_back(b);    // (the empty end-of-file marker block has nothing to inflate)
+        if (b.out_len) {                       // (the empty end-of-file marker block has nothing to inflate)
+            blocks.push_back(b);
+            if (starts) starts->push_back(pos);
+        }
         total += b.out_len;
         pos += bsize;
     }
@@ -1588,8 +1598,10 @@ int rb_is_bgzf(const uint8_t* data, uint64_t nbytes) {
     return data && nbytes >= 18 && data[0] == 0x1f && data[1] == 0x8b && data[2] == 8 && (data[3] & 4) && data[12] == 'B' && data[13] == 'C';
 }
 // The inflate step: block table, compressed bytes -> HBM, k_inflate_bgzf, CRC-32 / ISIZE verdict.  On RB_OK `out` holds the
-// `total` inflated bytes followed by `pad` bytes of head-room (the stream has been synchronised).
-static int inflate_to_device(rb_ctx* ctx, const uint8_t* bgzf, uint64_t nbytes, DevBuf& out, uint64_t& total, size_t pad) {
+// `total` inflated bytes followed by `pad` bytes of head-room (the stream has been synchronised).  block_base: blocks of the file in
+// front of `bgzf` (a share of a larger file), for the block numbers of the messages.
+static int inflate_to_device(rb_ctx* ctx, const uint8_t* bgzf, uint64_t nbytes, DevBuf& out, uint64_t& total, size_t pad,
+                             uint64_t block_base = 0) {
     std::vector<BgzfBlock> blocks;
     total = 0;
     if (!bgzf_blocks(bgzf, nbytes, blocks, total)) return fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: not a well-formed series of BGZF blocks");
@@ -1619,7 +1631,7 @@ static int inflate_to_device(rb_ctx* ctx, const uint8_t* bgzf, uint64_t nbytes, 
     release();
     if (e != cudaSuccess) { (void)cudaGetLastError(); return fail(ctx, RB_ERR_CUDA, "rb_inflate_bgzf: %s", cudaGetErrorString(e)); }
     if (h_err != ~0ull)
-        return fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: corrupt DEFLATE data in block %llu (code %u)", (unsigned long long)(h_err >> 8), (unsigned)(h_err & 0xFF));
+        return fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: corrupt DEFLATE data in block %llu (code %u)", (unsigned long long)((h_err >> 8) + block_base), (unsigned)(h_err & 0xFF));
     return RB_OK;
 }
 int rb_inflate_bgzf(rb_ctx* ctx, const uint8_t* bgzf, uint64_t nbytes, uint8_t** text, uint64_t* text_nbytes) {
@@ -1666,25 +1678,47 @@ struct DevScratch {  // device buffers of one call, released on every way out
     ~DevScratch() { for (DevBuf* d : bufs) d->release(); }
 };
 
-static int paf_upload_into(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64_t nbytes, rb_paf_info* info) {
+constexpr size_t TEXT_PAD = 4096;  // (16-byte loads of the last bytes)
+
+// the call's input -> text in HBM (`who` names the call in the messages)
+static int text_to_device(rb_ctx* ctx, const uint8_t* data, uint64_t nbytes, DevBuf& d_text, uint64_t& n, const char* who) {
+    n = 0;
+    if (rb_is_bgzf(data, nbytes)) return inflate_to_device(ctx, data, nbytes, d_text, n, TEXT_PAD);
+    if (nbytes >= 2 && data[0] == 0x1f && data[1] == 0x8b) return fail(ctx, RB_ERR_BAD_ARG, "%s: a plain gzip stream (not BGZF); inflate it first", who);
+    n = nbytes;
+    CU(d_text.ensure(n + TEXT_PAD));
+    if (n) CU(h2d_copy(d_text.p, data, n, ctx->stream));
+    return RB_OK;
+}
+
+// What the device parse of one text leaves for the host steps: counts, the first panic, the records' name bytes, then their ids.
+struct PafParsed {
+    uint64_t text_bytes = 0, n_lines = 0, cg_bytes = 0, panic = ~0ull;  // panic: (0-based line << 8) | LS_* of the first one
+    uint32_t n_rec = 0;
+    std::vector<uint64_t> noff;   // record r's names: bytes [noff[r], noff[r + 1]) of `names`, the query name's qlen[r] first
+    std::vector<uint32_t> qlen;
+    std::vector<char> names;
+    std::vector<uint32_t> ids;    // q ids, then t ids (paf_intern)
+};
+
+static int paf_panic(rb_ctx* ctx, uint64_t panic, uint64_t line_base) {
+    const unsigned long long line = (panic >> 8) + 1 + line_base;
+    switch ((uint32_t)(panic & 0xFF)) {
+        case rbpp::LS_FEW_COLUMNS: return fail(ctx, RB_ERR_REF_PAF_PARSE, "line %llu: assertion failed: t.len() >= 12", line);
+        case rbpp::LS_BAD_TAG: return fail(ctx, RB_ERR_REF_PAF_PARSE, "line %llu: assertion failed: PAF_TAG.is_match(token)", line);
+        default: return fail(ctx, RB_ERR_REF_CIGAR_PARSE, "line %llu: Unable to parse cigar string.", line);
+    }
+}
+
+// steps 1 - 3 of rb_batch_upload_paf on n bytes of text in HBM (16-byte aligned, TEXT_PAD bytes of head-room): lines, fields, scans,
+// the batch's columns and CIGAR text, the name bytes to the host.  A panic is left in p.panic (nothing is packed then).
+static int paf_parse_text(rb_ctx* ctx, rb_batch* b, const uint8_t* text, uint64_t n, PafParsed& p) {
     cudaStream_t s = ctx->stream;
     uint32_t* sc = ctx->scalars.as<uint32_t>();
     volatile uint64_t* hs = reinterpret_cast<volatile uint64_t*>(ctx->h_scalars);
-    DevBuf d_text, d_chunk, d_tws, d_part, d_lines, d_cols, d_rec;
-    DevScratch scratch{{&d_text, &d_chunk, &d_tws, &d_part, &d_lines, &d_cols, &d_rec}};
-    constexpr size_t TEXT_PAD = 4096;  // (16-byte loads of the last bytes)
-    uint64_t n = 0;
-    if (rb_is_bgzf(data, nbytes)) {
-        const int rc = inflate_to_device(ctx, data, nbytes, d_text, n, TEXT_PAD);
-        if (rc != RB_OK) return rc;
-    } else if (nbytes >= 2 && data[0] == 0x1f && data[1] == 0x8b) {
-        return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_upload_paf: a plain gzip stream (not BGZF); inflate it first");
-    } else {
-        n = nbytes;
-        CU(d_text.ensure(n + TEXT_PAD));
-        if (n) CU(h2d_copy(d_text.p, data, n, s));
-    }
-    const uint8_t* text = d_text.as<uint8_t>();
+    DevBuf d_chunk, d_tws, d_part, d_lines, d_cols, d_rec;
+    DevScratch scratch{{&d_chunk, &d_tws, &d_part, &d_lines, &d_cols, &d_rec}};
+    p.text_bytes = n;
     // 1. line starts: newline counts per 64 KiB, their scan, the starts; a last line without a terminator ends at n + 1 - 1
     uint64_t n_lines = 0;
     if (n) {
@@ -1751,20 +1785,16 @@ static int paf_upload_into(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64
     Publisher(ctx).u64(0, sc + SC_ERR_TOK).u64(1, rec_idx + nl).u64(2, cg_pos + nl).u64(3, name_pos + nl).go(s);
     CU(cudaStreamSynchronize(s));
     CU(cudaGetLastError());
-    const uint64_t panic = hs[0], n_rec64 = hs[1], cg_bytes = hs[2], name_bytes = hs[3];
-    if (panic != ~0ull) {
-        flush_times(ctx);
-        const unsigned long long line = (panic >> 8) + 1;
-        switch ((uint32_t)(panic & 0xFF)) {
-            case rbpp::LS_FEW_COLUMNS: return fail(ctx, RB_ERR_REF_PAF_PARSE, "line %llu: assertion failed: t.len() >= 12", line);
-            case rbpp::LS_BAD_TAG: return fail(ctx, RB_ERR_REF_PAF_PARSE, "line %llu: assertion failed: PAF_TAG.is_match(token)", line);
-            default: return fail(ctx, RB_ERR_REF_CIGAR_PARSE, "line %llu: Unable to parse cigar string.", line);
-        }
-    }
+    const uint64_t n_rec64 = hs[1], cg_bytes = hs[2], name_bytes = hs[3];
+    p.n_lines = nl;
+    p.panic = hs[0];
+    if (p.panic != ~0ull) { flush_times(ctx); return RB_OK; }
     const uint32_t n_rec = (uint32_t)n_rec64;
+    p.n_rec = n_rec; p.cg_bytes = cg_bytes;
     // 3. the batch's columns and CIGAR text
     b->n_rec = n_rec;
     b->rec_base = 0; b->byte_base = 0;
+    b->h_orig.clear();  // (a batch reused from rb_liftover may still map its rows to another call's records)
     b->invert = false;
     b->have_lift = b->have_stats = false;
     const size_t padded = text_layout(b, cg_bytes);
@@ -1790,37 +1820,47 @@ static int paf_upload_into(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64
     }
     const uint64_t tail0 = align_up(cg_bytes, 16);  // (k_paf_copy_cg wrote '0' up to here)
     CU(cudaMemsetAsync(raw + TEXT_FRONT_PAD + tail0, '0', padded - tail0, s));
-    // 4. names back to the host, interned, ids / names / emission order up again
+    // 4. the names back to the host (interned by paf_intern)
     b->h_cigar_off.resize((size_t)n_rec + 1);
-    std::vector<uint64_t> noff((size_t)n_rec + 1);
-    std::vector<uint32_t> qlen(n_rec);
-    std::vector<char> nbytes_h(name_bytes + 1);
+    p.noff.resize((size_t)n_rec + 1);
+    p.qlen.resize(n_rec);
+    p.names.resize(name_bytes + 1);
     CU(cudaMemcpyAsync(b->h_cigar_off.data(), b->cigar_off.p, ((size_t)n_rec + 1) * 8, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(noff.data(), rb + r_noff, ((size_t)n_rec + 1) * 8, cudaMemcpyDeviceToHost, s));
-    if (n_rec) CU(cudaMemcpyAsync(qlen.data(), rb + r_qlen, (size_t)n_rec * 4, cudaMemcpyDeviceToHost, s));
-    if (name_bytes) CU(cudaMemcpyAsync(nbytes_h.data(), rb + r_names, name_bytes, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(p.noff.data(), rb + r_noff, ((size_t)n_rec + 1) * 8, cudaMemcpyDeviceToHost, s));
+    if (n_rec) CU(cudaMemcpyAsync(p.qlen.data(), rb + r_qlen, (size_t)n_rec * 4, cudaMemcpyDeviceToHost, s));
+    if (name_bytes) CU(cudaMemcpyAsync(p.names.data(), rb + r_names, name_bytes, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     flush_times(ctx);
-    d_text.release(); d_cols.release(); d_lines.release();  // (before the host work: the text is not needed any more)
-    const char* nb = nbytes_h.data();
-    std::unordered_map<std::string, uint32_t> index;
-    b->h_names.clear();
-    b->h_names_off.assign(1, 0);
-    std::vector<uint32_t> h_ids((size_t)n_rec * 2);
+    return RB_OK;
+}
+
+// ids by first appearance, with the host reader's loop; `index` / names / names_off carry the table from one call to the next, so
+// the shares of one file interned in file order get the ids the whole file gets
+static void paf_intern(PafParsed& p, std::unordered_map<std::string, uint32_t>& index, std::vector<uint8_t>& names,
+                       std::vector<uint64_t>& names_off) {
+    const uint32_t n_rec = p.n_rec;
+    const char* nb = p.names.data();
+    p.ids.resize((size_t)n_rec * 2);
     rbn::intern_record_names(
-        n_rec, [&](size_t r) { return std::make_pair(nb + noff[r], (size_t)qlen[r]); },
-        [&](size_t r) { return std::make_pair(nb + noff[r] + qlen[r], (size_t)(noff[r + 1] - noff[r] - qlen[r])); },
-        [&](const char* p, size_t len) {
-            const auto ins = index.emplace(std::string(p, len), (uint32_t)(b->h_names_off.size() - 1));
+        n_rec, [&](size_t r) { return std::make_pair(nb + p.noff[r], (size_t)p.qlen[r]); },
+        [&](size_t r) { return std::make_pair(nb + p.noff[r] + p.qlen[r], (size_t)(p.noff[r + 1] - p.noff[r] - p.qlen[r])); },
+        [&](const char* q, size_t len) {
+            const auto ins = index.emplace(std::string(q, len), (uint32_t)(names_off.size() - 1));
             if (ins.second) {
-                b->h_names.insert(b->h_names.end(), p, p + len);
-                b->h_names_off.push_back(b->h_names.size());
+                names.insert(names.end(), q, q + len);
+                names_off.push_back(names.size());
             }
             return ins.first->second;
         },
-        h_ids.data(), h_ids.data() + n_rec);
-    const uint32_t n_names = (uint32_t)(b->h_names_off.size() - 1);
-    const uint64_t tbl_bytes = b->h_names.size();
+        p.ids.data(), p.ids.data() + n_rec);
+}
+
+// step 5: ids, the name table and the emission order up to the batch (asynchronous: b->busy)
+static int paf_upload_names(rb_ctx* ctx, rb_batch* b, const PafParsed& p, const uint8_t* names, const uint64_t* names_off, uint32_t n_names,
+                            const uint32_t* contig_rank) {
+    cudaStream_t s = ctx->stream;
+    const uint32_t n_rec = p.n_rec;
+    const uint64_t tbl_bytes = names_off[n_names];
     b->n_names = n_names;
     CU(b->names_off.ensure(((size_t)n_names + 1) * 8));
     CU(b->names.ensure(tbl_bytes + 8));
@@ -1829,10 +1869,10 @@ static int paf_upload_into(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64
                  s_end = s_rank + align_up((size_t)n_rec * 4, 64);
     CU(b->stage.ensure(s_end));
     uint8_t* sp = b->stage.p;
-    memcpy(sp + s_ids, h_ids.data(), (size_t)n_rec * 8);
-    memcpy(sp + s_noff, b->h_names_off.data(), ((size_t)n_names + 1) * 8);
-    if (tbl_bytes) memcpy(sp + s_names, b->h_names.data(), tbl_bytes);
-    emission_ranks(h_ids.data() + n_rec, n_rec, n_names, b->file_order, reinterpret_cast<uint32_t*>(sp + s_order),
+    memcpy(sp + s_ids, p.ids.data(), (size_t)n_rec * 8);
+    memcpy(sp + s_noff, names_off, ((size_t)n_names + 1) * 8);
+    if (tbl_bytes) memcpy(sp + s_names, names, tbl_bytes);
+    emission_ranks(p.ids.data() + n_rec, n_rec, n_names, b->file_order, contig_rank, reinterpret_cast<uint32_t*>(sp + s_order),
                    reinterpret_cast<uint32_t*>(sp + s_rank));
     if (n_rec) {
         CU(cudaMemcpyAsync(b->ids32.p, sp + s_ids, (size_t)n_rec * 8, cudaMemcpyHostToDevice, s));
@@ -1844,13 +1884,37 @@ static int paf_upload_into(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64
     b->busy = true;
     b->sum = rb_summary{};
     b->sum.cigar_bytes = b->n_bytes;
-    if (info) {
-        info->text_bytes = n; info->n_lines = nl; info->skipped = nl - n_rec;
-        info->n_rec = n_rec; info->n_names = n_names;
-        info->names = b->h_names.empty() ? nullptr : b->h_names.data();
-        info->names_off = b->h_names_off.data();
-        info->cigar_bytes = cg_bytes;
-    }
+    return RB_OK;
+}
+
+static void paf_fill_info(rb_paf_info* info, uint64_t text_bytes, uint64_t n_lines, uint64_t n_rec, const std::vector<uint8_t>& names,
+                          const std::vector<uint64_t>& names_off, uint64_t cg_bytes) {
+    if (!info) return;
+    info->text_bytes = text_bytes; info->n_lines = n_lines; info->skipped = n_lines - n_rec;
+    info->n_rec = (uint32_t)n_rec; info->n_names = (uint32_t)(names_off.size() - 1);
+    info->names = names.empty() ? nullptr : names.data();
+    info->names_off = names_off.data();
+    info->cigar_bytes = cg_bytes;
+}
+
+static int paf_upload_into(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64_t nbytes, rb_paf_info* info) {
+    DevBuf d_text;
+    DevScratch scratch{{&d_text}};
+    uint64_t n = 0;
+    int rc = text_to_device(ctx, data, nbytes, d_text, n, "rb_batch_upload_paf");
+    if (rc != RB_OK) return rc;
+    PafParsed p;
+    rc = paf_parse_text(ctx, b, d_text.as<uint8_t>(), n, p);
+    d_text.release();  // (before the host work: the text is not needed any more)
+    if (rc != RB_OK) return rc;
+    if (p.panic != ~0ull) return paf_panic(ctx, p.panic, 0);
+    std::unordered_map<std::string, uint32_t> index;
+    b->h_names.clear();
+    b->h_names_off.assign(1, 0);
+    paf_intern(p, index, b->h_names, b->h_names_off);
+    rc = paf_upload_names(ctx, b, p, b->h_names.data(), b->h_names_off.data(), (uint32_t)(b->h_names_off.size() - 1), nullptr);
+    if (rc != RB_OK) return rc;
+    paf_fill_info(info, n, p.n_lines, p.n_rec, b->h_names, b->h_names_off, p.cg_bytes);
     return RB_OK;
 }
 
@@ -1907,21 +1971,14 @@ static int bed_upload_into(rb_ctx* ctx, rb_batch* b, const uint8_t* data, uint64
     volatile uint64_t* hs = reinterpret_cast<volatile uint64_t*>(ctx->h_scalars);
     DevBuf d_text, d_chunk, d_part, d_lines, d_cols, d_tbl, d_rows, d_sort, d_ids;
     DevScratch scratch{{&d_text, &d_chunk, &d_part, &d_lines, &d_cols, &d_tbl, &d_rows, &d_sort, &d_ids}};
-    constexpr size_t TEXT_PAD = 4096;  // (16-byte loads of the last bytes)
     b->n_win = 0;
     b->wsrc = nullptr;
     b->general = false; b->default_ids = true; b->win_pending = false;
     b->have_lift = false;
     uint64_t n = 0;
-    if (rb_is_bgzf(data, nbytes)) {
-        const int rc = inflate_to_device(ctx, data, nbytes, d_text, n, TEXT_PAD);
+    {
+        const int rc = text_to_device(ctx, data, nbytes, d_text, n, "rb_batch_set_windows_bed");
         if (rc != RB_OK) return rc;
-    } else if (nbytes >= 2 && data[0] == 0x1f && data[1] == 0x8b) {
-        return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_set_windows_bed: a plain gzip stream (not BGZF); inflate it first");
-    } else {
-        n = nbytes;
-        CU(d_text.ensure(n + TEXT_PAD));
-        if (n) CU(h2d_copy(d_text.p, data, n, s));
     }
     const uint8_t* text = d_text.as<uint8_t>();
     // 1. line starts
@@ -2561,6 +2618,376 @@ static int stats_multi(rb_ctx* ctx, const rb_records* recs, rb_stats_out* stats)
     stats->id_by_all = reinterpret_cast<float*>(p + 9 * (size_t)n);
     stats->_owner = sblk;
     return RB_OK;
+}
+
+// ---- rb_liftover_text: PAF and BED bytes in, the rows of `rb liftover` out -----------------------------------------------------
+// One device (or a PAF below multi_min_bytes): rb_batch_upload_paf, rb_batch_set_windows_bed, rb_batch_liftover and the download on
+// the context's scratch batch.  D devices, one host thread each:
+//   split    plain text: D equal byte ranges, each uploaded by its own device; BGZF: runs of whole blocks balanced on ISIZE, each
+//            inflated by its own device.  k_first_newline finds each range's first '\n'; text_split.hpp says which bytes each device
+//            parses, and every device gathers them into a fresh buffer (its own bytes: a device copy; the others': peer copies).
+//   parse    steps 1 - 3 of rb_batch_upload_paf on every device at once; then the host interns the names device by device (file
+//            order: the ids of one device), ranks the contigs by first appearance in the whole file, and every device gets the
+//            global name table, its ids, the emission order (contig rank, file index) and rec_base = records on devices before it.
+//   windows  every device parses the whole BED against the same name table: identical tables and verdicts everywhere.
+//   lift     rb_batch_liftover everywhere (rec_idx always materialised); a lift error reports the smallest global record index.
+//   merge    global order = (contig rank, device): k_contig_runs finds each contig's rows on a device, the host lays out ONE pinned
+//            block, k_rebase_runs moves the line offsets and every device copies its (contig, device) cells into place — one copy
+//            per non-empty cell and output column.
+static int liftover_text_one(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, const uint8_t* bed, uint64_t bed_nbytes, int policy,
+                             uint32_t want, rb_lift_out* out, rb_stats_out* stats, rb_paf_info* paf_info, rb_bed_info* bed_info) {
+    if (!ctx->scratch) ctx->scratch = new rb_batch();
+    rb_batch* b = ctx->scratch;
+    if (b->busy) { CU(cudaStreamSynchronize(ctx->stream)); b->busy = false; }
+    int rc = paf_upload_into(ctx, b, paf, paf_nbytes, paf_info);
+    if (rc == RB_OK && cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+        (void)cudaGetLastError();
+        rc = fail(ctx, RB_ERR_CUDA, "upload failed");
+    }
+    b->busy = false;
+    if (rc == RB_OK) rc = bed_upload_into(ctx, b, bed, bed_nbytes, bed_info);
+    if (rc == RB_OK) rc = rb_batch_liftover(ctx, b, policy, want, stats != nullptr, nullptr);
+    if (rc == RB_OK) rc = rb_batch_download_lift(ctx, b, want, out, stats);
+    if (rc != RB_OK) {
+        cudaStreamSynchronize(ctx->stream);
+        b->busy = false;
+        b->n_win = 0; b->general = false; b->win_pending = false; b->have_lift = false;
+        flush_times(ctx);
+    }
+    return rc;
+}
+
+static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, const uint8_t* bed, uint64_t bed_nbytes, int policy,
+                               uint32_t want, rb_lift_out* out, rb_stats_out* stats, rb_paf_info* paf_info, rb_bed_info* bed_info) {
+    const int D = 1 + (int)ctx->peers.size();
+    std::vector<rb_ctx*> cs(1, ctx);
+    cs.insert(cs.end(), ctx->peers.begin(), ctx->peers.end());
+    // 1. the input's byte ranges
+    const bool bgzf = rb_is_bgzf(paf, paf_nbytes) != 0;
+    if (!bgzf && paf_nbytes >= 2 && paf[0] == 0x1f && paf[1] == 0x8b)
+        return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_upload_paf: a plain gzip stream (not BGZF); inflate it first");
+    std::vector<uint64_t> src((size_t)D + 1, paf_nbytes), blk_base((size_t)D, 0);
+    src[0] = 0;
+    if (bgzf) {
+        std::vector<BgzfBlock> blocks;
+        std::vector<uint64_t> starts;
+        uint64_t total = 0;
+        if (!bgzf_blocks(paf, paf_nbytes, blocks, total, &starts)) return fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: not a well-formed series of BGZF blocks");
+        size_t k = 0;
+        for (int d = 1; d < D; d++) {
+            const uint64_t target = total / (uint64_t)D * (uint64_t)d + total % (uint64_t)D * (uint64_t)d / (uint64_t)D;
+            while (k < blocks.size() && blocks[k].out_off < target) k++;
+            src[(size_t)d] = k < blocks.size() ? starts[k] : paf_nbytes;
+            blk_base[(size_t)d] = k;
+        }
+    } else {
+        for (int d = 1; d < D; d++) src[(size_t)d] = paf_nbytes / (uint64_t)D * (uint64_t)d + paf_nbytes % (uint64_t)D * (uint64_t)d / (uint64_t)D;
+    }
+    const uint32_t want_lift = want | RB_WANT_NUMERIC;  // (rec_idx places the rows)
+    const bool want_text = (want & (RB_WANT_TEXT | RB_WANT_STATS_TEXT)) != 0, want_num = (want & RB_WANT_NUMERIC) != 0;
+
+    struct Dev {
+        int rc = RB_OK;
+        DevBuf range, own, rank, runs_d, delta;
+        uint64_t n = 0, first_nl = rbt::NO_NEWLINE, rec_base = 0;
+        uint8_t last = 0;  // the range's last byte
+        PafParsed p;
+        rb_bed_info bi{};
+        rb_summary sum{};
+        std::vector<uint64_t> runs;            // row lo / row hi / byte lo / byte hi per contig rank
+        std::vector<uint64_t> at_row, at_byte; // where each of its cells goes in the merged output
+    };
+    std::vector<Dev> dv((size_t)D);
+    Rendezvous rv(D);
+    std::vector<rbt::Owned> plan;
+    std::vector<uint32_t> rank_of;  // name id -> contig rank (first appearance as t_name in the file)
+    uint32_t n_ranks = 0, n_names = 0;
+    rb_batch* b0 = ctx->scratch ? ctx->scratch : (ctx->scratch = new rb_batch());
+    PinnedBlock *blk = nullptr, *sblk = nullptr;
+    uint8_t* base = nullptr;
+    size_t o_text = 64, o_loff = 0, o_num = 0;
+    uint64_t tot_rows = 0, tot_bytes = 0, tot_pairs = 0;
+    int call_rc = RB_OK;
+    // the first failing device in device order (lift errors: the smallest global record index) fails the call
+    auto first_error = [&](bool by_record) {
+        uint64_t best = UINT64_MAX;
+        for (int k = 0; k < D; k++) {
+            if (dv[(size_t)k].rc == RB_OK) continue;
+            if (call_rc == RB_OK || (by_record && cs[(size_t)k]->err_rec < best)) {
+                call_rc = dv[(size_t)k].rc;
+                best = cs[(size_t)k]->err_rec;
+                if (k) ctx->err = cs[(size_t)k]->err;
+            }
+            if (!by_record) return;
+        }
+    };
+
+    auto work = [&](int d) {
+        rb_ctx* c = cs[(size_t)d];
+        Dev& me = dv[(size_t)d];
+        cudaSetDevice(c->device);
+        c->err.clear(); c->err_rec = UINT64_MAX;
+        if (!c->scratch) c->scratch = new rb_batch();
+        rb_batch* b = c->scratch;
+        cudaStream_t s = c->stream;
+        uint32_t* sc = c->scalars.as<uint32_t>();
+        volatile uint64_t* hs = reinterpret_cast<volatile uint64_t*>(c->h_scalars);
+        auto finish = [&] {
+            if (b->busy) { cudaStreamSynchronize(s); b->busy = false; }
+            me.range.release(); me.own.release(); me.rank.release(); me.runs_d.release(); me.delta.release();
+        };
+        // 1. this device's range -> HBM, its first '\n'
+        me.rc = [&]() -> int {
+            rb_ctx* ctx = c;  // (CU reports into this device's context)
+            if (b->busy) { CU(cudaStreamSynchronize(s)); b->busy = false; }
+            const uint64_t len = src[(size_t)d + 1] - src[(size_t)d];
+            if (bgzf) {
+                const int rc = inflate_to_device(c, paf + src[(size_t)d], len, me.range, me.n, TEXT_PAD, blk_base[(size_t)d]);
+                if (rc != RB_OK) return rc;
+            } else {
+                me.n = len;
+                CU(me.range.ensure(len + TEXT_PAD));
+                if (len) CU(h2d_copy(me.range.p, paf + src[(size_t)d], len, s));
+            }
+            if (me.n) {
+                CU(cudaMemsetAsync(sc + SC_ERR_TOK, 0xFF, 8, s));
+                {
+                    KScope k(c, "k_first_newline");
+                    launch_first_newline(me.range.as<uint8_t>(), me.n, reinterpret_cast<unsigned long long*>(sc + SC_ERR_TOK), s);
+                }
+                Publisher(c).u64(0, sc + SC_ERR_TOK).go(s);
+            }
+            CU(cudaStreamSynchronize(s));
+            if (me.n) {
+                me.first_nl = hs[0];
+                CU(cudaMemcpy(&me.last, me.range.as<uint8_t>() + me.n - 1, 1, cudaMemcpyDeviceToHost));
+            }
+            return RB_OK;
+        }();
+        rv.meet([&] {
+            first_error(false);
+            if (call_rc != RB_OK) return;
+            std::vector<uint64_t> size((size_t)D), nl((size_t)D);
+            std::vector<uint8_t> ends_nl((size_t)D);
+            for (int k = 0; k < D; k++) {
+                size[(size_t)k] = dv[(size_t)k].n; nl[(size_t)k] = dv[(size_t)k].first_nl;
+                ends_nl[(size_t)k] = dv[(size_t)k].n && dv[(size_t)k].last == '\n';
+            }
+            plan = rbt::plan_line_split(size, nl, ends_nl);
+        });
+        if (call_rc != RB_OK) { finish(); return; }
+        // 2. the lines this device owns -> one fresh buffer
+        me.rc = [&]() -> int {
+            rb_ctx* ctx = c;  // (CU reports into this device's context)
+            const rbt::Owned& o = plan[(size_t)d];
+            CU(me.own.ensure(o.bytes + TEXT_PAD));
+            uint64_t at = 0;
+            for (const rbt::Piece& pc : o.pieces) {
+                const Dev& from = dv[(size_t)pc.src];
+                if (pc.src == d) CU(cudaMemcpyAsync(me.own.as<uint8_t>() + at, from.range.as<uint8_t>() + pc.off, pc.len, cudaMemcpyDeviceToDevice, s));
+                else CU(cudaMemcpyPeerAsync(me.own.as<uint8_t>() + at, c->device, from.range.as<uint8_t>() + pc.off, cs[(size_t)pc.src]->device, pc.len, s));
+                at += pc.len;
+            }
+            CU(cudaStreamSynchronize(s));
+            return RB_OK;
+        }();
+        rv.meet([&] { first_error(false); });  // (every copy out of the ranges has finished)
+        me.range.release();
+        if (call_rc != RB_OK) { finish(); return; }
+        // 3. parse
+        me.rc = paf_parse_text(c, b, me.own.as<uint8_t>(), plan[(size_t)d].bytes, me.p);
+        me.own.release();
+        rv.meet([&] {
+            uint64_t lines = 0, recs = 0, text = 0, cg = 0;
+            for (int k = 0; k < D; k++) {  // the first error or panic in file order
+                Dev& o = dv[(size_t)k];
+                if (o.rc != RB_OK) { call_rc = o.rc; if (k) ctx->err = cs[(size_t)k]->err; return; }
+                if (o.p.panic != ~0ull) { call_rc = paf_panic(ctx, o.p.panic, lines); return; }
+                o.rec_base = recs;
+                lines += o.p.n_lines; recs += o.p.n_rec; text += o.p.text_bytes; cg += o.p.cg_bytes;
+            }
+            if (lines > 0xFFFFFFFFull) { call_rc = fail(ctx, RB_ERR_REF_PAF_PARSE, "more than 2^32 lines"); return; }
+            std::unordered_map<std::string, uint32_t> index;
+            b0->h_names.clear();
+            b0->h_names_off.assign(1, 0);
+            for (int k = 0; k < D; k++) paf_intern(dv[(size_t)k].p, index, b0->h_names, b0->h_names_off);
+            n_names = (uint32_t)(b0->h_names_off.size() - 1);
+            rank_of.assign(n_names, UINT32_MAX);
+            for (int k = 0; k < D; k++) {
+                const PafParsed& q = dv[(size_t)k].p;
+                for (uint32_t r = 0; r < q.n_rec; r++) {
+                    const uint32_t t = q.ids[(size_t)q.n_rec + r];
+                    if (rank_of[t] == UINT32_MAX) rank_of[t] = n_ranks++;
+                }
+            }
+            for (uint32_t& r : rank_of) if (r == UINT32_MAX) r = 0;  // (query-only names: never looked up)
+            paf_fill_info(paf_info, text, lines, recs, b0->h_names, b0->h_names_off, cg);
+        });
+        if (call_rc != RB_OK) { finish(); return; }
+        // 4. names, windows, lift, the contig runs of the rows
+        me.rc = [&]() -> int {
+            rb_ctx* ctx = c;  // (CU reports into this device's context)
+            int rc = paf_upload_names(c, b, me.p, b0->h_names.data(), b0->h_names_off.data(), n_names, rank_of.data());
+            if (rc != RB_OK) return rc;
+            b->rec_base = (uint32_t)me.rec_base;
+            CU(cudaStreamSynchronize(s));
+            b->busy = false;
+            rc = bed_upload_into(c, b, bed, bed_nbytes, &me.bi);
+            if (rc != RB_OK || b->n_rec == 0) return rc;
+            rc = rb_batch_liftover(c, b, policy, want_lift, stats != nullptr, &me.sum);
+            if (rc != RB_OK) return rc;
+            const uint64_t nk = me.sum.n_out, sk = b->row_stride ? b->row_stride : nk;
+            CU(me.rank.ensure((size_t)n_names * 4 + 8));
+            CU(me.runs_d.ensure((size_t)n_ranks * 32 + 64));
+            if (n_names) CU(cudaMemcpyAsync(me.rank.p, rank_of.data(), (size_t)n_names * 4, cudaMemcpyHostToDevice, s));
+            CU(cudaMemsetAsync(me.runs_d.p, 0, (size_t)n_ranks * 32, s));
+            {
+                KScope k(c, "k_contig_runs");
+                launch_contig_runs(nk, reinterpret_cast<const uint32_t*>(b->out_num.as<uint64_t>() + 6 * sk), b->rec_base,
+                                   b->ids32.as<uint32_t>() + b->n_rec, me.rank.as<uint32_t>(), want_text ? b->out_line_off.as<uint64_t>() : nullptr,
+                                   me.sum.out_bytes, me.runs_d.as<uint64_t>(), n_ranks, s);
+            }
+            me.runs.resize((size_t)n_ranks * 4);
+            if (n_ranks) CU(cudaMemcpyAsync(me.runs.data(), me.runs_d.p, (size_t)n_ranks * 32, cudaMemcpyDeviceToHost, s));
+            CU(cudaStreamSynchronize(s));
+            flush_times(c);
+            return RB_OK;
+        }();
+        auto layout = [&] {  // everybody's runs are known: lay out the one output block, cells in (contig rank, device) order
+            first_error(true);
+            if (call_rc != RB_OK) return;
+            for (int k = 0; k < D; k++) {
+                dv[(size_t)k].at_row.assign(n_ranks, 0); dv[(size_t)k].at_byte.assign(n_ranks, 0);
+                tot_pairs += dv[(size_t)k].sum.n_pairs;
+            }
+            for (uint32_t r = 0; r < n_ranks; r++)
+                for (int k = 0; k < D; k++) {
+                    Dev& o = dv[(size_t)k];
+                    if (o.runs.empty()) continue;
+                    o.at_row[r] = tot_rows; o.at_byte[r] = tot_bytes;
+                    tot_rows += o.runs[n_ranks + r] - o.runs[r];
+                    tot_bytes += o.runs[3 * (size_t)n_ranks + r] - o.runs[2 * (size_t)n_ranks + r];
+                }
+            uint64_t rows = 0;
+            for (int k = 0; k < D; k++) rows += dv[(size_t)k].sum.n_out;
+            if (!want_text)  // (no line offsets: the byte count is the devices' sum, as out->paf_nbytes of rb_liftover reports it)
+                for (int k = 0; k < D; k++) tot_bytes += dv[(size_t)k].sum.out_bytes;
+            if (rows != tot_rows) { call_rc = fail(ctx, RB_ERR_CUDA, "rb_liftover_text: the rows of a device are not grouped by contig"); return; }
+            const size_t text_room = want_text ? align_up(tot_bytes + 1, 64) : 0;
+            const size_t loff_bytes = want_text ? align_up((tot_rows + 1) * 8, 64) : 0;
+            const size_t num_bytes = want_num ? align_up(tot_rows * 56, 64) : 0;
+            blk = pinned_get(ctx, 64 + text_room + loff_bytes + num_bytes);
+            if (stats) sblk = pinned_get(ctx, (size_t)tot_rows * 40 + 64);
+            if (!blk || (stats && !sblk)) { call_rc = fail(ctx, RB_ERR_OOM, "pinned allocation of the merged output failed"); return; }
+            base = reinterpret_cast<uint8_t*>(blk->p);
+            o_loff = 64 + text_room;
+            o_num = o_loff + loff_bytes;
+        };
+        rv.meet([&] {
+            cudaSetDevice(ctx->device);  // (the pinned pool belongs to the first device's context)
+            layout();
+            cudaSetDevice(c->device);
+        });
+        if (call_rc != RB_OK) { finish(); return; }
+        // 5. this device's cells -> their places in the merged output
+        me.rc = [&]() -> int {
+            rb_ctx* ctx = c;  // (CU reports into this device's context)
+            const uint64_t nk = me.sum.n_out, sk = b->row_stride ? b->row_stride : nk, cap = tot_rows;
+            if (me.runs.empty() || nk == 0) return RB_OK;
+            const uint32_t* rec_idx = reinterpret_cast<const uint32_t*>(b->out_num.as<uint64_t>() + 6 * sk);
+            const uint64_t* runs = me.runs.data();
+            if (want_text) {
+                std::vector<uint64_t> delta(n_ranks, 0);
+                for (uint32_t r = 0; r < n_ranks; r++) delta[r] = me.at_byte[r] - runs[2 * (size_t)n_ranks + r];
+                CU(me.delta.ensure((size_t)n_ranks * 8 + 8));
+                CU(cudaMemcpyAsync(me.delta.p, delta.data(), (size_t)n_ranks * 8, cudaMemcpyHostToDevice, s));  // (pageable: staged before the call returns)
+                KScope k(c, "k_rebase_runs");
+                launch_rebase_runs(nk, rec_idx, b->rec_base, b->ids32.as<uint32_t>() + b->n_rec, me.rank.as<uint32_t>(), me.delta.as<uint64_t>(),
+                                   b->out_line_off.as<uint64_t>(), s);
+            }
+            for (uint32_t r = 0; r < n_ranks; r++) {
+                const uint64_t lo = runs[r], hi = runs[n_ranks + r], blo = runs[2 * (size_t)n_ranks + r], bhi = runs[3 * (size_t)n_ranks + r];
+                if (hi <= lo) continue;
+                const uint64_t rows = hi - lo, at = me.at_row[r];
+                if (want_text) {
+                    if (bhi > blo) CU(cudaMemcpyAsync(base + o_text + me.at_byte[r], b->out_text.as<uint8_t>() + blo, bhi - blo, cudaMemcpyDeviceToHost, s));
+                    CU(cudaMemcpyAsync(reinterpret_cast<uint64_t*>(base + o_loff) + at, b->out_line_off.as<uint64_t>() + lo, rows * 8, cudaMemcpyDeviceToHost, s));
+                }
+                if (want_num) {
+                    uint64_t* dn = reinterpret_cast<uint64_t*>(base + o_num);
+                    const uint64_t* sp = b->out_num.as<uint64_t>();
+                    CU(cudaMemcpy2DAsync(dn + at, cap * 8, sp + lo, sk * 8, rows * 8, 6, cudaMemcpyDeviceToHost, s));
+                    CU(cudaMemcpy2DAsync(reinterpret_cast<uint32_t*>(dn + 6 * cap) + at, cap * 4, reinterpret_cast<const uint32_t*>(sp + 6 * sk) + lo,
+                                         sk * 4, rows * 4, 2, cudaMemcpyDeviceToHost, s));
+                }
+                if (stats)
+                    CU(cudaMemcpy2DAsync(reinterpret_cast<uint32_t*>(sblk->p) + at, cap * 4, b->out_stats.as<uint32_t>() + lo, sk * 4, rows * 4, 10,
+                                         cudaMemcpyDeviceToHost, s));
+            }
+            CU(cudaStreamSynchronize(s));
+            flush_times(c);
+            return RB_OK;
+        }();
+        finish();
+    };
+    std::vector<std::thread> pool;
+    for (int d = 1; d < D; d++) pool.emplace_back(work, d);
+    work(0);
+    for (auto& th : pool) th.join();
+    cudaSetDevice(ctx->device);
+    auto release = [&] { if (blk) blk->in_use = false; if (sblk) sblk->in_use = false; };
+    if (call_rc == RB_OK) first_error(false);
+    if (call_rc != RB_OK) { release(); return call_rc; }
+    if (bed_info) *bed_info = dv[0].bi;
+    out->n_out = tot_rows; out->paf_nbytes = tot_bytes; out->n_pairs = tot_pairs; out->_owner = blk;
+    if (want_text) {
+        out->paf_text = base + o_text;
+        out->line_off = reinterpret_cast<uint64_t*>(base + o_loff);
+        out->line_off[tot_rows] = tot_bytes;
+        out->paf_text[tot_bytes] = 0;
+    }
+    if (want_num) {
+        uint64_t* p = reinterpret_cast<uint64_t*>(base + o_num);
+        const uint64_t c = tot_rows;
+        out->q_st = p; out->q_en = p + c; out->t_st = p + 2 * c; out->t_en = p + 3 * c; out->nmatch = p + 4 * c; out->aln_len = p + 5 * c;
+        out->rec_idx = reinterpret_cast<uint32_t*>(p + 6 * c);
+        out->win_idx = out->rec_idx + c;
+    }
+    if (stats) {
+        uint32_t* p = reinterpret_cast<uint32_t*>(sblk->p);
+        const uint64_t c = tot_rows;
+        stats->n = tot_rows;
+        stats->equal = p; stats->diff = p + c; stats->ins = p + 2 * c; stats->del = p + 3 * c; stats->ins_events = p + 4 * c;
+        stats->del_events = p + 5 * c; stats->matches = p + 6 * c;
+        stats->id_by_matches = reinterpret_cast<float*>(p + 7 * c); stats->id_by_events = reinterpret_cast<float*>(p + 8 * c);
+        stats->id_by_all = reinterpret_cast<float*>(p + 9 * c);
+        stats->_owner = sblk;
+    }
+    return RB_OK;
+}
+
+int rb_liftover_text(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, const uint8_t* bed, uint64_t bed_nbytes, int policy,
+                     uint32_t want, rb_lift_out* out, rb_stats_out* stats, rb_paf_info* paf_info, rb_bed_info* bed_info) {
+    if (!ctx) return RB_ERR_NO_DEVICE;
+    if (paf_info) memset(paf_info, 0, sizeof *paf_info);
+    if (bed_info) memset(bed_info, 0, sizeof *bed_info);
+    if (!out) return fail(ctx, RB_ERR_BAD_ARG, "out is null");
+    memset(out, 0, sizeof *out);
+    if (stats) memset(stats, 0, sizeof *stats);
+    if ((!paf && paf_nbytes) || (!bed && bed_nbytes)) return fail(ctx, RB_ERR_BAD_ARG, "rb_liftover_text: null data");
+    if (want & RB_WANT_QBED) return fail(ctx, RB_ERR_BAD_ARG, "rb_liftover_text: RB_WANT_QBED is not supported");
+    if (policy != RB_POLICY_RIGHTMOST && policy != RB_POLICY_EARLY_EXIT) return fail(ctx, RB_ERR_BAD_ARG, "unknown policy %d", policy);
+    if ((want & RB_WANT_STATS_TEXT) && (want & RB_WANT_TEXT)) return fail(ctx, RB_ERR_BAD_ARG, "RB_WANT_STATS_TEXT and RB_WANT_TEXT exclude each other");
+    cudaSetDevice(ctx->device);
+    if (ctx->peers.empty() || paf_nbytes < ctx->multi_min_bytes)
+        return liftover_text_one(ctx, paf, paf_nbytes, bed, bed_nbytes, policy, want, out, stats, paf_info, bed_info);
+    const int rc = liftover_text_multi(ctx, paf, paf_nbytes, bed, bed_nbytes, policy, want, out, stats, paf_info, bed_info);
+    if (rc != RB_OK) {
+        if (paf_info && !paf_info->names_off) memset(paf_info, 0, sizeof *paf_info);
+        memset(out, 0, sizeof *out);
+        if (stats) memset(stats, 0, sizeof *stats);
+    }
+    return rc;
 }
 
 // ---- rb_liftover in slices, on one device or several ------------------------------------------------

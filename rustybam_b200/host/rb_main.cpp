@@ -111,12 +111,12 @@ int main(int argc, char** argv) {
         }
         return rbh::Paf::from_file(path);
     };
-    // RB_DEVICE_PARSE=1: `rb liftover` (plain, --stats, --largest) and `rb stats --paf` on one GPU hand the file's bytes to
-    // rb_batch_upload_paf — lines are split and parsed on the device — instead of parsing them on the host; `rb liftover` hands the
-    // BED's bytes to rb_batch_set_windows_bed the same way.  A plain file is mapped, a .bgz / .gz that is BGZF goes as it is
+    // RB_DEVICE_PARSE=1: `rb [--gpus N] liftover` (plain, --stats, --largest) hands the bytes of the PAF and the BED to one
+    // rb_liftover_text call — lines are split and parsed on the device(s) — instead of parsing them on the host; `rb stats --paf` on
+    // one GPU hands the PAF's bytes to rb_batch_upload_paf.  A plain file is mapped, a .bgz / .gz that is BGZF goes as it is
     // (inflated on the device), a plain .gz and stdin are inflated / read by rbh::read_all first.
     const char* dp = getenv("RB_DEVICE_PARSE");
-    const bool device_parse = dp && dp[0] == '1' && n_gpus == 1 && !qbed && (cmd == "liftover" || cmd == "stats");
+    const bool device_parse = dp && dp[0] == '1' && !qbed && (cmd == "liftover" || (cmd == "stats" && n_gpus == 1));
     rb_batch* batch = nullptr;
     rb_paf_info info{};
     struct InputBytes {
@@ -183,28 +183,29 @@ int main(int argc, char** argv) {
             InputBytes bed_in;
             input_bytes(bed, bed_in);
             mark("read_bed");
-            rc = upload_paf(input);
-            mark("device_parse_paf");
-            if (rc == RB_OK) {
+            const uint32_t want = (stats_rows ? RB_WANT_STATS_TEXT : RB_WANT_TEXT) | (largest ? RB_WANT_NUMERIC : 0u);
+            rb_lift_out out{};
+            rb_paf_info pinfo{};
+            {
+                InputBytes paf_in;
+                input_bytes(input, paf_in);
+                rc = rb_liftover_text(ctx, paf_in.data, paf_in.n, bed_in.data, bed_in.n, policy, want, &out, nullptr, &pinfo, nullptr);
+            }
+            mark("rb_liftover_text");
+            if (pinfo.names_off) {  // the PAF parsed
+                if (pinfo.skipped) fprintf(stderr, "\nUnable to parse %zu PAF record(s). Skipped.\n", (size_t)pinfo.skipped);
                 if (stats_rows) { fputs(rbh::stats_header(false).c_str(), stdout); fflush(stdout); }  // main.rs:51
-                rc = rb_batch_set_windows_bed(ctx, batch, bed_in.data, bed_in.n, nullptr);
-                mark("device_parse_bed");
-                const uint32_t want = (stats_rows ? RB_WANT_STATS_TEXT : RB_WANT_TEXT) | (largest ? RB_WANT_NUMERIC : 0u);
-                rb_lift_out out{};
-                if (rc == RB_OK) rc = rb_batch_liftover(ctx, batch, policy, want, 0, nullptr);
-                if (rc == RB_OK) rc = rb_batch_download_lift(ctx, batch, want, &out, nullptr);
-                mark("rb_batch_liftover");
-                if (rc == RB_OK) {
-                    if (largest) {  // main.rs:200-208
-                        const std::string rows = rbh::largest_rows(out);
-                        fwrite(rows.data(), 1, rows.size(), stdout);
-                    } else {
-                        fwrite(out.paf_text, 1, out.paf_nbytes, stdout);
-                    }
-                    fflush(stdout);
-                    mark("write");
-                    rb_free_lift_out(ctx, &out);
+            }
+            if (rc == RB_OK) {
+                if (largest) {  // main.rs:200-208
+                    const std::string rows = rbh::largest_rows(out);
+                    fwrite(rows.data(), 1, rows.size(), stdout);
+                } else {
+                    fwrite(out.paf_text, 1, out.paf_nbytes, stdout);
                 }
+                fflush(stdout);
+                mark("write");
+                rb_free_lift_out(ctx, &out);
             }
         } else if (cmd == "stats") {
             fputs(rbh::stats_header(qbed).c_str(), stdout);  // printed before the input is read (main.rs:51)
