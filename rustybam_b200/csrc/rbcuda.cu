@@ -410,6 +410,99 @@ NumDev num_view(const rb_batch* b, uint64_t n) {
     return d;
 }
 
+// The pinned output of a call.  Rows block: a 64-byte front, the text, (rows + 1) line offsets and the numeric columns (6 x u64,
+// then 2 x u32 per row: 56 B).  Stats block: the 10 columns of rb_stats_out (40 B per row).  Columns sit `cap` rows apart.
+struct RowsOut {
+    PinnedBlock *blk = nullptr, *sblk = nullptr;
+    uint64_t cap = 0;
+    size_t cap_text = 0;  // text bytes the rows block has room for
+    size_t o_loff = 0, o_num = 0;
+    bool text = false, num = false;
+
+    int reserve(rb_ctx* ctx, uint64_t cap_rows, size_t text_bytes, uint32_t want, bool with_stats) {
+        text = (want & (RB_WANT_TEXT | RB_WANT_STATS_TEXT)) != 0;  // (stats rows are the text)
+        num = (want & RB_WANT_NUMERIC) != 0;
+        cap = cap_rows;
+        const size_t loff = text ? align_up((cap + 1) * 8, 64) : 0, nums = num ? align_up(cap * 56, 64) : 0;
+        const size_t need = 64 + (text ? align_up(text_bytes + 1, 64) : 0) + loff + nums;
+        blk = pinned_get(ctx, need);
+        if (!blk) return fail(ctx, RB_ERR_OOM, "pinned allocation of %zu bytes failed", need);
+        o_loff = 64 + (blk->cap - 64 - loff - nums) / 64 * 64;  // the text gets every byte the block has beyond the tables
+        o_num = o_loff + loff;
+        cap_text = text ? o_loff - 128 : 0;
+        return with_stats ? reserve_stats(ctx, cap_rows) : RB_OK;
+    }
+    int reserve_stats(rb_ctx* ctx, uint64_t cap_rows) {
+        cap = cap_rows;
+        const size_t need = (size_t)cap * 40 + 64;
+        sblk = pinned_get(ctx, need);
+        if (!sblk) { release(); return fail(ctx, RB_ERR_OOM, "pinned allocation of %zu bytes failed", need); }
+        return RB_OK;
+    }
+    // enqueue on `s`: rows [row_lo, row_lo + n_rows) of batch b (text bytes [byte_lo, byte_lo + n_bytes)) -> output rows from at_row
+    // (text from at_byte).  The line offsets travel as they are on the device: rebasing them is the caller's.
+    int copy_rows(rb_ctx* ctx, const rb_batch* b, uint64_t row_lo, uint64_t n_rows, uint64_t byte_lo, uint64_t n_bytes, uint64_t at_row,
+                  uint64_t at_byte, cudaStream_t s) const {
+        // device columns: row_stride apart after a liftover (0: n_out); without a rows block, rb_batch_stats' one row per record
+        const uint64_t sk = !blk ? b->n_rec : b->row_stride ? b->row_stride : b->sum.n_out;
+        uint8_t* base = blk ? static_cast<uint8_t*>(blk->p) : nullptr;
+        if (text) {
+            if (n_bytes) CU(cudaMemcpyAsync(base + 64 + at_byte, b->out_text.as<uint8_t>() + byte_lo, n_bytes, cudaMemcpyDeviceToHost, s));
+            if (n_rows)
+                CU(cudaMemcpyAsync(reinterpret_cast<uint64_t*>(base + o_loff) + at_row, b->out_line_off.as<uint64_t>() + row_lo, n_rows * 8,
+                                   cudaMemcpyDeviceToHost, s));
+        }
+        if (!n_rows) return RB_OK;
+        if (num) {  // one strided copy per table
+            uint64_t* dn = reinterpret_cast<uint64_t*>(base + o_num);
+            const uint64_t* sp = b->out_num.as<uint64_t>();
+            CU(cudaMemcpy2DAsync(dn + at_row, cap * 8, sp + row_lo, sk * 8, n_rows * 8, 6, cudaMemcpyDeviceToHost, s));
+            CU(cudaMemcpy2DAsync(reinterpret_cast<uint32_t*>(dn + 6 * cap) + at_row, cap * 4, reinterpret_cast<const uint32_t*>(sp + 6 * sk) + row_lo,
+                                 sk * 4, n_rows * 4, 2, cudaMemcpyDeviceToHost, s));
+        }
+        if (sblk)
+            CU(cudaMemcpy2DAsync(static_cast<uint32_t*>(sblk->p) + at_row, cap * 4, b->out_stats.as<uint32_t>() + row_lo, sk * 4, n_rows * 4, 10,
+                                 cudaMemcpyDeviceToHost, s));
+        return RB_OK;
+    }
+    // the caller's views, once every copy has landed (out / stats: nullable)
+    void finish(rb_lift_out* out, rb_stats_out* stats, uint64_t n_rows, uint64_t n_bytes, uint64_t n_pairs) const {
+        const uint64_t c = cap;
+        if (out) {
+            memset(out, 0, sizeof *out);
+            out->n_out = n_rows; out->paf_nbytes = n_bytes; out->n_pairs = n_pairs; out->_owner = blk;
+            uint8_t* base = static_cast<uint8_t*>(blk->p);
+            if (text) {
+                out->paf_text = base + 64;
+                out->line_off = reinterpret_cast<uint64_t*>(base + o_loff);
+                out->line_off[n_rows] = n_bytes;
+                out->paf_text[n_bytes] = 0;
+            }
+            if (num) {
+                uint64_t* p = reinterpret_cast<uint64_t*>(base + o_num);
+                out->q_st = p; out->q_en = p + c; out->t_st = p + 2 * c; out->t_en = p + 3 * c; out->nmatch = p + 4 * c; out->aln_len = p + 5 * c;
+                out->rec_idx = reinterpret_cast<uint32_t*>(p + 6 * c);
+                out->win_idx = out->rec_idx + c;
+            }
+        }
+        if (stats) {
+            uint32_t* p = static_cast<uint32_t*>(sblk->p);
+            memset(stats, 0, sizeof *stats);
+            stats->n = n_rows;
+            stats->equal = p; stats->diff = p + c; stats->ins = p + 2 * c; stats->del = p + 3 * c; stats->ins_events = p + 4 * c;
+            stats->del_events = p + 5 * c; stats->matches = p + 6 * c;
+            stats->id_by_matches = reinterpret_cast<float*>(p + 7 * c); stats->id_by_events = reinterpret_cast<float*>(p + 8 * c);
+            stats->id_by_all = reinterpret_cast<float*>(p + 9 * c);
+            stats->_owner = sblk;
+        }
+    }
+    void release() {
+        if (blk) blk->in_use = false;
+        if (sblk) sblk->in_use = false;
+        blk = sblk = nullptr;
+    }
+};
+
 // RB_TOKSCAN=1 in the environment: tokeniser and sample scan as ONE kernel (k_tok_scan) instead of k_tokenise + k_samples.
 // Parity-clean but opt-in: measured at C4 it takes 0.83 ms against 0.22 + 0.32 ms — a tile is 4 KB of text (~1 500 ops), so
 // 32 700 tiles queue behind one another in the 64-byte-payload look-back, whose frontier moves 32 tiles per ~0.8 us round.
@@ -1478,29 +1571,27 @@ static int batch_invert(rb_ctx* ctx, rb_batch* b, uint32_t want, rb_summary* sum
     return lift_tail(ctx, b, win, RB_POLICY_RIGHTMOST, TAIL_WHOLE, want, 0, P, n_ops, summary);
 }
 
-static int download_stats(rb_ctx* ctx, rb_batch* b, uint64_t n, uint64_t stride, rb_stats_out* st) {  // columns are `stride` rows apart on the device
-    memset(st, 0, sizeof *st);
-    PinnedBlock* blk = pinned_get(ctx, (size_t)n * 40 + 64);
-    if (!blk) return fail(ctx, RB_ERR_OOM, "pinned allocation of %llu bytes failed", (unsigned long long)(n * 40));
-    if (n) CU(cudaMemcpy2DAsync(blk->p, (size_t)n * 4, b->out_stats.p, (size_t)stride * 4, (size_t)n * 4, 10, cudaMemcpyDeviceToHost, ctx->stream));
-    uint32_t* p = reinterpret_cast<uint32_t*>(blk->p);
-    st->n = n;
-    st->equal = p; st->diff = p + n; st->ins = p + 2 * n; st->del = p + 3 * n; st->ins_events = p + 4 * n;
-    st->del_events = p + 5 * n; st->matches = p + 6 * n;
-    st->id_by_matches = reinterpret_cast<float*>(p + 7 * n); st->id_by_events = reinterpret_cast<float*>(p + 8 * n);
-    st->id_by_all = reinterpret_cast<float*>(p + 9 * n);
-    st->_owner = blk;
-    return RB_OK;
+// the copies of a download have been enqueued on the context's stream (rc: unless that failed): wait for them
+static int download_wait(rb_ctx* ctx, RowsOut& rows, int rc) {
+    if (rc == RB_OK && cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+        (void)cudaGetLastError();
+        rc = fail(ctx, RB_ERR_CUDA, "cudaStreamSynchronize(ctx->stream) after the device -> host copies failed");
+    }
+    if (rc != RB_OK) rows.release();
+    return rc;
 }
 
 int rb_batch_download_stats(rb_ctx* ctx, rb_batch* b, rb_stats_out* st) {
     if (!ctx || !b || !st) return RB_ERR_BAD_ARG;
     if (!b->have_stats) return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_stats has not run on this batch");
     cudaSetDevice(ctx->device);
-    const int rc = download_stats(ctx, b, b->n_rec, b->n_rec, st);
-    if (rc != RB_OK) return rc;
-    CU(cudaStreamSynchronize(ctx->stream));
-    return RB_OK;
+    memset(st, 0, sizeof *st);
+    RowsOut rows;
+    int rc = rows.reserve_stats(ctx, b->n_rec);
+    if (rc == RB_OK) rc = rows.copy_rows(ctx, b, 0, b->n_rec, 0, 0, 0, 0, ctx->stream);
+    rc = download_wait(ctx, rows, rc);
+    if (rc == RB_OK) rows.finish(nullptr, st, b->n_rec, 0, 0);
+    return rc;
 }
 
 int rb_batch_download_lift(rb_ctx* ctx, rb_batch* b, uint32_t want, rb_lift_out* out, rb_stats_out* st) {
@@ -1513,42 +1604,14 @@ int rb_batch_download_lift(rb_ctx* ctx, rb_batch* b, uint32_t want, rb_lift_out*
     }
     if (want & ~b->want) return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_liftover did not materialise the requested outputs");
     cudaSetDevice(ctx->device);
-    cudaStream_t s = ctx->stream;
     memset(out, 0, sizeof *out);
     const uint64_t n = b->sum.n_out, nb = b->sum.out_bytes;
-    size_t need = 64;
-    const size_t o_text = need; if (want & RB_WANT_TEXT) need += align_up(nb + 1, 64);
-    const size_t o_loff = need; if (want & RB_WANT_TEXT) need += align_up((n + 1) * 8, 64);
-    const size_t o_num = need; if (want & RB_WANT_NUMERIC) need += align_up(n * 56, 64);
-    PinnedBlock* blk = pinned_get(ctx, need);
-    if (!blk) return fail(ctx, RB_ERR_OOM, "pinned allocation of %zu bytes failed", need);
-    uint8_t* base = reinterpret_cast<uint8_t*>(blk->p);
-    out->n_out = n; out->paf_nbytes = nb; out->n_pairs = b->sum.n_pairs; out->_owner = blk;
-    if (want & RB_WANT_TEXT) {
-        out->paf_text = base + o_text;
-        out->line_off = reinterpret_cast<uint64_t*>(base + o_loff);
-        if (nb) CU(cudaMemcpyAsync(out->paf_text, b->out_text.p, nb, cudaMemcpyDeviceToHost, s));
-        CU(cudaMemcpyAsync(out->line_off, b->out_line_off.p, (n + 1) * 8, cudaMemcpyDeviceToHost, s));
-    }
-    if (want & RB_WANT_NUMERIC) {
-        uint64_t* p = reinterpret_cast<uint64_t*>(base + o_num);
-        if (n) {
-            const uint64_t stride = b->row_stride ? b->row_stride : n;
-            CU(cudaMemcpy2DAsync(p, n * 8, b->out_num.p, stride * 8, n * 8, 6, cudaMemcpyDeviceToHost, s));
-            CU(cudaMemcpy2DAsync(p + 6 * n, n * 4, b->out_num.as<uint64_t>() + 6 * stride, stride * 4, n * 4, 2, cudaMemcpyDeviceToHost, s));
-        }
-        out->q_st = p; out->q_en = p + n; out->t_st = p + 2 * n; out->t_en = p + 3 * n; out->nmatch = p + 4 * n;
-        out->aln_len = p + 5 * n;
-        out->rec_idx = reinterpret_cast<uint32_t*>(p + 6 * n);
-        out->win_idx = out->rec_idx + n;
-    }
-    if (st) {
-        const int rc = download_stats(ctx, b, n, b->row_stride ? b->row_stride : n, st);
-        if (rc != RB_OK) return rc;
-    }
-    CU(cudaStreamSynchronize(s));
-    if (out->paf_text) out->paf_text[nb] = 0;
-    return RB_OK;
+    RowsOut rows;
+    int rc = rows.reserve(ctx, n, nb, want, st != nullptr);
+    if (rc == RB_OK) rc = rows.copy_rows(ctx, b, 0, n, 0, nb, 0, 0, ctx->stream);
+    rc = download_wait(ctx, rows, rc);
+    if (rc == RB_OK) rows.finish(out, st, n, nb, b->sum.n_pairs);
+    return rc;
 }
 
 void rb_free_lift_out(rb_ctx*, rb_lift_out* out) {
@@ -2294,40 +2357,20 @@ int rb_batch_records(rb_ctx* ctx, rb_batch* b, int with_cigar, rb_records* out) 
 // Returns false for name ids out of range (reported properly by the unsliced path); `identity` = file order already.
 static bool emission_order(const rb_records* R, std::vector<uint32_t>& ord, bool& identity) {
     const uint32_t n = R->n_rec;
-    std::vector<int64_t> first(R->n_names, -1);
-    std::vector<uint32_t> cnt, grp(n);
-    for (uint32_t i = 0; i < n; i++) {
-        const uint32_t t = R->t_id[i];
-        if (t >= R->n_names) return false;
-        int64_t& f = first[t];
-        if (f < 0) { f = (int64_t)cnt.size(); cnt.push_back(0); }
-        grp[i] = (uint32_t)f;
-        cnt[grp[i]]++;
-    }
-    std::vector<uint32_t> start(cnt.size() + 1, 0);
-    for (size_t g = 0; g < cnt.size(); g++) start[g + 1] = start[g] + cnt[g];
+    for (uint32_t i = 0; i < n; i++)
+        if (R->t_id[i] >= R->n_names) return false;
+    std::vector<uint32_t> rank(n);
     ord.resize(n);
+    emission_ranks(R->t_id, n, R->n_names, false, nullptr, ord.data(), rank.data());
     identity = true;
-    for (uint32_t i = 0; i < n; i++) {
-        const uint32_t k = start[grp[i]]++;
-        ord[k] = i;
-        identity = identity && (k == i);
-    }
+    for (uint32_t i = 0; i < n && identity; i++) identity = ord[i] == i;
     return true;
 }
 
 static int liftover_unsliced(rb_ctx* ctx, const rb_records* recs, const rb_windows* wins, int policy, uint32_t want, rb_lift_out* out,
-                             rb_stats_out* stats, bool windows_uploaded) {
+                             rb_stats_out* stats) {
     rb_batch* b = ctx->scratch;
-    int rc;
-    if (windows_uploaded) {
-        const RecSel all{nullptr, 0, recs->n_rec};
-        rc = upload_cigar(ctx, b, recs, all);
-        if (rc == RB_OK) rc = upload_columns(ctx, b, recs, all);
-        if (rc != RB_OK && b->busy) { cudaStreamSynchronize(ctx->stream); b->busy = false; }
-    } else {
-        rc = upload_into(ctx, b, recs, wins);
-    }
+    int rc = upload_into(ctx, b, recs, wins);
     if (rc != RB_OK) return rc;
     rc = rb_batch_liftover(ctx, b, policy, want, stats != nullptr, nullptr);
     if (rc != RB_OK) return rc;
@@ -2385,181 +2428,178 @@ bool partition_by_bytes(const rb_records* R, const std::vector<uint32_t>& ord, i
     cut.push_back(n);
     return true;
 }
+
+// The devices of a context (device 0: the context itself, then its peers) and the status of each in the call in progress.
+struct Devices {
+    rb_ctx* ctx;
+    int n;
+    std::vector<int> rc;
+    explicit Devices(rb_ctx* c) : ctx(c), n(1 + (int)c->peers.size()), rc((size_t)n, RB_OK) {}
+    rb_ctx* at(int d) const { return d ? ctx->peers[(size_t)d - 1] : ctx; }
+
+    // fn(d, c) on every device, devices 1 .. n-1 on threads of their own and device 0 on the caller's.  Before it, each device
+    // clears its error, gets its scratch batch and waits for a batch of an earlier call still in flight; rc[d] says whether that
+    // worked (fn runs either way, so that it reaches every rendezvous of the call).
+    template <class F> void run(F&& fn) {
+        auto one = [&](int d) {
+            rb_ctx* c = at(d);
+            cudaSetDevice(c->device);
+            c->err.clear(); c->err_rec = UINT64_MAX;
+            if (!c->scratch) c->scratch = new rb_batch();
+            rc[(size_t)d] = [c] {
+                rb_ctx* ctx = c;  // (CU reports into this device's context)
+                if (c->scratch->busy) { CU(cudaStreamSynchronize(c->stream)); c->scratch->busy = false; }
+                return (int)RB_OK;
+            }();
+            fn(d, c);
+        };
+        std::vector<std::thread> pool;
+        for (int d = 1; d < n; d++) pool.emplace_back(one, d);
+        one(0);
+        for (auto& th : pool) th.join();
+        cudaSetDevice(ctx->device);
+    }
+
+    // the status that fails the call: the first failing device in device order, or (by_record: errors of the lift) the one that
+    // reports the smallest record index.  ctx->err takes that device's message.
+    int error(bool by_record) const {
+        int k = -1;
+        for (int d = 0; d < n; d++)
+            if (rc[(size_t)d] != RB_OK && (k < 0 || (by_record && at(d)->err_rec < at(k)->err_rec))) k = d;
+        if (k < 0) return RB_OK;
+        if (k) ctx->err = at(k)->err;
+        return rc[(size_t)k];
+    }
+};
+
+// The window rows one device of a split rb_liftover uploads: those of the contigs of its records, which travel in front of their
+// CIGAR text; on the first device also the rest of the table, for the check kernel looks at all of it.
+struct WindowRows {
+    std::vector<uint8_t> seen;                        // contigs whose rows are on their way
+    std::vector<std::pair<uint32_t, uint32_t>> done;  // row ranges on their way
+
+    // the rows of the contigs of records ord[lo .. hi)
+    int contigs(rb_ctx* c, rb_batch* b, const rb_records* R, const rb_windows* W, const uint32_t* ord, uint32_t lo, uint32_t hi,
+                cudaStream_t s) {
+        seen.resize(R->n_names, 0);
+        for (uint32_t i = lo; i < hi; i++) {
+            const uint32_t t = R->t_id[ord[i]];
+            if (seen[t]) continue;
+            seen[t] = 1;
+            const uint32_t r0 = b->h_clo[t], r1 = b->h_chi[t];
+            if (r1 <= r0) continue;
+            const int rc = windows_upload_rows(c, b, W, r0, r1, s);
+            if (rc != RB_OK) return rc;
+            done.emplace_back(r0, r1);
+        }
+        return RB_OK;
+    }
+    // every row not uploaded yet, then the table check (after `after`, if given) and its verdict
+    int rest(rb_ctx* c, rb_batch* b, const rb_records* R, const rb_windows* W, cudaStream_t s, cudaEvent_t after = nullptr) {
+        std::sort(done.begin(), done.end());
+        uint32_t at = 0;
+        int rc = RB_OK;
+        for (auto& iv : done) {
+            if (rc == RB_OK && iv.first > at) rc = windows_upload_rows(c, b, W, at, iv.first, s);
+            at = std::max(at, iv.second);
+        }
+        if (rc == RB_OK && at < b->n_win) rc = windows_upload_rows(c, b, W, at, b->n_win, s);
+        if (rc == RB_OK && after && cudaStreamWaitEvent(s, after, 0) != cudaSuccess) rc = fail(c, RB_ERR_CUDA, "cudaStreamWaitEvent");
+        if (rc == RB_OK) rc = windows_check(c, b, R, s);
+        if (rc == RB_OK) rc = upload_windows_end(c, b, R, W);  // waits for the verdict
+        return rc;
+    }
+};
+
+// for the length of a call: --qbed (the columns are swapped) and RB_WANT_STATS_TEXT, on the context and all its peers
+struct CallFlags {
+    rb_ctx* ctx;
+    CallFlags(rb_ctx* c, bool invert, bool stats_text) : ctx(c) { set(invert, stats_text); }
+    ~CallFlags() { set(false, false); }
+    void set(bool invert, bool stats_text) {
+        ctx->invert = invert; ctx->stats_text = stats_text;
+        for (rb_ctx* p : ctx->peers) { p->invert = invert; p->stats_text = stats_text; }
+    }
+};
 }  // namespace
 }  // extern "C++"
 
 // returns 1 when the call was not spread (the caller runs it on the first device), else an rb_status
 static int liftover_multi(rb_ctx* ctx, const rb_records* recs, const rb_windows* wins, int policy, uint32_t want, rb_lift_out* out,
                           rb_stats_out* stats) {
-    const int D = 1 + (int)ctx->peers.size();
+    Devices dev(ctx);
+    const int D = dev.n;
     if (!recs || !wins || !wins->n_win || recs->n_rec < 2u * (uint32_t)D || !recs->cigar_off || !recs->t_id ||
         recs->cigar_nbytes < ctx->multi_min_bytes || recs->cigar_off[recs->n_rec] != recs->cigar_nbytes || ctx->profiling)
         return 1;
     std::vector<uint32_t> ord, cut;
     bool identity = true;
     if (!emission_order(recs, ord, identity) || !partition_by_bytes(recs, ord, D, cut)) return 1;
-    std::vector<rb_ctx*> cs(1, ctx);
-    cs.insert(cs.end(), ctx->peers.begin(), ctx->peers.end());
 
-    struct Dev { int rc = RB_OK; rb_summary sum{}; uint64_t row_base = 0, byte_base = 0; bool general = false; };
+    struct Dev { rb_summary sum{}; uint64_t row_base = 0, byte_base = 0; bool general = false; };
     std::vector<Dev> dv((size_t)D);
     Rendezvous rv(D);
-    PinnedBlock *blk = nullptr, *sblk = nullptr;
-    uint8_t* base = nullptr;
-    size_t o_text = 64, o_loff = 0, o_num = 0;
+    RowsOut rows;
     uint64_t tot_rows = 0, tot_bytes = 0, tot_pairs = 0;
     int call_rc = RB_OK;
     bool fall_back = false;
 
-    auto work = [&](int d) {
-        rb_ctx* c = cs[(size_t)d];
+    dev.run([&](int d, rb_ctx* c) {
         Dev& me = dv[(size_t)d];
-        cudaSetDevice(c->device);
-        c->invert = ctx->invert;
-        c->err.clear(); c->err_rec = UINT64_MAX;
-        if (!c->scratch) c->scratch = new rb_batch();
         rb_batch* b = c->scratch;
         cudaStream_t s = c->stream;
-        auto run = [&]() -> int {
-            if (b->busy) { if (cudaStreamSynchronize(s) != cudaSuccess) return fail(c, RB_ERR_CUDA, "cudaStreamSynchronize"); b->busy = false; }
+        int& status = dev.rc[(size_t)d];
+        if (status == RB_OK) status = [&]() -> int {
             b->n_rec = 0; b->have_lift = b->have_stats = false;
             int rc = windows_prepare(c, b, recs, wins);
-            if (rc != RB_OK) return rc;
-            // the window rows of this device's contigs travel in front of its CIGAR text
-            std::vector<uint8_t> up(recs->n_names, 0);
-            std::vector<std::pair<uint32_t, uint32_t>> rows_up;
-            for (uint32_t i = cut[(size_t)d]; i < cut[(size_t)d + 1]; i++) {
-                const uint32_t t = recs->t_id[ord[i]];
-                if (up[t]) continue;
-                up[t] = 1;
-                const uint32_t lo = b->h_clo[t], hi = b->h_chi[t];
-                if (hi <= lo) continue;
-                rc = windows_upload_rows(c, b, wins, lo, hi, s);
-                if (rc != RB_OK) return rc;
-                rows_up.emplace_back(lo, hi);
-            }
-            rc = windows_upload_aux(c, b, recs, wins, s);
+            WindowRows wr;
+            if (rc == RB_OK) rc = wr.contigs(c, b, recs, wins, ord.data(), cut[(size_t)d], cut[(size_t)d + 1], s);
+            if (rc == RB_OK) rc = windows_upload_aux(c, b, recs, wins, s);
             if (rc != RB_OK) return rc;
             const RecSel sel{identity ? nullptr : ord.data() + cut[(size_t)d], cut[(size_t)d], cut[(size_t)d + 1] - cut[(size_t)d]};
             rc = upload_cigar(c, b, recs, sel);
             if (rc == RB_OK) rc = upload_columns(c, b, recs, sel);
-            if (rc != RB_OK) return rc;
-            rc = rb_batch_liftover(c, b, policy, want, stats != nullptr, &me.sum);
-            if (rc != RB_OK) return rc;
-            if (d == 0) {  // the first device also sees the rest of the table: the check kernel looks at all of it
-                std::sort(rows_up.begin(), rows_up.end());
-                uint32_t at = 0;
-                for (auto& iv : rows_up) {
-                    if (rc == RB_OK && iv.first > at) rc = windows_upload_rows(c, b, wins, at, iv.first, s);
-                    at = std::max(at, iv.second);
-                }
-                if (rc == RB_OK && at < b->n_win) rc = windows_upload_rows(c, b, wins, at, b->n_win, s);
-                if (rc == RB_OK) rc = windows_check(c, b, recs, s);
-                if (rc == RB_OK) rc = upload_windows_end(c, b, recs, wins);  // waits for the verdict
+            if (rc == RB_OK) rc = rb_batch_liftover(c, b, policy, want, stats != nullptr, &me.sum);
+            if (rc == RB_OK && d == 0) {
+                rc = wr.rest(c, b, recs, wins, s);
                 me.general = b->general;
             }
             return rc;
-        };
-        me.rc = run();
-        if (me.rc != RB_OK && b->busy) { cudaStreamSynchronize(s); b->busy = false; }
+        }();
+        if (status != RB_OK && b->busy) { cudaStreamSynchronize(s); b->busy = false; }
         rv.meet([&] {  // everybody's sizes are known: lay out the one output block
-            uint64_t best_err = UINT64_MAX;
-            for (int k = 0; k < D; k++) {
-                if (dv[(size_t)k].rc != RB_OK && (call_rc == RB_OK || cs[(size_t)k]->err_rec < best_err)) {
-                    call_rc = dv[(size_t)k].rc;
-                    best_err = cs[(size_t)k]->err_rec;
-                    if (k) ctx->err = cs[(size_t)k]->err;
-                }
-                if (dv[(size_t)k].general) fall_back = true;  // nested rows / file order != sorted order: single-batch path
-            }
+            call_rc = dev.error(true);
+            for (const Dev& o : dv) fall_back |= o.general;  // nested rows / file order != sorted order: single-batch path
             if (call_rc != RB_OK || fall_back) return;
-            for (int k = 0; k < D; k++) {
-                dv[(size_t)k].row_base = tot_rows; dv[(size_t)k].byte_base = tot_bytes;
-                tot_rows += dv[(size_t)k].sum.n_out; tot_bytes += dv[(size_t)k].sum.out_bytes; tot_pairs += dv[(size_t)k].sum.n_pairs;
+            for (Dev& o : dv) {
+                o.row_base = tot_rows; o.byte_base = tot_bytes;
+                tot_rows += o.sum.n_out; tot_bytes += o.sum.out_bytes; tot_pairs += o.sum.n_pairs;
             }
             cudaSetDevice(ctx->device);
-            const size_t text_room = (want & RB_WANT_TEXT) ? align_up(tot_bytes + 1, 64) : 0;
-            const size_t loff_bytes = (want & RB_WANT_TEXT) ? align_up((tot_rows + 1) * 8, 64) : 0;
-            const size_t num_bytes = (want & RB_WANT_NUMERIC) ? align_up(tot_rows * 56, 64) : 0;
-            blk = pinned_get(ctx, 64 + text_room + loff_bytes + num_bytes);
-            if (stats) sblk = pinned_get(ctx, (size_t)tot_rows * 40 + 64);
-            if (!blk || (stats && !sblk)) { call_rc = fail(ctx, RB_ERR_OOM, "pinned allocation of the merged output failed"); return; }
-            base = reinterpret_cast<uint8_t*>(blk->p);
-            o_loff = 64 + text_room;
-            o_num = o_loff + loff_bytes;
+            call_rc = rows.reserve(ctx, tot_rows, tot_bytes, want, stats != nullptr);
             cudaSetDevice(c->device);
         });
         if (call_rc != RB_OK || fall_back) return;
         // ---- this device's rows -> their place in the merged output ----
-        auto copy = [&]() -> int {
+        status = [&]() -> int {
             rb_ctx* ctx = c;  // (CU reports into this device's context)
-            const uint64_t nk = me.sum.n_out, sk = b->row_stride ? b->row_stride : nk, cap = tot_rows;
-            if (want & RB_WANT_TEXT) {
-                launch_add_u64(b->out_line_off.as<uint64_t>(), nk, me.byte_base, s);
-                if (me.sum.out_bytes) CU(cudaMemcpyAsync(base + o_text + me.byte_base, b->out_text.p, me.sum.out_bytes, cudaMemcpyDeviceToHost, s));
-                if (nk) CU(cudaMemcpyAsync(reinterpret_cast<uint64_t*>(base + o_loff) + me.row_base, b->out_line_off.p, nk * 8, cudaMemcpyDeviceToHost, s));
-            }
-            if ((want & RB_WANT_NUMERIC) && nk) {
-                uint64_t* dn = reinterpret_cast<uint64_t*>(base + o_num);
-                const uint64_t* sp = b->out_num.as<uint64_t>();
-                CU(cudaMemcpy2DAsync(dn + me.row_base, cap * 8, sp, sk * 8, nk * 8, 6, cudaMemcpyDeviceToHost, s));
-                uint32_t* d32 = reinterpret_cast<uint32_t*>(dn + 6 * cap);
-                const uint32_t* s32 = reinterpret_cast<const uint32_t*>(sp + 6 * sk);
-                CU(cudaMemcpy2DAsync(d32 + me.row_base, cap * 4, s32, sk * 4, nk * 4, 2, cudaMemcpyDeviceToHost, s));
-            }
-            if (stats && nk) {
-                uint32_t* ds = reinterpret_cast<uint32_t*>(sblk->p);
-                CU(cudaMemcpy2DAsync(ds + me.row_base, cap * 4, b->out_stats.as<uint32_t>(), sk * 4, nk * 4, 10, cudaMemcpyDeviceToHost, s));
-            }
+            if (want & RB_WANT_TEXT) launch_add_u64(b->out_line_off.as<uint64_t>(), me.sum.n_out, me.byte_base, s);
+            const int rc = rows.copy_rows(c, b, 0, me.sum.n_out, 0, me.sum.out_bytes, me.row_base, me.byte_base, s);
+            if (rc != RB_OK) return rc;
             CU(cudaStreamSynchronize(s));
             return RB_OK;
-        };
-        me.rc = copy();
-    };
-    std::vector<std::thread> pool;
-    for (int d = 1; d < D; d++) pool.emplace_back(work, d);
-    work(0);
-    for (auto& th : pool) th.join();
-    cudaSetDevice(ctx->device);
-    for (rb_ctx* p : ctx->peers) p->invert = false;
-    auto release = [&] { if (blk) blk->in_use = false; if (sblk) sblk->in_use = false; };
-    if (fall_back && call_rc == RB_OK) { release(); return 1; }
-    if (call_rc != RB_OK) { release(); return call_rc; }
-    for (int d = 0; d < D; d++)
-        if (dv[(size_t)d].rc != RB_OK) { if (d) ctx->err = cs[(size_t)d]->err; release(); return dv[(size_t)d].rc; }
-    memset(out, 0, sizeof *out);
-    if (stats) memset(stats, 0, sizeof *stats);
-    out->n_out = tot_rows; out->paf_nbytes = tot_bytes; out->n_pairs = tot_pairs; out->_owner = blk;
-    if (want & RB_WANT_TEXT) {
-        out->paf_text = base + o_text;
-        out->line_off = reinterpret_cast<uint64_t*>(base + o_loff);
-        out->line_off[tot_rows] = tot_bytes;
-        if (tot_rows == 0) out->line_off[0] = 0;
-        out->paf_text[tot_bytes] = 0;
-    }
-    if (want & RB_WANT_NUMERIC) {
-        uint64_t* p = reinterpret_cast<uint64_t*>(base + o_num);
-        const uint64_t c = tot_rows;
-        out->q_st = p; out->q_en = p + c; out->t_st = p + 2 * c; out->t_en = p + 3 * c; out->nmatch = p + 4 * c; out->aln_len = p + 5 * c;
-        out->rec_idx = reinterpret_cast<uint32_t*>(p + 6 * c);
-        out->win_idx = out->rec_idx + c;
-    }
-    if (stats) {
-        uint32_t* p = reinterpret_cast<uint32_t*>(sblk->p);
-        const uint64_t c = tot_rows;
-        stats->n = tot_rows;
-        stats->equal = p; stats->diff = p + c; stats->ins = p + 2 * c; stats->del = p + 3 * c; stats->ins_events = p + 4 * c;
-        stats->del_events = p + 5 * c; stats->matches = p + 6 * c;
-        stats->id_by_matches = reinterpret_cast<float*>(p + 7 * c); stats->id_by_events = reinterpret_cast<float*>(p + 8 * c);
-        stats->id_by_all = reinterpret_cast<float*>(p + 9 * c);
-        stats->_owner = sblk;
-    }
+        }();
+    });
+    if (call_rc == RB_OK) call_rc = dev.error(false);
+    if (call_rc != RB_OK || fall_back) { rows.release(); return call_rc != RB_OK ? call_rc : 1; }
+    rows.finish(out, stats, tot_rows, tot_bytes, tot_pairs);
     return RB_OK;
 }
 
 // rb_stats on a multi-device context: runs of records in FILE order, balanced on CIGAR bytes; rows land at their record index
 static int stats_multi(rb_ctx* ctx, const rb_records* recs, rb_stats_out* stats) {
-    const int D = 1 + (int)ctx->peers.size();
+    Devices dev(ctx);
+    const int D = dev.n;
     if (!recs || recs->n_rec < 2u * (uint32_t)D || !recs->cigar_off || recs->cigar_nbytes < ctx->multi_min_bytes ||
         recs->cigar_off[recs->n_rec] != recs->cigar_nbytes || ctx->profiling)
         return 1;
@@ -2572,51 +2612,29 @@ static int stats_multi(rb_ctx* ctx, const rb_records* recs, rb_stats_out* stats)
         cut.push_back(i);
     }
     cut.push_back(n);
-    std::vector<rb_ctx*> cs(1, ctx);
-    cs.insert(cs.end(), ctx->peers.begin(), ctx->peers.end());
-    PinnedBlock* sblk = pinned_get(ctx, (size_t)n * 40 + 64);
-    if (!sblk) return fail(ctx, RB_ERR_OOM, "pinned allocation of %llu bytes failed", (unsigned long long)n * 40);
-    std::vector<int> rcs((size_t)D, RB_OK);
-    auto work = [&](int d) {
-        rb_ctx* c = cs[(size_t)d];
-        rb_ctx* ctx = c;  // (CU reports into this device's context)
-        cudaSetDevice(c->device);
-        c->invert = false;
-        c->err.clear(); c->err_rec = UINT64_MAX;
-        if (!c->scratch) c->scratch = new rb_batch();
+    RowsOut rows;
+    int rc = rows.reserve_stats(ctx, n);
+    if (rc != RB_OK) return rc;
+    dev.run([&](int d, rb_ctx* c) {
         rb_batch* b = c->scratch;
-        auto run = [&]() -> int {
-            if (b->busy) { CU(cudaStreamSynchronize(c->stream)); b->busy = false; }
+        int& status = dev.rc[(size_t)d];
+        if (status == RB_OK) status = [&]() -> int {
+            rb_ctx* ctx = c;  // (CU reports into this device's context)
             const RecSel sel{nullptr, cut[(size_t)d], cut[(size_t)d + 1] - cut[(size_t)d]};
             int rc = upload_cigar(c, b, recs, sel);
             if (rc == RB_OK) rc = windows_prepare(c, b, recs, nullptr);
             if (rc == RB_OK) rc = upload_columns(c, b, recs, sel);
             if (rc == RB_OK) rc = rb_batch_stats(c, b, nullptr);
+            if (rc == RB_OK) rc = rows.copy_rows(c, b, 0, sel.n, 0, 0, sel.r0, 0, c->stream);
             if (rc != RB_OK) return rc;
-            const uint64_t nk = sel.n;
-            if (nk) CU(cudaMemcpy2DAsync(reinterpret_cast<uint32_t*>(sblk->p) + sel.r0, (size_t)n * 4, b->out_stats.p, nk * 4, nk * 4, 10,
-                                         cudaMemcpyDeviceToHost, c->stream));
             CU(cudaStreamSynchronize(c->stream));
             return RB_OK;
-        };
-        rcs[(size_t)d] = run();
-        if (rcs[(size_t)d] != RB_OK && b->busy) { cudaStreamSynchronize(c->stream); b->busy = false; }
-    };
-    std::vector<std::thread> pool;
-    for (int d = 1; d < D; d++) pool.emplace_back(work, d);
-    work(0);
-    for (auto& th : pool) th.join();
-    cudaSetDevice(ctx->device);
-    for (int d = 0; d < D; d++)  // devices hold runs of the file order: the first failing device holds the first failing record
-        if (rcs[(size_t)d] != RB_OK) { if (d) ctx->err = cs[(size_t)d]->err; sblk->in_use = false; return rcs[(size_t)d]; }
-    memset(stats, 0, sizeof *stats);
-    uint32_t* p = reinterpret_cast<uint32_t*>(sblk->p);
-    stats->n = n;
-    stats->equal = p; stats->diff = p + n; stats->ins = p + 2 * (size_t)n; stats->del = p + 3 * (size_t)n; stats->ins_events = p + 4 * (size_t)n;
-    stats->del_events = p + 5 * (size_t)n; stats->matches = p + 6 * (size_t)n;
-    stats->id_by_matches = reinterpret_cast<float*>(p + 7 * (size_t)n); stats->id_by_events = reinterpret_cast<float*>(p + 8 * (size_t)n);
-    stats->id_by_all = reinterpret_cast<float*>(p + 9 * (size_t)n);
-    stats->_owner = sblk;
+        }();
+        if (status != RB_OK && b->busy) { cudaStreamSynchronize(c->stream); b->busy = false; }
+    });
+    rc = dev.error(false);  // devices hold runs of the file order: the first failing device holds the first failing record
+    if (rc != RB_OK) { rows.release(); return rc; }
+    rows.finish(nullptr, stats, n, 0, 0);
     return RB_OK;
 }
 
@@ -2659,9 +2677,8 @@ static int liftover_text_one(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbyte
 
 static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, const uint8_t* bed, uint64_t bed_nbytes, int policy,
                                uint32_t want, rb_lift_out* out, rb_stats_out* stats, rb_paf_info* paf_info, rb_bed_info* bed_info) {
-    const int D = 1 + (int)ctx->peers.size();
-    std::vector<rb_ctx*> cs(1, ctx);
-    cs.insert(cs.end(), ctx->peers.begin(), ctx->peers.end());
+    Devices dev(ctx);
+    const int D = dev.n;
     // 1. the input's byte ranges
     const bool bgzf = rb_is_bgzf(paf, paf_nbytes) != 0;
     if (!bgzf && paf_nbytes >= 2 && paf[0] == 0x1f && paf[1] == 0x8b)
@@ -2684,10 +2701,9 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
         for (int d = 1; d < D; d++) src[(size_t)d] = paf_nbytes / (uint64_t)D * (uint64_t)d + paf_nbytes % (uint64_t)D * (uint64_t)d / (uint64_t)D;
     }
     const uint32_t want_lift = want | RB_WANT_NUMERIC;  // (rec_idx places the rows)
-    const bool want_text = (want & (RB_WANT_TEXT | RB_WANT_STATS_TEXT)) != 0, want_num = (want & RB_WANT_NUMERIC) != 0;
+    const bool want_text = (want & (RB_WANT_TEXT | RB_WANT_STATS_TEXT)) != 0;
 
     struct Dev {
-        int rc = RB_OK;
         DevBuf range, own, rank, runs_d, delta;
         uint64_t n = 0, first_nl = rbt::NO_NEWLINE, rec_base = 0;
         uint8_t last = 0;  // the range's last byte
@@ -2703,43 +2719,24 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
     std::vector<uint32_t> rank_of;  // name id -> contig rank (first appearance as t_name in the file)
     uint32_t n_ranks = 0, n_names = 0;
     rb_batch* b0 = ctx->scratch ? ctx->scratch : (ctx->scratch = new rb_batch());
-    PinnedBlock *blk = nullptr, *sblk = nullptr;
-    uint8_t* base = nullptr;
-    size_t o_text = 64, o_loff = 0, o_num = 0;
+    RowsOut rows;
     uint64_t tot_rows = 0, tot_bytes = 0, tot_pairs = 0;
     int call_rc = RB_OK;
-    // the first failing device in device order (lift errors: the smallest global record index) fails the call
-    auto first_error = [&](bool by_record) {
-        uint64_t best = UINT64_MAX;
-        for (int k = 0; k < D; k++) {
-            if (dv[(size_t)k].rc == RB_OK) continue;
-            if (call_rc == RB_OK || (by_record && cs[(size_t)k]->err_rec < best)) {
-                call_rc = dv[(size_t)k].rc;
-                best = cs[(size_t)k]->err_rec;
-                if (k) ctx->err = cs[(size_t)k]->err;
-            }
-            if (!by_record) return;
-        }
-    };
 
-    auto work = [&](int d) {
-        rb_ctx* c = cs[(size_t)d];
+    dev.run([&](int d, rb_ctx* c) {
         Dev& me = dv[(size_t)d];
-        cudaSetDevice(c->device);
-        c->err.clear(); c->err_rec = UINT64_MAX;
-        if (!c->scratch) c->scratch = new rb_batch();
+        int& status = dev.rc[(size_t)d];
         rb_batch* b = c->scratch;
         cudaStream_t s = c->stream;
         uint32_t* sc = c->scalars.as<uint32_t>();
         volatile uint64_t* hs = reinterpret_cast<volatile uint64_t*>(c->h_scalars);
-        auto finish = [&] {
+        auto cleanup = [&] {
             if (b->busy) { cudaStreamSynchronize(s); b->busy = false; }
             me.range.release(); me.own.release(); me.rank.release(); me.runs_d.release(); me.delta.release();
         };
         // 1. this device's range -> HBM, its first '\n'
-        me.rc = [&]() -> int {
+        if (status == RB_OK) status = [&]() -> int {
             rb_ctx* ctx = c;  // (CU reports into this device's context)
-            if (b->busy) { CU(cudaStreamSynchronize(s)); b->busy = false; }
             const uint64_t len = src[(size_t)d + 1] - src[(size_t)d];
             if (bgzf) {
                 const int rc = inflate_to_device(c, paf + src[(size_t)d], len, me.range, me.n, TEXT_PAD, blk_base[(size_t)d]);
@@ -2765,7 +2762,7 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
             return RB_OK;
         }();
         rv.meet([&] {
-            first_error(false);
+            call_rc = dev.error(false);
             if (call_rc != RB_OK) return;
             std::vector<uint64_t> size((size_t)D), nl((size_t)D);
             std::vector<uint8_t> ends_nl((size_t)D);
@@ -2775,9 +2772,9 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
             }
             plan = rbt::plan_line_split(size, nl, ends_nl);
         });
-        if (call_rc != RB_OK) { finish(); return; }
+        if (call_rc != RB_OK) { cleanup(); return; }
         // 2. the lines this device owns -> one fresh buffer
-        me.rc = [&]() -> int {
+        status = [&]() -> int {
             rb_ctx* ctx = c;  // (CU reports into this device's context)
             const rbt::Owned& o = plan[(size_t)d];
             CU(me.own.ensure(o.bytes + TEXT_PAD));
@@ -2785,23 +2782,23 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
             for (const rbt::Piece& pc : o.pieces) {
                 const Dev& from = dv[(size_t)pc.src];
                 if (pc.src == d) CU(cudaMemcpyAsync(me.own.as<uint8_t>() + at, from.range.as<uint8_t>() + pc.off, pc.len, cudaMemcpyDeviceToDevice, s));
-                else CU(cudaMemcpyPeerAsync(me.own.as<uint8_t>() + at, c->device, from.range.as<uint8_t>() + pc.off, cs[(size_t)pc.src]->device, pc.len, s));
+                else CU(cudaMemcpyPeerAsync(me.own.as<uint8_t>() + at, c->device, from.range.as<uint8_t>() + pc.off, dev.at(pc.src)->device, pc.len, s));
                 at += pc.len;
             }
             CU(cudaStreamSynchronize(s));
             return RB_OK;
         }();
-        rv.meet([&] { first_error(false); });  // (every copy out of the ranges has finished)
+        rv.meet([&] { call_rc = dev.error(false); });  // (every copy out of the ranges has finished)
         me.range.release();
-        if (call_rc != RB_OK) { finish(); return; }
+        if (call_rc != RB_OK) { cleanup(); return; }
         // 3. parse
-        me.rc = paf_parse_text(c, b, me.own.as<uint8_t>(), plan[(size_t)d].bytes, me.p);
+        status = paf_parse_text(c, b, me.own.as<uint8_t>(), plan[(size_t)d].bytes, me.p);
         me.own.release();
         rv.meet([&] {
             uint64_t lines = 0, recs = 0, text = 0, cg = 0;
             for (int k = 0; k < D; k++) {  // the first error or panic in file order
                 Dev& o = dv[(size_t)k];
-                if (o.rc != RB_OK) { call_rc = o.rc; if (k) ctx->err = cs[(size_t)k]->err; return; }
+                if (dev.rc[(size_t)k] != RB_OK) { call_rc = dev.error(false); return; }  // (k is the first failing device)
                 if (o.p.panic != ~0ull) { call_rc = paf_panic(ctx, o.p.panic, lines); return; }
                 o.rec_base = recs;
                 lines += o.p.n_lines; recs += o.p.n_rec; text += o.p.text_bytes; cg += o.p.cg_bytes;
@@ -2823,9 +2820,9 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
             for (uint32_t& r : rank_of) if (r == UINT32_MAX) r = 0;  // (query-only names: never looked up)
             paf_fill_info(paf_info, text, lines, recs, b0->h_names, b0->h_names_off, cg);
         });
-        if (call_rc != RB_OK) { finish(); return; }
+        if (call_rc != RB_OK) { cleanup(); return; }
         // 4. names, windows, lift, the contig runs of the rows
-        me.rc = [&]() -> int {
+        status = [&]() -> int {
             rb_ctx* ctx = c;  // (CU reports into this device's context)
             int rc = paf_upload_names(c, b, me.p, b0->h_names.data(), b0->h_names_off.data(), n_names, rank_of.data());
             if (rc != RB_OK) return rc;
@@ -2854,7 +2851,7 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
             return RB_OK;
         }();
         auto layout = [&] {  // everybody's runs are known: lay out the one output block, cells in (contig rank, device) order
-            first_error(true);
+            call_rc = dev.error(true);
             if (call_rc != RB_OK) return;
             for (int k = 0; k < D; k++) {
                 dv[(size_t)k].at_row.assign(n_ranks, 0); dv[(size_t)k].at_byte.assign(n_ranks, 0);
@@ -2868,31 +2865,23 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
                     tot_rows += o.runs[n_ranks + r] - o.runs[r];
                     tot_bytes += o.runs[3 * (size_t)n_ranks + r] - o.runs[2 * (size_t)n_ranks + r];
                 }
-            uint64_t rows = 0;
-            for (int k = 0; k < D; k++) rows += dv[(size_t)k].sum.n_out;
+            uint64_t rows_in = 0;
+            for (int k = 0; k < D; k++) rows_in += dv[(size_t)k].sum.n_out;
             if (!want_text)  // (no line offsets: the byte count is the devices' sum, as out->paf_nbytes of rb_liftover reports it)
                 for (int k = 0; k < D; k++) tot_bytes += dv[(size_t)k].sum.out_bytes;
-            if (rows != tot_rows) { call_rc = fail(ctx, RB_ERR_CUDA, "rb_liftover_text: the rows of a device are not grouped by contig"); return; }
-            const size_t text_room = want_text ? align_up(tot_bytes + 1, 64) : 0;
-            const size_t loff_bytes = want_text ? align_up((tot_rows + 1) * 8, 64) : 0;
-            const size_t num_bytes = want_num ? align_up(tot_rows * 56, 64) : 0;
-            blk = pinned_get(ctx, 64 + text_room + loff_bytes + num_bytes);
-            if (stats) sblk = pinned_get(ctx, (size_t)tot_rows * 40 + 64);
-            if (!blk || (stats && !sblk)) { call_rc = fail(ctx, RB_ERR_OOM, "pinned allocation of the merged output failed"); return; }
-            base = reinterpret_cast<uint8_t*>(blk->p);
-            o_loff = 64 + text_room;
-            o_num = o_loff + loff_bytes;
+            if (rows_in != tot_rows) { call_rc = fail(ctx, RB_ERR_CUDA, "rb_liftover_text: the rows of a device are not grouped by contig"); return; }
+            call_rc = rows.reserve(ctx, tot_rows, tot_bytes, want, stats != nullptr);
         };
         rv.meet([&] {
             cudaSetDevice(ctx->device);  // (the pinned pool belongs to the first device's context)
             layout();
             cudaSetDevice(c->device);
         });
-        if (call_rc != RB_OK) { finish(); return; }
+        if (call_rc != RB_OK) { cleanup(); return; }
         // 5. this device's cells -> their places in the merged output
-        me.rc = [&]() -> int {
+        status = [&]() -> int {
             rb_ctx* ctx = c;  // (CU reports into this device's context)
-            const uint64_t nk = me.sum.n_out, sk = b->row_stride ? b->row_stride : nk, cap = tot_rows;
+            const uint64_t nk = me.sum.n_out, sk = b->row_stride ? b->row_stride : nk;
             if (me.runs.empty() || nk == 0) return RB_OK;
             const uint32_t* rec_idx = reinterpret_cast<const uint32_t*>(b->out_num.as<uint64_t>() + 6 * sk);
             const uint64_t* runs = me.runs.data();
@@ -2908,61 +2897,19 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
             for (uint32_t r = 0; r < n_ranks; r++) {
                 const uint64_t lo = runs[r], hi = runs[n_ranks + r], blo = runs[2 * (size_t)n_ranks + r], bhi = runs[3 * (size_t)n_ranks + r];
                 if (hi <= lo) continue;
-                const uint64_t rows = hi - lo, at = me.at_row[r];
-                if (want_text) {
-                    if (bhi > blo) CU(cudaMemcpyAsync(base + o_text + me.at_byte[r], b->out_text.as<uint8_t>() + blo, bhi - blo, cudaMemcpyDeviceToHost, s));
-                    CU(cudaMemcpyAsync(reinterpret_cast<uint64_t*>(base + o_loff) + at, b->out_line_off.as<uint64_t>() + lo, rows * 8, cudaMemcpyDeviceToHost, s));
-                }
-                if (want_num) {
-                    uint64_t* dn = reinterpret_cast<uint64_t*>(base + o_num);
-                    const uint64_t* sp = b->out_num.as<uint64_t>();
-                    CU(cudaMemcpy2DAsync(dn + at, cap * 8, sp + lo, sk * 8, rows * 8, 6, cudaMemcpyDeviceToHost, s));
-                    CU(cudaMemcpy2DAsync(reinterpret_cast<uint32_t*>(dn + 6 * cap) + at, cap * 4, reinterpret_cast<const uint32_t*>(sp + 6 * sk) + lo,
-                                         sk * 4, rows * 4, 2, cudaMemcpyDeviceToHost, s));
-                }
-                if (stats)
-                    CU(cudaMemcpy2DAsync(reinterpret_cast<uint32_t*>(sblk->p) + at, cap * 4, b->out_stats.as<uint32_t>() + lo, sk * 4, rows * 4, 10,
-                                         cudaMemcpyDeviceToHost, s));
+                const int rc = rows.copy_rows(c, b, lo, hi - lo, blo, bhi - blo, me.at_row[r], me.at_byte[r], s);
+                if (rc != RB_OK) return rc;
             }
             CU(cudaStreamSynchronize(s));
             flush_times(c);
             return RB_OK;
         }();
-        finish();
-    };
-    std::vector<std::thread> pool;
-    for (int d = 1; d < D; d++) pool.emplace_back(work, d);
-    work(0);
-    for (auto& th : pool) th.join();
-    cudaSetDevice(ctx->device);
-    auto release = [&] { if (blk) blk->in_use = false; if (sblk) sblk->in_use = false; };
-    if (call_rc == RB_OK) first_error(false);
-    if (call_rc != RB_OK) { release(); return call_rc; }
+        cleanup();
+    });
+    if (call_rc == RB_OK) call_rc = dev.error(false);
+    if (call_rc != RB_OK) { rows.release(); return call_rc; }
     if (bed_info) *bed_info = dv[0].bi;
-    out->n_out = tot_rows; out->paf_nbytes = tot_bytes; out->n_pairs = tot_pairs; out->_owner = blk;
-    if (want_text) {
-        out->paf_text = base + o_text;
-        out->line_off = reinterpret_cast<uint64_t*>(base + o_loff);
-        out->line_off[tot_rows] = tot_bytes;
-        out->paf_text[tot_bytes] = 0;
-    }
-    if (want_num) {
-        uint64_t* p = reinterpret_cast<uint64_t*>(base + o_num);
-        const uint64_t c = tot_rows;
-        out->q_st = p; out->q_en = p + c; out->t_st = p + 2 * c; out->t_en = p + 3 * c; out->nmatch = p + 4 * c; out->aln_len = p + 5 * c;
-        out->rec_idx = reinterpret_cast<uint32_t*>(p + 6 * c);
-        out->win_idx = out->rec_idx + c;
-    }
-    if (stats) {
-        uint32_t* p = reinterpret_cast<uint32_t*>(sblk->p);
-        const uint64_t c = tot_rows;
-        stats->n = tot_rows;
-        stats->equal = p; stats->diff = p + c; stats->ins = p + 2 * c; stats->del = p + 3 * c; stats->ins_events = p + 4 * c;
-        stats->del_events = p + 5 * c; stats->matches = p + 6 * c;
-        stats->id_by_matches = reinterpret_cast<float*>(p + 7 * c); stats->id_by_events = reinterpret_cast<float*>(p + 8 * c);
-        stats->id_by_all = reinterpret_cast<float*>(p + 9 * c);
-        stats->_owner = sblk;
-    }
+    rows.finish(out, stats, tot_rows, tot_bytes, tot_pairs);
     return RB_OK;
 }
 
@@ -3018,7 +2965,8 @@ static int ensure_slice_streams(rb_ctx* ctx) {
 static int liftover_sliced(rb_ctx* ctx, const rb_records* recs, const rb_windows* wins, int policy, uint32_t want, rb_lift_out* out,
                            rb_stats_out* stats) {
     const uint64_t SLICE_MIN_BYTES = ctx->slice_min_bytes;
-    const int D = 1 + (int)ctx->peers.size();
+    Devices dev(ctx);
+    const int D = dev.n;
     std::vector<uint32_t> ord;  // records in emission order
     bool identity = true;
     const bool try_slices = SLICE_MIN_BYTES && !ctx->profiling && recs && wins && wins->n_win && recs->n_rec >= 2 && recs->cigar_off &&
@@ -3032,8 +2980,6 @@ static int liftover_sliced(rb_ctx* ctx, const rb_records* recs, const rb_windows
         if (trace) fprintf(stderr, "[rb_liftover] %8.3f ms  %s %u\n",
                            std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count(), what, k);
     };
-    std::vector<rb_ctx*> cs(1, ctx);
-    cs.insert(cs.end(), ctx->peers.begin(), ctx->peers.end());
 
     // ---- slice boundaries (record granularity, balanced on CIGAR bytes) and an upper bound on the rows ----
     const uint32_t n = recs->n_rec;
@@ -3061,29 +3007,18 @@ static int liftover_sliced(rb_ctx* ctx, const rb_records* recs, const rb_windows
     cut.push_back(n);
     const uint32_t n_slices = (uint32_t)cut.size() - 1;
     if (n_slices < (uint32_t)D) return 1;  // fewer slices than devices (a few huge records): the exact multi-device path
-    for (rb_ctx* c : cs) {
-        cudaSetDevice(c->device);
-        if (!c->scratch) c->scratch = new rb_batch();
-        rb_ctx* ctx = c;  // (CU reports into this device's context)
-        CU(ensure_slice_streams(c) == RB_OK ? cudaSuccess : cudaErrorUnknown);
-        if (c->scratch->busy) { CU(cudaStreamSynchronize(c->stream)); c->scratch->busy = false; }
+    dev.run([&](int d, rb_ctx* c) {  // streams, work areas, host-side window bookkeeping (contig ranges); the rows travel with the slices
+        int& status = dev.rc[(size_t)d];
+        if (status == RB_OK) status = ensure_slice_streams(c);
+        if (status != RB_OK) return;
         c->scratch->n_rec = 0; c->scratch->have_lift = c->scratch->have_stats = false;
         for (int k = 0; k < 2; k++) {
             if (!c->slice[k]) c->slice[k] = new rb_batch();
             c->slice[k]->wsrc = c->scratch;
         }
-        c->invert = cs[0]->invert; c->stats_text = cs[0]->stats_text;
-        c->err.clear(); c->err_rec = UINT64_MAX;
-    }
-    cudaSetDevice(ctx->device);
-    {   // host-side window bookkeeping (contig ranges) once per device; the rows travel with the slices
-        for (rb_ctx* c : cs) {
-            cudaSetDevice(c->device);
-            const int rc = windows_prepare(c, c->scratch, recs, wins);
-            if (rc != RB_OK) { if (c != ctx) ctx->err = c->err; cudaSetDevice(ctx->device); return rc; }
-        }
-        cudaSetDevice(ctx->device);
-    }
+        status = windows_prepare(c, c->scratch, recs, wins);
+    });
+    if (const int rc = dev.error(false)) return rc;
     rb_batch* wb0 = ctx->scratch;
     uint64_t cap_rows = 0;  // pairs of the unstripped records >= pairs examined >= rows
     for (uint32_t i = 0; i < n; i++) {
@@ -3102,48 +3037,26 @@ static int liftover_sliced(rb_ctx* ctx, const rb_records* recs, const rb_windows
         std::vector<uint8_t> known;
         bool abort = false;                // an error, or the estimates do not hold: everybody stops
         bool fall_back = false;            // ... and the caller takes the exact path
-        int rc = RB_OK;
-        uint64_t err_rec = UINT64_MAX;
-        std::string err;
-        PinnedBlock *blk = nullptr, *sblk = nullptr;
-        uint8_t* base = nullptr;
-        size_t o_text = 64, o_loff = 0, o_num = 0, cap_text = 0;
     } sh;
     sh.sum.assign(n_slices, rb_summary{});
     sh.known.assign(n_slices, 0);
+    RowsOut rows;
     memset(out, 0, sizeof *out);
     if (stats) memset(stats, 0, sizeof *stats);
 
-    auto raise = [&](rb_ctx* c, int code, bool fall_back) {  // first error in record order wins
+    auto stop = [&](bool fall_back) {
         std::lock_guard<std::mutex> lk(sh.m);
-        if (fall_back) sh.fall_back = true;
-        else if (sh.rc == RB_OK || c->err_rec < sh.err_rec) { sh.rc = code; sh.err_rec = c->err_rec; sh.err = c->err; }
+        sh.fall_back = sh.fall_back || fall_back;
         sh.abort = true;
         sh.cv.notify_all();
     };
 
-    auto work = [&](int d) {
-        rb_ctx* c = cs[(size_t)d];
-        cudaSetDevice(c->device);
+    dev.run([&](int d, rb_ctx* c) {
         rb_batch* wb = c->scratch;
         cudaStream_t A = c->stream, B = c->copy_stream, U = c->up_stream;
         std::vector<uint32_t> mine;  // this device's slices
         for (uint32_t k = (uint32_t)d; k < n_slices; k += (uint32_t)D) mine.push_back(k);
-        std::vector<uint8_t> contig_up(recs->n_names, 0);
-        std::vector<std::pair<uint32_t, uint32_t>> rows_up;  // uploaded row ranges
-        auto upload_slice_windows = [&](uint32_t k, cudaStream_t st) {  // a slice only needs the window rows of its own contigs
-            for (uint32_t i = cut[k]; i < cut[k + 1]; i++) {
-                const uint32_t t = recs->t_id[ord[i]];
-                if (contig_up[t]) continue;
-                contig_up[t] = 1;
-                const uint32_t lo = wb->h_clo[t], hi = wb->h_chi[t];
-                if (hi <= lo) continue;
-                const int r2 = windows_upload_rows(c, wb, wins, lo, hi, st);
-                if (r2 != RB_OK) return r2;
-                rows_up.emplace_back(lo, hi);
-            }
-            return (int)RB_OK;
-        };
+        WindowRows wr;  // a slice only needs the window rows of its own contigs
         auto upload_slice = [&](size_t j) {  // j = position in `mine`
             const uint32_t k = mine[j];
             rb_batch* sb = c->slice[j & 1];
@@ -3151,7 +3064,7 @@ static int liftover_sliced(rb_ctx* ctx, const rb_records* recs, const rb_windows
             // on the upload stream, beside the kernels of the slice before; the work area's own previous kernels (two slices
             // back) must have finished reading its inputs
             if (j >= 2 && cudaStreamWaitEvent(U, c->ev_done[j & 1], 0) != cudaSuccess) return fail(c, RB_ERR_CUDA, "cudaStreamWaitEvent");
-            int r2 = j ? upload_slice_windows(k, U) : (int)RB_OK;
+            int r2 = j ? wr.contigs(c, wb, recs, wins, ord.data(), cut[k], cut[k + 1], U) : (int)RB_OK;
             if (r2 != RB_OK) return r2;
             c->upload_on = U;
             r2 = upload_cigar(c, sb, recs, sel);
@@ -3164,7 +3077,7 @@ static int liftover_sliced(rb_ctx* ctx, const rb_records* recs, const rb_windows
         auto run = [&]() -> int {
             rb_ctx* ctx = c;  // (CU reports into this device's context)
             if (mine.empty()) return RB_OK;
-            int rc = upload_slice_windows(mine[0], A);
+            int rc = wr.contigs(c, wb, recs, wins, ord.data(), cut[mine[0]], cut[mine[0] + 1], A);
             if (rc == RB_OK) rc = windows_upload_aux(c, wb, recs, wins, A);
             if (rc != RB_OK) return rc;
             CU(cudaEventRecord(c->ev_wfirst, A));
@@ -3195,98 +3108,51 @@ static int liftover_sliced(rb_ctx* ctx, const rb_records* recs, const rb_windows
                         if (sh.abort) return true;
                         for (uint32_t q = 0; q < k; q++)
                             if (!sh.known[q]) return false;
-                        return k == 0 || sh.blk != nullptr;
+                        return k == 0 || rows.blk != nullptr;
                     });
                     if (sh.abort) return RB_OK;
                     for (uint32_t q = 0; q < k; q++) { byte_base += sh.sum[q].out_bytes; row_base += sh.sum[q].n_out; }
                     if (k == 0) {  // sizes of the first slice are known: reserve the pinned output (text size extrapolated, rows bounded)
                         const uint64_t slice_bytes = sb->n_bytes;
                         const double scale = slice_bytes ? (double)total_bytes / (double)slice_bytes : 1.0;
-                        const size_t loff_bytes = (want & RB_WANT_TEXT) ? align_up((cap_rows + 1) * 8, 64) : 0;
-                        const size_t num_bytes = (want & RB_WANT_NUMERIC) ? align_up(cap_rows * 56, 64) : 0;
                         size_t text_est = 0;
                         if (want & RB_WANT_TEXT) {
                             text_est = (size_t)((double)sm.out_bytes * scale * 1.25) + (size_t)std::min<uint64_t>(4u << 20, total_bytes / 4 + 4096);  // slices differ in their rows-per-byte mix
                             if (sm.n_out == 0) text_est = (size_t)total_bytes + (size_t)cap_rows * 200 + 4096;  // nothing to extrapolate from
                         }
-                        const size_t need = 64 + align_up(text_est + 1, 64) + loff_bytes + num_bytes;
-                        cudaSetDevice(cs[0]->device);
-                        PinnedBlock* blk = pinned_get(cs[0], need);
-                        PinnedBlock* sblk = (blk && stats) ? pinned_get(cs[0], (size_t)cap_rows * 40 + 64) : nullptr;
-                        cudaSetDevice(c->device);
-                        if (!blk || (stats && !sblk)) {
-                            if (blk) blk->in_use = false;
-                            sh.rc = fail(cs[0], RB_ERR_OOM, "pinned allocation of %zu bytes failed", need);
-                            sh.err = cs[0]->err;
-                            sh.abort = true;
-                            sh.cv.notify_all();
-                            return RB_OK;
-                        }
-                        sh.base = reinterpret_cast<uint8_t*>(blk->p);
-                        const size_t text_room = (blk->cap - 64 - loff_bytes - num_bytes) / 64 * 64;  // the text gets every byte the block has beyond the tables
-                        sh.cap_text = (want & RB_WANT_TEXT) ? text_room - 64 : 0;
-                        sh.o_loff = 64 + text_room;
-                        sh.o_num = sh.o_loff + loff_bytes;
-                        sh.sblk = sblk;
-                        sh.blk = blk;
+                        rc = rows.reserve(c, cap_rows, text_est, want, stats != nullptr);  // (slice 0 is the first device's: c is ctx)
+                        if (rc != RB_OK) return rc;
                         sh.cv.notify_all();
                     }
                 }
-                if (((want & RB_WANT_TEXT) && byte_base + sm.out_bytes > sh.cap_text) || row_base + sm.n_out > cap_rows) {
+                if (((want & RB_WANT_TEXT) && byte_base + sm.out_bytes > rows.cap_text) || row_base + sm.n_out > cap_rows) {
                     // the text extrapolation was too small (or the table is not the sorted, non-nested layout the row bound assumes)
                     if (d == 0) T("text estimate too small: falling back", k);
-                    raise(c, RB_OK, true);
+                    stop(true);
                     return RB_OK;
                 }
                 // ---- device -> host of this slice on the copy stream ----
                 CU(cudaStreamWaitEvent(B, c->ev_done[j & 1], 0));
-                const uint64_t nk = sm.n_out;
-                uint8_t* base = sh.base;
-                if (want & RB_WANT_TEXT) {
-                    launch_add_u64(sb->out_line_off.as<uint64_t>(), nk, byte_base, B);  // offsets in the caller's concatenated text
-                    if (sm.out_bytes) CU(cudaMemcpyAsync(base + sh.o_text + byte_base, sb->out_text.p, sm.out_bytes, cudaMemcpyDeviceToHost, B));
-                    if (nk) CU(cudaMemcpyAsync(reinterpret_cast<uint64_t*>(base + sh.o_loff) + row_base, sb->out_line_off.p, nk * 8, cudaMemcpyDeviceToHost, B));
-                }
-                if ((want & RB_WANT_NUMERIC) && nk) {
-                    uint64_t* dn = reinterpret_cast<uint64_t*>(base + sh.o_num);
-                    const uint64_t* sp = sb->out_num.as<uint64_t>();
-                    // one strided copy per table: columns are `row_stride` rows apart on the device and cap_rows apart in the pinned block
-                    const uint64_t sk = sb->row_stride ? sb->row_stride : nk;
-                    CU(cudaMemcpy2DAsync(dn + row_base, cap_rows * 8, sp, sk * 8, nk * 8, 6, cudaMemcpyDeviceToHost, B));
-                    uint32_t* d32 = reinterpret_cast<uint32_t*>(dn + 6 * cap_rows);
-                    const uint32_t* s32 = reinterpret_cast<const uint32_t*>(sp + 6 * sk);
-                    CU(cudaMemcpy2DAsync(d32 + row_base, cap_rows * 4, s32, sk * 4, nk * 4, 2, cudaMemcpyDeviceToHost, B));
-                }
-                if (stats && nk) {
-                    uint32_t* ds = reinterpret_cast<uint32_t*>(sh.sblk->p);
-                    const uint64_t sk = sb->row_stride ? sb->row_stride : nk;
-                    CU(cudaMemcpy2DAsync(ds + row_base, cap_rows * 4, sb->out_stats.as<uint32_t>(), sk * 4, nk * 4, 10, cudaMemcpyDeviceToHost, B));
-                }
+                if (want & RB_WANT_TEXT) launch_add_u64(sb->out_line_off.as<uint64_t>(), sm.n_out, byte_base, B);  // offsets in the caller's concatenated text
+                rc = rows.copy_rows(c, sb, 0, sm.n_out, 0, sm.out_bytes, row_base, byte_base, B);
+                if (rc != RB_OK) return rc;
                 CU(cudaEventRecord(c->ev_d2h[j & 1], B));
             }
             if (d == 0) {  // rows no slice of this device needed, then the table check (its verdict is read before the call returns)
-                std::sort(rows_up.begin(), rows_up.end());
-                uint32_t at = 0;
-                for (auto& iv : rows_up) {
-                    if (rc == RB_OK && iv.first > at) rc = windows_upload_rows(c, wb, wins, at, iv.first, U);
-                    at = std::max(at, iv.second);
-                }
-                if (rc == RB_OK && at < wb->n_win) rc = windows_upload_rows(c, wb, wins, at, wb->n_win, U);
-                if (rc == RB_OK && cudaStreamWaitEvent(U, c->ev_wfirst, 0) != cudaSuccess) rc = fail(c, RB_ERR_CUDA, "cudaStreamWaitEvent");
-                if (rc == RB_OK) rc = windows_check(c, wb, recs, U);
-                if (rc == RB_OK) rc = upload_windows_end(c, wb, recs, wins);  // waits for the verdict
+                rc = wr.rest(c, wb, recs, wins, U, c->ev_wfirst);
                 if (rc != RB_OK) return rc;
                 if (wb->general) {  // nested rows / file order != sorted order: the single-batch path handles those (rare)
                     T("general window layout: falling back", 0);
-                    raise(c, RB_OK, true);
+                    stop(true);
                     return RB_OK;
                 }
             }
             CU(cudaStreamSynchronize(B));
             return RB_OK;
         };
-        const int rc = run();
-        if (rc != RB_OK) raise(c, rc, false);
+        int& status = dev.rc[(size_t)d];
+        if (status == RB_OK) status = run();
+        if (status != RB_OK) stop(false);
         // whatever happened: nothing of this call may still be in flight on this device when the function returns
         c->upload_on = nullptr;
         cudaStreamSynchronize(U);
@@ -3295,74 +3161,42 @@ static int liftover_sliced(rb_ctx* ctx, const rb_records* recs, const rb_windows
         for (int k = 0; k < 2; k++)
             if (c->slice[k]) c->slice[k]->busy = false;
         wb->busy = false;
-    };
-    std::vector<std::thread> pool;
-    for (int d = 1; d < D; d++) pool.emplace_back(work, d);
-    work(0);
-    for (auto& th : pool) th.join();
-    cudaSetDevice(ctx->device);
-    for (rb_ctx* p : ctx->peers) p->invert = false;
+    });
     T("all devices drained", n_slices);
-    if (sh.abort) {
-        if (sh.blk) sh.blk->in_use = false;
-        if (sh.sblk) sh.sblk->in_use = false;
-        if (sh.rc != RB_OK) { ctx->err = sh.err; return sh.rc; }
-        return 1;  // the exact path
-    }
+    const int rc = dev.error(true);  // the first error in record order wins
+    if (rc != RB_OK || sh.fall_back) { rows.release(); return rc != RB_OK ? rc : 1; }  // (1: the exact path)
     uint64_t row_base = 0, byte_base = 0, pairs = 0;
     for (uint32_t k = 0; k < n_slices; k++) { row_base += sh.sum[k].n_out; byte_base += sh.sum[k].out_bytes; pairs += sh.sum[k].n_pairs; }
-    uint8_t* base = sh.base;
-    out->n_out = row_base; out->paf_nbytes = byte_base; out->n_pairs = pairs; out->_owner = sh.blk;
-    if (want & RB_WANT_TEXT) {
-        out->paf_text = base + sh.o_text;
-        out->line_off = reinterpret_cast<uint64_t*>(base + sh.o_loff);
-        out->line_off[row_base] = byte_base;
-        if (row_base == 0) out->line_off[0] = 0;
-        out->paf_text[byte_base] = 0;
-    }
-    if (want & RB_WANT_NUMERIC) {
-        uint64_t* p = reinterpret_cast<uint64_t*>(base + sh.o_num);
-        out->q_st = p; out->q_en = p + cap_rows; out->t_st = p + 2 * cap_rows; out->t_en = p + 3 * cap_rows;
-        out->nmatch = p + 4 * cap_rows; out->aln_len = p + 5 * cap_rows;
-        out->rec_idx = reinterpret_cast<uint32_t*>(p + 6 * cap_rows);
-        out->win_idx = out->rec_idx + cap_rows;
-    }
-    if (stats) {
-        uint32_t* p = reinterpret_cast<uint32_t*>(sh.sblk->p);
-        const uint64_t c = cap_rows;
-        stats->n = row_base;
-        stats->equal = p; stats->diff = p + c; stats->ins = p + 2 * c; stats->del = p + 3 * c; stats->ins_events = p + 4 * c;
-        stats->del_events = p + 5 * c; stats->matches = p + 6 * c;
-        stats->id_by_matches = reinterpret_cast<float*>(p + 7 * c); stats->id_by_events = reinterpret_cast<float*>(p + 8 * c);
-        stats->id_by_all = reinterpret_cast<float*>(p + 9 * c);
-        stats->_owner = sh.sblk;
-    }
+    rows.finish(out, stats, row_base, byte_base, pairs);
     return RB_OK;
+}
+
+// query and target change places: the column pointers are swapped (the ops get inverted on the device right after tokenising)
+static rb_records swap_query_target(const rb_records& r) {
+    rb_records s = r;
+    std::swap(s.q_len, s.t_len); std::swap(s.q_st, s.t_st); std::swap(s.q_en, s.t_en);
+    std::swap(s.q_id, s.t_id);
+    return s;
 }
 
 int rb_liftover(rb_ctx* ctx, const rb_records* recs, const rb_windows* wins, int policy, uint32_t want, rb_lift_out* out,
                 rb_stats_out* stats) {
     if (!ctx) return RB_ERR_NO_DEVICE;
     if (!out) return fail(ctx, RB_ERR_BAD_ARG, "out is null");
-    // liftover --qbed (liftover.rs:139-148): every record swaps query and target first — here the column pointers
-    // change places and the ops are inverted on the device right after tokenising
+    // liftover --qbed (liftover.rs:139-148): every record swaps query and target first
+    const bool invert = (want & RB_WANT_QBED) && recs;
     rb_records swapped;
-    struct InvertScope { rb_ctx* c; ~InvertScope() { c->invert = false; } } invert_scope{ctx};
-    if ((want & RB_WANT_QBED) && recs) {
-        swapped = *recs;
-        std::swap(swapped.q_len, swapped.t_len); std::swap(swapped.q_st, swapped.t_st); std::swap(swapped.q_en, swapped.t_en);
-        std::swap(swapped.q_id, swapped.t_id);
+    if (invert) {
+        swapped = swap_query_target(*recs);
         recs = &swapped;
-        ctx->invert = true;
     }
     want &= ~RB_WANT_QBED;
-    struct StatsTextScope { rb_ctx* c; ~StatsTextScope() { c->stats_text = false; for (rb_ctx* p : c->peers) p->stats_text = false; } } st_scope{ctx};
-    if (want & RB_WANT_STATS_TEXT) {
+    const bool stats_text = (want & RB_WANT_STATS_TEXT) != 0;
+    if (stats_text) {
         if (want & RB_WANT_TEXT) return fail(ctx, RB_ERR_BAD_ARG, "RB_WANT_STATS_TEXT and RB_WANT_TEXT exclude each other");
         want = (want & ~RB_WANT_STATS_TEXT) | RB_WANT_TEXT;  // from here on the stats rows are "the text"
-        ctx->stats_text = true;
-        for (rb_ctx* p : ctx->peers) p->stats_text = true;
     }
+    CallFlags flags(ctx, invert, stats_text);
     cudaSetDevice(ctx->device);
     {   // large calls: slices dealt round-robin to the context's devices, both PCIe directions and the SMs busy at once
         const int src = liftover_sliced(ctx, recs, wins, policy, want, out, stats);
@@ -3373,7 +3207,7 @@ int rb_liftover(rb_ctx* ctx, const rb_records* recs, const rb_windows* wins, int
         if (mrc != 1) return mrc;  // (1: not spread — too small, or a window layout the single-batch path handles)
     }
     if (!ctx->scratch) ctx->scratch = new rb_batch();
-    return liftover_unsliced(ctx, recs, wins, policy, want, out, stats, false);
+    return liftover_unsliced(ctx, recs, wins, policy, want, out, stats);
 }
 
 // replaces the `for paf in records { aligned_pairs(); break_paf_on_indels(); println! }` loop of `rb break-paf`
@@ -3402,11 +3236,8 @@ int rb_invert(rb_ctx* ctx, const rb_records* recs, uint32_t want, rb_lift_out* o
     cudaSetDevice(ctx->device);
     if (!ctx->scratch) ctx->scratch = new rb_batch();
     rb_batch* b = ctx->scratch;
-    rb_records swapped = *recs;  // the column pointers change places; the ops are inverted on the device after tokenising
-    std::swap(swapped.q_len, swapped.t_len); std::swap(swapped.q_st, swapped.t_st); std::swap(swapped.q_en, swapped.t_en);
-    std::swap(swapped.q_id, swapped.t_id);
-    struct InvertScope { rb_ctx* c; ~InvertScope() { c->invert = false; } } invert_scope{ctx};
-    ctx->invert = true;
+    const rb_records swapped = swap_query_target(*recs);
+    CallFlags flags(ctx, true, false);
     b->file_order = true;
     int rc = upload_into(ctx, b, &swapped, nullptr);
     b->file_order = false;
