@@ -279,6 +279,19 @@ int rb_batch_windows(rb_ctx* ctx, rb_batch* b, rb_windows* out);
 int rb_liftover_text(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, const uint8_t* bed, uint64_t bed_nbytes, int policy,
                      uint32_t want, rb_lift_out* out, rb_stats_out* stats /* nullable */, rb_paf_info* paf_info, rb_bed_info* bed_info);
 
+/* `rb stats --paf [--qbed]` from the file's bytes: paf = plain text or BGZF (rb_is_bgzf), as rb_batch_upload_paf takes it.
+ * One row per record in FILE order (main.rs:53-56).  With RB_WANT_STATS_TEXT, rows->paf_text / line_off hold the rows the reference
+ * prints (bamstats.rs:239-270), formatted on the device; want = 0: only the counters (stats).  Any other want bit -> RB_ERR_BAD_ARG.
+ * qbed != 0 prints the query block first (the `--qbed` column order).  The header line (main.rs:51) is the caller's.
+ * rows->n_out = the record count, n_pairs = n_out, the numeric mirror is NULL.  The coordinates are the record's columns as read
+ * (stats_from_paf strips nothing).  stats (nullable) receives the counters and identities of rb_stats, bit for bit.
+ * On an N-device context the PAF is split into N byte ranges cut at line starts, as rb_liftover_text splits it (a PAF below
+ * multi_min_bytes stays on the first device).  Errors, statuses and messages: those of rb_batch_upload_paf + rb_batch_stats; line
+ * numbers and record indices count over the whole file.  info is nullable and is filled once the PAF has parsed (also when a later
+ * step fails); info->names stays valid until the next call on ctx. */
+int rb_stats_text(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, int qbed, uint32_t want, rb_lift_out* rows,
+                  rb_stats_out* stats /* nullable */, rb_paf_info* info);
+
 /* ---- host helper: stable sort of BED rows by (t_id, st) into the rb_windows layout ----
  * perm_out[n_win] receives, for each sorted position, the BED row it came from. */
 int rb_sort_windows(uint32_t n_win, const uint32_t* t_id, const uint64_t* st, uint32_t* perm_out);

@@ -87,6 +87,9 @@ extern "C" {
     /// `rb liftover --bed` from the files' bytes (PAF and BED text or BGZF), the PAF parsed across every device of the context
     pub fn rb_liftover_text(ctx: *mut rb_ctx, paf: *const u8, paf_nbytes: u64, bed: *const u8, bed_nbytes: u64, policy: c_int, want: u32,
                             out: *mut rb_lift_out, stats: *mut rb_stats_out, paf_info: *mut rb_paf_info, bed_info: *mut rb_bed_info) -> c_int;
+    /// `rb stats --paf [--qbed]` from the file's bytes (PAF text or BGZF): the rows formatted on the device(s), in file order
+    pub fn rb_stats_text(ctx: *mut rb_ctx, paf: *const u8, paf_nbytes: u64, qbed: c_int, want: u32, rows: *mut rb_lift_out,
+                         stats: *mut rb_stats_out, info: *mut rb_paf_info) -> c_int;
     pub fn rb_batch_liftover(ctx: *mut rb_ctx, b: *mut rb_batch, policy: c_int, want: u32, with_stats: c_int, summary: *mut rb_summary) -> c_int;
     pub fn rb_batch_download_lift(ctx: *mut rb_ctx, b: *mut rb_batch, want: u32, out: *mut rb_lift_out, stats: *mut rb_stats_out) -> c_int;
     pub fn rb_batch_free(ctx: *mut rb_ctx, b: *mut rb_batch);

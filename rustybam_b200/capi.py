@@ -27,7 +27,7 @@ EXPORTS = [
     "rb_liftover", "rb_stats", "rb_break_paf", "rb_invert", "rb_trim_paf", "rb_trim_paf_begin", "rb_trim_paf_round", "rb_trim_paf_end", "rb_batch_break", "rb_free_lift_out", "rb_free_stats_out", "rb_batch_upload", "rb_batch_liftover", "rb_batch_stats",
     "rb_batch_download_lift", "rb_batch_download_stats", "rb_batch_free", "rb_sort_windows", "rb_version", "rb_host_register",
     "rb_host_unregister", "rb_is_bgzf", "rb_inflate_bgzf", "rb_free_text", "rb_batch_upload_paf", "rb_batch_set_windows", "rb_batch_records",
-    "rb_batch_set_windows_bed", "rb_batch_windows", "rb_liftover_text",
+    "rb_batch_set_windows_bed", "rb_batch_windows", "rb_liftover_text", "rb_stats_text",
 ]
 
 u8p, u32p, u64p, f32p = C.POINTER(C.c_uint8), C.POINTER(C.c_uint32), C.POINTER(C.c_uint64), C.POINTER(C.c_float)
@@ -134,6 +134,8 @@ def load():
     lib.rb_batch_windows.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(RbWindows)]
     lib.rb_liftover_text.argtypes = [C.c_void_p, C.c_char_p, C.c_uint64, C.c_char_p, C.c_uint64, C.c_int, C.c_uint32, C.POINTER(RbLiftOut),
                                      C.POINTER(RbStatsOut), C.POINTER(RbPafInfo), C.POINTER(RbBedInfo)]
+    lib.rb_stats_text.argtypes = [C.c_void_p, C.c_char_p, C.c_uint64, C.c_int, C.c_uint32, C.POINTER(RbLiftOut), C.POINTER(RbStatsOut),
+                                  C.POINTER(RbPafInfo)]
     lib.rb_host_register.argtypes = [C.c_void_p, C.c_uint64]
     lib.rb_host_unregister.argtypes = [C.c_void_p]
     _lib = lib
@@ -213,6 +215,14 @@ def _np(ptr, n, dtype):
     if n == 0 or not ptr:
         return np.zeros(0, dtype=dtype)
     return np.ctypeslib.as_array(ptr, shape=(n,)).copy()
+
+
+def _paf_info(pi):
+    nn = int(pi.n_names)
+    off = _np(pi.names_off, nn + 1, np.uint64) if pi.names_off else np.zeros(1, np.uint64)
+    blob = C.string_at(pi.names, int(off[-1])) if nn and int(off[-1]) else b""
+    return dict(names=[blob[int(off[i]):int(off[i + 1])] for i in range(nn)], n_rec=int(pi.n_rec), n_lines=int(pi.n_lines),
+                skipped=int(pi.skipped), text_bytes=int(pi.text_bytes), cigar_bytes=int(pi.cigar_bytes))
 
 
 class Context:
@@ -405,12 +415,21 @@ class Context:
         self.lib.rb_free_lift_out(self.h, C.byref(out))
         if stats:
             self.lib.rb_free_stats_out(self.h, C.byref(st))
-        nn = int(pi.n_names)
-        off = _np(pi.names_off, nn + 1, np.uint64) if pi.names_off else np.zeros(1, np.uint64)
-        blob = C.string_at(pi.names, int(off[-1])) if nn and int(off[-1]) else b""
-        res["paf_info"] = dict(names=[blob[int(off[i]):int(off[i + 1])] for i in range(nn)], n_rec=int(pi.n_rec), n_lines=int(pi.n_lines),
-                               skipped=int(pi.skipped), text_bytes=int(pi.text_bytes), cigar_bytes=int(pi.cigar_bytes))
+        res["paf_info"] = _paf_info(pi)
         res["bed_info"] = {k: int(getattr(bi, k)) for k, _ in RbBedInfo._fields_}
+        return res
+
+    def stats_text(self, paf: bytes, qbed=False, want=WANT_STATS_TEXT, stats=True):
+        """rb_stats_text: PAF bytes (text or BGZF) in, the rows of `rb stats --paf [--qbed]` (without the header line) out, one per
+        record in file order; on a multi-device context every device parses and formats its share.  The dict of liftover_text()
+        without "bed_info"; want=0 returns the counters only."""
+        out, st, pi = RbLiftOut(), RbStatsOut(), RbPafInfo()
+        self._check(self.lib.rb_stats_text(self.h, paf, len(paf), int(bool(qbed)), want, C.byref(out), C.byref(st) if stats else None, C.byref(pi)))
+        res = self._collect_lift(out, st if stats else None, WANT_TEXT if want & WANT_STATS_TEXT else 0)
+        self.lib.rb_free_lift_out(self.h, C.byref(out))
+        if stats:
+            self.lib.rb_free_stats_out(self.h, C.byref(st))
+        res["paf_info"] = _paf_info(pi)
         return res
 
     # ---- resident batches ----

@@ -135,9 +135,10 @@ RB_HD void f32_mul_64x32(uint64_t a, uint32_t b, uint64_t& hi, uint64_t& lo) {  
     lo = l + (h << 32);
     hi = (h >> 32) + (lo < l ? 1ull : 0ull);
 }
-// the big-integer core as a call of its own (its 256-bit temporaries live on the stack: kept out of the caller's frame)
+// the big-integer core as a call of its own (its 256-bit temporaries live on the stack: kept out of the caller's frame); static: one
+// copy in every translation unit that uses it
 #if defined(__CUDACC__)
-__host__ __device__ __noinline__
+static __host__ __device__ __noinline__
 #else
 inline
 #endif

@@ -266,6 +266,12 @@ void launch_contig_runs(uint64_t n, const uint32_t* rec_idx, uint32_t rec_base, 
                         const uint64_t* line_off, uint64_t out_bytes, uint64_t* runs, uint32_t n_ranks, cudaStream_t s);
 void launch_rebase_runs(uint64_t n, const uint32_t* rec_idx, uint32_t rec_base, const uint32_t* t_id, const uint32_t* rank_of,
                         const uint64_t* delta, uint64_t* line_off, cudaStream_t s);
+// rb_stats_text (stats_row_kernels.cu): the `rb stats --paf` rows of a batch's records after rb_batch_stats.  line_off: n_rec + 1
+// entries; launch_stats_row_len leaves the row lengths there, launch_stats_row_scan (tmp nullptr: tmp_bytes = the scratch it needs)
+// turns them into offsets in place with the total at [n_rec], launch_stats_rows writes the rows.
+void launch_stats_row_len(const RecInput& in, const StatsDev& st, uint64_t* line_off, cudaStream_t s);
+cudaError_t launch_stats_row_scan(uint64_t* line_off, uint32_t n_rec, void* tmp, size_t& tmp_bytes, cudaStream_t s);
+void launch_stats_rows(const RecInput& in, const StatsDev& st, const uint64_t* line_off, uint8_t* out, bool qbed, cudaStream_t s);
 // BED text -> the window tables of a batch (bed_parse_kernels.cu; the rules are bed_parse_core.cuh's).  Per-line columns:
 struct BedLineCols {
     const uint64_t* line_start;

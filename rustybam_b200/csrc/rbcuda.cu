@@ -2521,6 +2521,167 @@ struct CallFlags {
         for (rb_ctx* p : ctx->peers) { p->invert = invert; p->stats_text = stats_text; }
     }
 };
+
+// Steps 1 - 3 of a text call on the D devices of a context (rb_liftover_text, rb_stats_text), one host thread per device:
+//   split  plain text: D equal byte ranges, each uploaded by its own device; BGZF: runs of whole blocks balanced on ISIZE, each
+//          inflated by its own device.  k_first_newline finds each range's first '\n'; text_split.hpp says which bytes each device
+//          parses, and every device gathers them into a fresh buffer (its own bytes: a device copy; the others': peer copies).
+//   parse  steps 1 - 3 of rb_batch_upload_paf on every device at once; then the host interns the names device by device (file
+//          order: the ids of one device) and ranks the contigs by first appearance in the whole file.  Device d holds records
+//          rec_base .. rec_base + p.n_rec of the file; the first error or panic in file order fails the call.
+struct TextParts {
+    struct Part {
+        DevBuf range, own;
+        uint64_t n = 0, first_nl = rbt::NO_NEWLINE, rec_base = 0;
+        uint8_t last = 0;  // the range's last byte
+        PafParsed p;
+    };
+    Devices& dev;
+    Rendezvous& rv;
+    int& call_rc;
+    const uint8_t* paf;
+    uint64_t paf_nbytes;
+    bool bgzf = false;
+    std::vector<uint64_t> src, blk_base;
+    std::vector<Part> part;
+    std::vector<rbt::Owned> plan;
+    std::vector<uint32_t> rank_of;  // name id -> contig rank (first appearance as t_name in the file)
+    uint32_t n_ranks = 0, n_names = 0;
+    rb_batch* b0 = nullptr;         // holds the name table: the first device's scratch batch
+
+    TextParts(Devices& d, Rendezvous& r, int& rc, const uint8_t* data, uint64_t n)
+        : dev(d), rv(r), call_rc(rc), paf(data), paf_nbytes(n), part((size_t)d.n) {}
+
+    // on the caller's thread, before Devices::run: the input's byte ranges
+    int split() {
+        rb_ctx* ctx = dev.ctx;
+        const int D = dev.n;
+        bgzf = rb_is_bgzf(paf, paf_nbytes) != 0;
+        if (!bgzf && paf_nbytes >= 2 && paf[0] == 0x1f && paf[1] == 0x8b)
+            return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_upload_paf: a plain gzip stream (not BGZF); inflate it first");
+        src.assign((size_t)D + 1, paf_nbytes);
+        blk_base.assign((size_t)D, 0);
+        src[0] = 0;
+        if (bgzf) {
+            std::vector<BgzfBlock> blocks;
+            std::vector<uint64_t> starts;
+            uint64_t total = 0;
+            if (!bgzf_blocks(paf, paf_nbytes, blocks, total, &starts)) return fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: not a well-formed series of BGZF blocks");
+            size_t k = 0;
+            for (int d = 1; d < D; d++) {
+                const uint64_t target = total / (uint64_t)D * (uint64_t)d + total % (uint64_t)D * (uint64_t)d / (uint64_t)D;
+                while (k < blocks.size() && blocks[k].out_off < target) k++;
+                src[(size_t)d] = k < blocks.size() ? starts[k] : paf_nbytes;
+                blk_base[(size_t)d] = k;
+            }
+        } else {
+            for (int d = 1; d < D; d++) src[(size_t)d] = paf_nbytes / (uint64_t)D * (uint64_t)d + paf_nbytes % (uint64_t)D * (uint64_t)d / (uint64_t)D;
+        }
+        b0 = ctx->scratch ? ctx->scratch : (ctx->scratch = new rb_batch());
+        return RB_OK;
+    }
+
+    // device d's thread (c: its context, b: its scratch batch): steps 1 - 3 and the interning; info is filled once the whole PAF has
+    // parsed.  false: the call has failed (call_rc); the caller releases the part either way.
+    bool parse(int d, rb_ctx* c, rb_paf_info* info) {
+        const int D = dev.n;
+        Part& me = part[(size_t)d];
+        int& status = dev.rc[(size_t)d];
+        rb_batch* b = c->scratch;
+        cudaStream_t s = c->stream;
+        uint32_t* sc = c->scalars.as<uint32_t>();
+        volatile uint64_t* hs = reinterpret_cast<volatile uint64_t*>(c->h_scalars);
+        // 1. this device's range -> HBM, its first '\n'
+        if (status == RB_OK) status = [&]() -> int {
+            rb_ctx* ctx = c;  // (CU reports into this device's context)
+            const uint64_t len = src[(size_t)d + 1] - src[(size_t)d];
+            if (bgzf) {
+                const int rc = inflate_to_device(c, paf + src[(size_t)d], len, me.range, me.n, TEXT_PAD, blk_base[(size_t)d]);
+                if (rc != RB_OK) return rc;
+            } else {
+                me.n = len;
+                CU(me.range.ensure(len + TEXT_PAD));
+                if (len) CU(h2d_copy(me.range.p, paf + src[(size_t)d], len, s));
+            }
+            if (me.n) {
+                CU(cudaMemsetAsync(sc + SC_ERR_TOK, 0xFF, 8, s));
+                {
+                    KScope k(c, "k_first_newline");
+                    launch_first_newline(me.range.as<uint8_t>(), me.n, reinterpret_cast<unsigned long long*>(sc + SC_ERR_TOK), s);
+                }
+                Publisher(c).u64(0, sc + SC_ERR_TOK).go(s);
+            }
+            CU(cudaStreamSynchronize(s));
+            if (me.n) {
+                me.first_nl = hs[0];
+                CU(cudaMemcpy(&me.last, me.range.as<uint8_t>() + me.n - 1, 1, cudaMemcpyDeviceToHost));
+            }
+            return RB_OK;
+        }();
+        rv.meet([&] {
+            call_rc = dev.error(false);
+            if (call_rc != RB_OK) return;
+            std::vector<uint64_t> size((size_t)D), nl((size_t)D);
+            std::vector<uint8_t> ends_nl((size_t)D);
+            for (int k = 0; k < D; k++) {
+                size[(size_t)k] = part[(size_t)k].n; nl[(size_t)k] = part[(size_t)k].first_nl;
+                ends_nl[(size_t)k] = part[(size_t)k].n && part[(size_t)k].last == '\n';
+            }
+            plan = rbt::plan_line_split(size, nl, ends_nl);
+        });
+        if (call_rc != RB_OK) return false;
+        // 2. the lines this device owns -> one fresh buffer
+        status = [&]() -> int {
+            rb_ctx* ctx = c;  // (CU reports into this device's context)
+            const rbt::Owned& o = plan[(size_t)d];
+            CU(me.own.ensure(o.bytes + TEXT_PAD));
+            uint64_t at = 0;
+            for (const rbt::Piece& pc : o.pieces) {
+                const Part& from = part[(size_t)pc.src];
+                if (pc.src == d) CU(cudaMemcpyAsync(me.own.as<uint8_t>() + at, from.range.as<uint8_t>() + pc.off, pc.len, cudaMemcpyDeviceToDevice, s));
+                else CU(cudaMemcpyPeerAsync(me.own.as<uint8_t>() + at, c->device, from.range.as<uint8_t>() + pc.off, dev.at(pc.src)->device, pc.len, s));
+                at += pc.len;
+            }
+            CU(cudaStreamSynchronize(s));
+            return RB_OK;
+        }();
+        rv.meet([&] { call_rc = dev.error(false); });  // (every copy out of the ranges has finished)
+        me.range.release();
+        if (call_rc != RB_OK) return false;
+        // 3. parse
+        status = paf_parse_text(c, b, me.own.as<uint8_t>(), plan[(size_t)d].bytes, me.p);
+        me.own.release();
+        rv.meet([&] {
+            rb_ctx* ctx = dev.ctx;
+            uint64_t lines = 0, recs = 0, text = 0, cg = 0;
+            for (int k = 0; k < D; k++) {  // the first error or panic in file order
+                Part& o = part[(size_t)k];
+                if (dev.rc[(size_t)k] != RB_OK) { call_rc = dev.error(false); return; }  // (k is the first failing device)
+                if (o.p.panic != ~0ull) { call_rc = paf_panic(ctx, o.p.panic, lines); return; }
+                o.rec_base = recs;
+                lines += o.p.n_lines; recs += o.p.n_rec; text += o.p.text_bytes; cg += o.p.cg_bytes;
+            }
+            if (lines > 0xFFFFFFFFull) { call_rc = fail(ctx, RB_ERR_REF_PAF_PARSE, "more than 2^32 lines"); return; }
+            std::unordered_map<std::string, uint32_t> index;
+            b0->h_names.clear();
+            b0->h_names_off.assign(1, 0);
+            for (int k = 0; k < D; k++) paf_intern(part[(size_t)k].p, index, b0->h_names, b0->h_names_off);
+            n_names = (uint32_t)(b0->h_names_off.size() - 1);
+            rank_of.assign(n_names, UINT32_MAX);
+            for (int k = 0; k < D; k++) {
+                const PafParsed& q = part[(size_t)k].p;
+                for (uint32_t r = 0; r < q.n_rec; r++) {
+                    const uint32_t t = q.ids[(size_t)q.n_rec + r];
+                    if (rank_of[t] == UINT32_MAX) rank_of[t] = n_ranks++;
+                }
+            }
+            for (uint32_t& r : rank_of) if (r == UINT32_MAX) r = 0;  // (query-only names: never looked up)
+            paf_fill_info(info, text, lines, recs, b0->h_names, b0->h_names_off, cg);
+        });
+        return call_rc == RB_OK;
+    }
+    void release(int d) { part[(size_t)d].range.release(); part[(size_t)d].own.release(); }
+};
 }  // namespace
 }  // extern "C++"
 
@@ -2641,12 +2802,8 @@ static int stats_multi(rb_ctx* ctx, const rb_records* recs, rb_stats_out* stats)
 // ---- rb_liftover_text: PAF and BED bytes in, the rows of `rb liftover` out -----------------------------------------------------
 // One device (or a PAF below multi_min_bytes): rb_batch_upload_paf, rb_batch_set_windows_bed, rb_batch_liftover and the download on
 // the context's scratch batch.  D devices, one host thread each:
-//   split    plain text: D equal byte ranges, each uploaded by its own device; BGZF: runs of whole blocks balanced on ISIZE, each
-//            inflated by its own device.  k_first_newline finds each range's first '\n'; text_split.hpp says which bytes each device
-//            parses, and every device gathers them into a fresh buffer (its own bytes: a device copy; the others': peer copies).
-//   parse    steps 1 - 3 of rb_batch_upload_paf on every device at once; then the host interns the names device by device (file
-//            order: the ids of one device), ranks the contigs by first appearance in the whole file, and every device gets the
-//            global name table, its ids, the emission order (contig rank, file index) and rec_base = records on devices before it.
+//   split, parse  TextParts; then every device gets the global name table, its ids, the emission order (contig rank, file index)
+//            and rec_base = records on devices before it.
 //   windows  every device parses the whole BED against the same name table: identical tables and verdicts everywhere.
 //   lift     rb_batch_liftover everywhere (rec_idx always materialised); a lift error reports the smallest global record index.
 //   merge    global order = (contig rank, device): k_contig_runs finds each contig's rows on a device, the host lays out ONE pinned
@@ -2679,154 +2836,44 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
                                uint32_t want, rb_lift_out* out, rb_stats_out* stats, rb_paf_info* paf_info, rb_bed_info* bed_info) {
     Devices dev(ctx);
     const int D = dev.n;
-    // 1. the input's byte ranges
-    const bool bgzf = rb_is_bgzf(paf, paf_nbytes) != 0;
-    if (!bgzf && paf_nbytes >= 2 && paf[0] == 0x1f && paf[1] == 0x8b)
-        return fail(ctx, RB_ERR_BAD_ARG, "rb_batch_upload_paf: a plain gzip stream (not BGZF); inflate it first");
-    std::vector<uint64_t> src((size_t)D + 1, paf_nbytes), blk_base((size_t)D, 0);
-    src[0] = 0;
-    if (bgzf) {
-        std::vector<BgzfBlock> blocks;
-        std::vector<uint64_t> starts;
-        uint64_t total = 0;
-        if (!bgzf_blocks(paf, paf_nbytes, blocks, total, &starts)) return fail(ctx, RB_ERR_BAD_ARG, "rb_inflate_bgzf: not a well-formed series of BGZF blocks");
-        size_t k = 0;
-        for (int d = 1; d < D; d++) {
-            const uint64_t target = total / (uint64_t)D * (uint64_t)d + total % (uint64_t)D * (uint64_t)d / (uint64_t)D;
-            while (k < blocks.size() && blocks[k].out_off < target) k++;
-            src[(size_t)d] = k < blocks.size() ? starts[k] : paf_nbytes;
-            blk_base[(size_t)d] = k;
-        }
-    } else {
-        for (int d = 1; d < D; d++) src[(size_t)d] = paf_nbytes / (uint64_t)D * (uint64_t)d + paf_nbytes % (uint64_t)D * (uint64_t)d / (uint64_t)D;
-    }
+    Rendezvous rv(D);
+    int call_rc = RB_OK;
+    TextParts tp(dev, rv, call_rc, paf, paf_nbytes);
+    const int src_rc = tp.split();
+    if (src_rc != RB_OK) return src_rc;
     const uint32_t want_lift = want | RB_WANT_NUMERIC;  // (rec_idx places the rows)
     const bool want_text = (want & (RB_WANT_TEXT | RB_WANT_STATS_TEXT)) != 0;
 
     struct Dev {
-        DevBuf range, own, rank, runs_d, delta;
-        uint64_t n = 0, first_nl = rbt::NO_NEWLINE, rec_base = 0;
-        uint8_t last = 0;  // the range's last byte
-        PafParsed p;
+        DevBuf rank, runs_d, delta;
         rb_bed_info bi{};
         rb_summary sum{};
         std::vector<uint64_t> runs;            // row lo / row hi / byte lo / byte hi per contig rank
         std::vector<uint64_t> at_row, at_byte; // where each of its cells goes in the merged output
     };
     std::vector<Dev> dv((size_t)D);
-    Rendezvous rv(D);
-    std::vector<rbt::Owned> plan;
-    std::vector<uint32_t> rank_of;  // name id -> contig rank (first appearance as t_name in the file)
-    uint32_t n_ranks = 0, n_names = 0;
-    rb_batch* b0 = ctx->scratch ? ctx->scratch : (ctx->scratch = new rb_batch());
+    const std::vector<uint32_t>& rank_of = tp.rank_of;
+    const uint32_t& n_ranks = tp.n_ranks;
     RowsOut rows;
     uint64_t tot_rows = 0, tot_bytes = 0, tot_pairs = 0;
-    int call_rc = RB_OK;
 
     dev.run([&](int d, rb_ctx* c) {
         Dev& me = dv[(size_t)d];
         int& status = dev.rc[(size_t)d];
         rb_batch* b = c->scratch;
         cudaStream_t s = c->stream;
-        uint32_t* sc = c->scalars.as<uint32_t>();
-        volatile uint64_t* hs = reinterpret_cast<volatile uint64_t*>(c->h_scalars);
         auto cleanup = [&] {
             if (b->busy) { cudaStreamSynchronize(s); b->busy = false; }
-            me.range.release(); me.own.release(); me.rank.release(); me.runs_d.release(); me.delta.release();
+            tp.release(d);
+            me.rank.release(); me.runs_d.release(); me.delta.release();
         };
-        // 1. this device's range -> HBM, its first '\n'
-        if (status == RB_OK) status = [&]() -> int {
-            rb_ctx* ctx = c;  // (CU reports into this device's context)
-            const uint64_t len = src[(size_t)d + 1] - src[(size_t)d];
-            if (bgzf) {
-                const int rc = inflate_to_device(c, paf + src[(size_t)d], len, me.range, me.n, TEXT_PAD, blk_base[(size_t)d]);
-                if (rc != RB_OK) return rc;
-            } else {
-                me.n = len;
-                CU(me.range.ensure(len + TEXT_PAD));
-                if (len) CU(h2d_copy(me.range.p, paf + src[(size_t)d], len, s));
-            }
-            if (me.n) {
-                CU(cudaMemsetAsync(sc + SC_ERR_TOK, 0xFF, 8, s));
-                {
-                    KScope k(c, "k_first_newline");
-                    launch_first_newline(me.range.as<uint8_t>(), me.n, reinterpret_cast<unsigned long long*>(sc + SC_ERR_TOK), s);
-                }
-                Publisher(c).u64(0, sc + SC_ERR_TOK).go(s);
-            }
-            CU(cudaStreamSynchronize(s));
-            if (me.n) {
-                me.first_nl = hs[0];
-                CU(cudaMemcpy(&me.last, me.range.as<uint8_t>() + me.n - 1, 1, cudaMemcpyDeviceToHost));
-            }
-            return RB_OK;
-        }();
-        rv.meet([&] {
-            call_rc = dev.error(false);
-            if (call_rc != RB_OK) return;
-            std::vector<uint64_t> size((size_t)D), nl((size_t)D);
-            std::vector<uint8_t> ends_nl((size_t)D);
-            for (int k = 0; k < D; k++) {
-                size[(size_t)k] = dv[(size_t)k].n; nl[(size_t)k] = dv[(size_t)k].first_nl;
-                ends_nl[(size_t)k] = dv[(size_t)k].n && dv[(size_t)k].last == '\n';
-            }
-            plan = rbt::plan_line_split(size, nl, ends_nl);
-        });
-        if (call_rc != RB_OK) { cleanup(); return; }
-        // 2. the lines this device owns -> one fresh buffer
-        status = [&]() -> int {
-            rb_ctx* ctx = c;  // (CU reports into this device's context)
-            const rbt::Owned& o = plan[(size_t)d];
-            CU(me.own.ensure(o.bytes + TEXT_PAD));
-            uint64_t at = 0;
-            for (const rbt::Piece& pc : o.pieces) {
-                const Dev& from = dv[(size_t)pc.src];
-                if (pc.src == d) CU(cudaMemcpyAsync(me.own.as<uint8_t>() + at, from.range.as<uint8_t>() + pc.off, pc.len, cudaMemcpyDeviceToDevice, s));
-                else CU(cudaMemcpyPeerAsync(me.own.as<uint8_t>() + at, c->device, from.range.as<uint8_t>() + pc.off, dev.at(pc.src)->device, pc.len, s));
-                at += pc.len;
-            }
-            CU(cudaStreamSynchronize(s));
-            return RB_OK;
-        }();
-        rv.meet([&] { call_rc = dev.error(false); });  // (every copy out of the ranges has finished)
-        me.range.release();
-        if (call_rc != RB_OK) { cleanup(); return; }
-        // 3. parse
-        status = paf_parse_text(c, b, me.own.as<uint8_t>(), plan[(size_t)d].bytes, me.p);
-        me.own.release();
-        rv.meet([&] {
-            uint64_t lines = 0, recs = 0, text = 0, cg = 0;
-            for (int k = 0; k < D; k++) {  // the first error or panic in file order
-                Dev& o = dv[(size_t)k];
-                if (dev.rc[(size_t)k] != RB_OK) { call_rc = dev.error(false); return; }  // (k is the first failing device)
-                if (o.p.panic != ~0ull) { call_rc = paf_panic(ctx, o.p.panic, lines); return; }
-                o.rec_base = recs;
-                lines += o.p.n_lines; recs += o.p.n_rec; text += o.p.text_bytes; cg += o.p.cg_bytes;
-            }
-            if (lines > 0xFFFFFFFFull) { call_rc = fail(ctx, RB_ERR_REF_PAF_PARSE, "more than 2^32 lines"); return; }
-            std::unordered_map<std::string, uint32_t> index;
-            b0->h_names.clear();
-            b0->h_names_off.assign(1, 0);
-            for (int k = 0; k < D; k++) paf_intern(dv[(size_t)k].p, index, b0->h_names, b0->h_names_off);
-            n_names = (uint32_t)(b0->h_names_off.size() - 1);
-            rank_of.assign(n_names, UINT32_MAX);
-            for (int k = 0; k < D; k++) {
-                const PafParsed& q = dv[(size_t)k].p;
-                for (uint32_t r = 0; r < q.n_rec; r++) {
-                    const uint32_t t = q.ids[(size_t)q.n_rec + r];
-                    if (rank_of[t] == UINT32_MAX) rank_of[t] = n_ranks++;
-                }
-            }
-            for (uint32_t& r : rank_of) if (r == UINT32_MAX) r = 0;  // (query-only names: never looked up)
-            paf_fill_info(paf_info, text, lines, recs, b0->h_names, b0->h_names_off, cg);
-        });
-        if (call_rc != RB_OK) { cleanup(); return; }
+        if (!tp.parse(d, c, paf_info)) { cleanup(); return; }
         // 4. names, windows, lift, the contig runs of the rows
         status = [&]() -> int {
             rb_ctx* ctx = c;  // (CU reports into this device's context)
-            int rc = paf_upload_names(c, b, me.p, b0->h_names.data(), b0->h_names_off.data(), n_names, rank_of.data());
+            int rc = paf_upload_names(c, b, tp.part[(size_t)d].p, tp.b0->h_names.data(), tp.b0->h_names_off.data(), tp.n_names, rank_of.data());
             if (rc != RB_OK) return rc;
-            b->rec_base = (uint32_t)me.rec_base;
+            b->rec_base = (uint32_t)tp.part[(size_t)d].rec_base;
             CU(cudaStreamSynchronize(s));
             b->busy = false;
             rc = bed_upload_into(c, b, bed, bed_nbytes, &me.bi);
@@ -2834,9 +2881,9 @@ static int liftover_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nby
             rc = rb_batch_liftover(c, b, policy, want_lift, stats != nullptr, &me.sum);
             if (rc != RB_OK) return rc;
             const uint64_t nk = me.sum.n_out, sk = b->row_stride ? b->row_stride : nk;
-            CU(me.rank.ensure((size_t)n_names * 4 + 8));
+            CU(me.rank.ensure((size_t)tp.n_names * 4 + 8));
             CU(me.runs_d.ensure((size_t)n_ranks * 32 + 64));
-            if (n_names) CU(cudaMemcpyAsync(me.rank.p, rank_of.data(), (size_t)n_names * 4, cudaMemcpyHostToDevice, s));
+            if (tp.n_names) CU(cudaMemcpyAsync(me.rank.p, rank_of.data(), (size_t)tp.n_names * 4, cudaMemcpyHostToDevice, s));
             CU(cudaMemsetAsync(me.runs_d.p, 0, (size_t)n_ranks * 32, s));
             {
                 KScope k(c, "k_contig_runs");
@@ -2932,6 +2979,155 @@ int rb_liftover_text(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, const
     if (rc != RB_OK) {
         if (paf_info && !paf_info->names_off) memset(paf_info, 0, sizeof *paf_info);
         memset(out, 0, sizeof *out);
+        if (stats) memset(stats, 0, sizeof *stats);
+    }
+    return rc;
+}
+
+// ---- rb_stats_text: PAF bytes in, the rows of `rb stats --paf` out --------------------------------------------------------------
+// rb_batch_stats (k_rec_prep mode 0), then k_stats_rows on the batch's resident columns: the rows of its records in out_text /
+// out_line_off (text), laid out for RowsOut::copy_rows like the rows of a liftover — n_out = n_rec, the Stats columns n_rec apart.
+static int batch_stats_rows(rb_ctx* ctx, rb_batch* b, int qbed, bool text) {
+    cudaStream_t s = ctx->stream;
+    const uint32_t n = b->n_rec;
+    b->sum.n_out = n; b->sum.n_pairs = n; b->sum.out_bytes = 0; b->row_stride = n;
+    if (n == 0) return RB_OK;
+    int rc = rb_batch_stats(ctx, b, nullptr);
+    if (rc != RB_OK || !text) return rc;
+    const RecInput in = rec_input(b);
+    const StatsDev st = stats_view(b, n);
+    CU(b->out_line_off.ensure(((size_t)n + 1) * 8));
+    uint64_t* loff = b->out_line_off.as<uint64_t>();
+    {
+        KScope k(ctx, "k_stats_row_len");
+        launch_stats_row_len(in, st, loff, s);
+    }
+    size_t tmp = 0;
+    CU(launch_stats_row_scan(loff, n, nullptr, tmp, s));
+    CU(b->line_len.ensure(tmp + 16));
+    {
+        KScope k(ctx, "cub_scan_row_len");
+        CU(launch_stats_row_scan(loff, n, b->line_len.p, tmp, s));
+    }
+    volatile uint64_t* hs = reinterpret_cast<volatile uint64_t*>(ctx->h_scalars);
+    Publisher(ctx).u64(0, loff + n).go(s);
+    CU(cudaStreamSynchronize(s));
+    const uint64_t nb = hs[0];
+    CU(b->out_text.ensure(nb + 64));
+    {
+        KScope k(ctx, "k_stats_rows");
+        launch_stats_rows(in, st, loff, b->out_text.as<uint8_t>(), qbed != 0, s);
+    }
+    CU(cudaGetLastError());
+    b->sum.out_bytes = nb;
+    return RB_OK;
+}
+
+// One device (or a PAF below multi_min_bytes): the batch path on the context's scratch batch.
+static int stats_text_one(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, int qbed, bool text, rb_lift_out* out, rb_stats_out* stats,
+                          rb_paf_info* info) {
+    if (!ctx->scratch) ctx->scratch = new rb_batch();
+    rb_batch* b = ctx->scratch;
+    if (b->busy) { CU(cudaStreamSynchronize(ctx->stream)); b->busy = false; }
+    int rc = paf_upload_into(ctx, b, paf, paf_nbytes, info);
+    if (rc == RB_OK && cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+        (void)cudaGetLastError();
+        rc = fail(ctx, RB_ERR_CUDA, "upload failed");
+    }
+    b->busy = false;
+    if (rc == RB_OK) rc = batch_stats_rows(ctx, b, qbed, text);
+    RowsOut rows;
+    if (rc == RB_OK) rc = rows.reserve(ctx, b->n_rec, b->sum.out_bytes, text ? RB_WANT_TEXT : 0u, stats != nullptr);
+    if (rc == RB_OK) rc = rows.copy_rows(ctx, b, 0, b->n_rec, 0, b->sum.out_bytes, 0, 0, ctx->stream);
+    rc = download_wait(ctx, rows, rc);
+    if (rc == RB_OK) rows.finish(out, stats, b->n_rec, b->sum.out_bytes, b->n_rec);
+    else cudaStreamSynchronize(ctx->stream);
+    flush_times(ctx);
+    return rc;
+}
+
+// D devices: TextParts splits and parses the PAF; every device runs batch_stats_rows on its records (rec_base: integrity errors name
+// global record indices).  The devices hold runs of the file order, so the merge is a concatenation: device d's rows go to row
+// rec_base, its bytes behind the bytes of the devices before it, and its line offsets move by that many bytes.
+static int stats_text_multi(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, int qbed, bool text, rb_lift_out* out, rb_stats_out* stats,
+                            rb_paf_info* info) {
+    Devices dev(ctx);
+    const int D = dev.n;
+    Rendezvous rv(D);
+    int call_rc = RB_OK;
+    TextParts tp(dev, rv, call_rc, paf, paf_nbytes);
+    const int src_rc = tp.split();
+    if (src_rc != RB_OK) return src_rc;
+    std::vector<uint64_t> byte_base((size_t)D, 0);
+    RowsOut rows;
+    uint64_t tot_rows = 0, tot_bytes = 0;
+
+    dev.run([&](int d, rb_ctx* c) {
+        int& status = dev.rc[(size_t)d];
+        rb_batch* b = c->scratch;
+        cudaStream_t s = c->stream;
+        auto cleanup = [&] {
+            if (b->busy) { cudaStreamSynchronize(s); b->busy = false; }
+            tp.release(d);
+        };
+        if (!tp.parse(d, c, info)) { cleanup(); return; }
+        status = [&]() -> int {
+            rb_ctx* ctx = c;  // (CU reports into this device's context)
+            int rc = paf_upload_names(c, b, tp.part[(size_t)d].p, tp.b0->h_names.data(), tp.b0->h_names_off.data(), tp.n_names, nullptr);
+            if (rc != RB_OK) return rc;
+            b->rec_base = (uint32_t)tp.part[(size_t)d].rec_base;
+            CU(cudaStreamSynchronize(s));
+            b->busy = false;
+            return batch_stats_rows(c, b, qbed, text);
+        }();
+        rv.meet([&] {  // every device's sizes are known: lay out the one output block
+            call_rc = dev.error(false);  // (devices hold runs of the file order: the first failing device holds the first failing record)
+            if (call_rc != RB_OK) return;
+            for (int k = 0; k < D; k++) {
+                byte_base[(size_t)k] = tot_bytes;
+                tot_rows += dev.at(k)->scratch->n_rec;
+                tot_bytes += dev.at(k)->scratch->sum.out_bytes;
+            }
+            cudaSetDevice(ctx->device);  // (the pinned pool belongs to the first device's context)
+            call_rc = rows.reserve(ctx, tot_rows, tot_bytes, text ? RB_WANT_TEXT : 0u, stats != nullptr);
+            cudaSetDevice(c->device);
+        });
+        if (call_rc != RB_OK) { cleanup(); return; }
+        // this device's rows -> their place in the merged output
+        status = [&]() -> int {
+            rb_ctx* ctx = c;  // (CU reports into this device's context)
+            const uint64_t n = b->n_rec, nb = b->sum.out_bytes;
+            if (text && n && byte_base[(size_t)d]) launch_add_u64(b->out_line_off.as<uint64_t>(), n, byte_base[(size_t)d], s);
+            const int rc = rows.copy_rows(c, b, 0, n, 0, nb, tp.part[(size_t)d].rec_base, byte_base[(size_t)d], s);
+            if (rc != RB_OK) return rc;
+            CU(cudaStreamSynchronize(s));
+            flush_times(c);
+            return RB_OK;
+        }();
+        cleanup();
+    });
+    if (call_rc == RB_OK) call_rc = dev.error(false);
+    if (call_rc != RB_OK) { rows.release(); return call_rc; }
+    rows.finish(out, stats, tot_rows, tot_bytes, tot_rows);
+    return RB_OK;
+}
+
+int rb_stats_text(rb_ctx* ctx, const uint8_t* paf, uint64_t paf_nbytes, int qbed, uint32_t want, rb_lift_out* rows, rb_stats_out* stats,
+                  rb_paf_info* info) {
+    if (!ctx) return RB_ERR_NO_DEVICE;
+    if (info) memset(info, 0, sizeof *info);
+    if (!rows) return fail(ctx, RB_ERR_BAD_ARG, "rows is null");
+    memset(rows, 0, sizeof *rows);
+    if (stats) memset(stats, 0, sizeof *stats);
+    if (!paf && paf_nbytes) return fail(ctx, RB_ERR_BAD_ARG, "rb_stats_text: null data");
+    if (want & ~RB_WANT_STATS_TEXT) return fail(ctx, RB_ERR_BAD_ARG, "rb_stats_text: want takes RB_WANT_STATS_TEXT or 0");
+    cudaSetDevice(ctx->device);
+    const bool text = want != 0;
+    const int rc = ctx->peers.empty() || paf_nbytes < ctx->multi_min_bytes ? stats_text_one(ctx, paf, paf_nbytes, qbed, text, rows, stats, info)
+                                                                         : stats_text_multi(ctx, paf, paf_nbytes, qbed, text, rows, stats, info);
+    if (rc != RB_OK) {
+        if (info && !info->names_off) memset(info, 0, sizeof *info);
+        memset(rows, 0, sizeof *rows);
         if (stats) memset(stats, 0, sizeof *stats);
     }
     return rc;

@@ -112,13 +112,11 @@ int main(int argc, char** argv) {
         return rbh::Paf::from_file(path);
     };
     // RB_DEVICE_PARSE=1: `rb [--gpus N] liftover` (plain, --stats, --largest) hands the bytes of the PAF and the BED to one
-    // rb_liftover_text call — lines are split and parsed on the device(s) — instead of parsing them on the host; `rb stats --paf` on
-    // one GPU hands the PAF's bytes to rb_batch_upload_paf.  A plain file is mapped, a .bgz / .gz that is BGZF goes as it is
-    // (inflated on the device), a plain .gz and stdin are inflated / read by rbh::read_all first.
+    // rb_liftover_text call, and `rb [--gpus N] stats --paf [--qbed]` the bytes of the PAF to one rb_stats_text call — lines are split
+    // and parsed (and the stats rows formatted) on the device(s) instead of on the host.  A plain file is mapped, a .bgz / .gz that is
+    // BGZF goes as it is (inflated on the device), a plain .gz and stdin are inflated / read by rbh::read_all first.
     const char* dp = getenv("RB_DEVICE_PARSE");
-    const bool device_parse = dp && dp[0] == '1' && !qbed && (cmd == "liftover" || (cmd == "stats" && n_gpus == 1));
-    rb_batch* batch = nullptr;
-    rb_paf_info info{};
+    const bool device_parse = dp && dp[0] == '1' && ((cmd == "liftover" && !qbed) || cmd == "stats");
     struct InputBytes {
         std::string owned;
         const uint8_t* data = nullptr;
@@ -147,35 +145,25 @@ int main(int argc, char** argv) {
         }
         if (!in.map) { in.data = reinterpret_cast<const uint8_t*>(in.owned.data()); in.n = in.owned.size(); }
     };
-    auto upload_paf = [&](const std::string& path) {
-        int st = 0;
-        {
-            InputBytes in;
-            input_bytes(path, in);
-            batch = rb_batch_upload_paf(ctx, in.data, in.n, &info, &st);
-        }
-        if (!batch) return st;
-        if (info.skipped) fprintf(stderr, "\nUnable to parse %zu PAF record(s). Skipped.\n", (size_t)info.skipped);
-        return (int)RB_OK;
-    };
     int rc = 0;
     try {
         if (device_parse && cmd == "stats") {
             fputs(rbh::stats_header(qbed).c_str(), stdout);  // printed before the input is read (main.rs:51)
             fflush(stdout);
-            rc = upload_paf(input);
-            mark("device_parse_paf");
-            rb_stats_out st{};
-            rb_records recs{};
-            if (rc == RB_OK) rc = rb_batch_stats(ctx, batch, nullptr);
-            if (rc == RB_OK) rc = rb_batch_download_stats(ctx, batch, &st);
-            if (rc == RB_OK) rc = rb_batch_records(ctx, batch, 0, &recs);
-            mark("rb_batch_stats");
+            rb_lift_out out{};
+            rb_paf_info pinfo{};
+            {
+                InputBytes paf_in;
+                input_bytes(input, paf_in);
+                rc = rb_stats_text(ctx, paf_in.data, paf_in.n, qbed ? 1 : 0, RB_WANT_STATS_TEXT, &out, nullptr, &pinfo);
+            }
+            mark("rb_stats_text");
+            if (pinfo.names_off && pinfo.skipped) fprintf(stderr, "\nUnable to parse %zu PAF record(s). Skipped.\n", (size_t)pinfo.skipped);
             if (rc == RB_OK) {
-                rbh::write_stats_rows(stdout, recs, st, qbed);
+                fwrite(out.paf_text, 1, out.paf_nbytes, stdout);
                 fflush(stdout);
-                mark("format_write");
-                rb_free_stats_out(ctx, &st);
+                mark("write");
+                rb_free_lift_out(ctx, &out);
             }
         } else if (device_parse) {
             if (bed.empty()) return usage();
@@ -284,18 +272,15 @@ int main(int argc, char** argv) {
         }
     } catch (const rbh::Panic& e) {
         fprintf(stderr, "thread 'main' panicked: %s\n", e.what());
-        if (batch) rb_batch_free(ctx, batch);
         rb_ctx_destroy(ctx);
         return 101;
     }
     if (rc != RB_OK) {
         fprintf(stderr, "rb: %s\n", rb_last_error(ctx));
         const bool ref_panic = (rc <= RB_ERR_REF_CIGAR_PARSE && rc >= RB_ERR_REF_INDEX) || rc == RB_ERR_REF_PAF_PARSE;
-        if (batch) rb_batch_free(ctx, batch);
         rb_ctx_destroy(ctx);
         return ref_panic ? 101 : 1;
     }
-    if (batch) rb_batch_free(ctx, batch);
     rb_ctx_destroy(ctx);
     mark("destroy");
     if (timing)

@@ -709,16 +709,6 @@ void write_stats_rows(FILE* f, const Paf& paf, const rb_stats_out& st, bool qbed
     write_rows(f, paf.size(), [&](std::string& out, size_t i) { append_stats_row(out, paf, i, st, qbed); });
 }
 
-void write_stats_rows(FILE* f, const rb_records& recs, const rb_stats_out& st, bool qbed) {
-    auto name = [&](uint32_t id) {
-        return std::string(reinterpret_cast<const char*>(recs.names) + recs.names_off[id], (size_t)(recs.names_off[id + 1] - recs.names_off[id]));
-    };
-    write_rows(f, recs.n_rec, [&](std::string& out, size_t i) {
-        append_row(out, name(recs.q_id[i]), name(recs.t_id[i]), recs.strand[i], recs.q_st[i], recs.q_en[i], recs.q_len[i], recs.t_st[i],
-                   recs.t_en[i], recs.t_len[i], st, i, qbed);
-    });
-}
-
 // ---------------------------------------------------------------------------------------------
 // --largest (host-side post-filter over the rows the GPU produced; needs RB_WANT_TEXT | RB_WANT_NUMERIC)
 // ---------------------------------------------------------------------------------------------

@@ -121,8 +121,6 @@ void append_row(std::string& out, const std::string& q_name, const std::string& 
                 uint64_t q_len, uint64_t t_st, uint64_t t_en, uint64_t t_len, const rb_stats_out& st, size_t i, bool qbed);
 // every row of `paf` (bamstats.rs:239-270), formatted on all host threads, written to `f` in row order
 void write_stats_rows(FILE* f, const Paf& paf, const rb_stats_out& st, bool qbed);
-// the same for records the library holds (rb_batch_records of a batch parsed on the device)
-void write_stats_rows(FILE* f, const rb_records& recs, const rb_stats_out& st, bool qbed);
 
 // ---- synthetic whole-genome-scale eqx PAF (SURVEY §8d, configs C2-C5) ----
 struct SynthParams {
